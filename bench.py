@@ -50,7 +50,14 @@ def parse():
     ap.add_argument("--store-rows", type=int, default=1 << 20,
                     help="cfg5: rows of each rank's synthetic token store (chunk id -> row modulo this; a full store is "
                          "16 KB per chunk, 800 GB at 50M chunks)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write every array the last timed step returned as DIR/<name>.npy (float32 / float64, at most "
+                         "64 MB in all), so that two builds can be compared output for output on the same inputs")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if a.workload == "cfg5":
         if "THR_BENCH_CHUNKS" not in os.environ and a.chunks == 10_000_000:
             a.chunks = 50_000_000
@@ -137,6 +144,42 @@ def digest(*tensors) -> str:
     for t in tensors:
         h.update(t.detach().contiguous().cpu().numpy().tobytes())
     return h.hexdigest()[:16]
+
+
+DUMP_LIMIT = 64 << 20   # bytes written by --dump-outputs
+
+
+def host_outputs(out) -> dict:
+    """The non-empty fields of a SearchOutput as host arrays: float64 stays float64, other floating point becomes
+    float32, ids, ranks, counts and flags become float64 (exact for every id below 2^53)."""
+    import dataclasses
+    import torch
+    arrays = {}
+    for f in dataclasses.fields(out):
+        t = getattr(out, f.name)
+        if t is None:
+            continue
+        if t.dtype != torch.float64:
+            t = t.float() if t.is_floating_point() else t.double()
+        arrays[f.name] = t.detach().cpu().numpy()
+    return arrays
+
+
+def dump_outputs(arrays: dict, dirpath: str, limit: int = DUMP_LIMIT) -> None:
+    """DIR/<name>.npy for every array.  Every array is indexed by query first; if they exceed `limit` together, the same
+    fixed, seeded sample of queries is kept in each, and DIR/query_rows.npy lists which."""
+    import numpy as np
+    d = Path(dirpath)
+    d.mkdir(parents=True, exist_ok=True)
+    B = next(iter(arrays.values())).shape[0]
+    per_query = sum(a.nbytes for a in arrays.values()) / B
+    if per_query * B > limit:
+        n = max(1, int((limit - 8 * B) // per_query))
+        rows = np.sort(np.random.default_rng(0).choice(B, size=n, replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["query_rows"] = rows.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", np.ascontiguousarray(a))
 
 
 def make_config(args, world: int):
@@ -470,6 +513,7 @@ def main():
                "lex_digest": digest(out.lex_ids, out.lex_scores, out.lex_count)}
     if rerank:
         digests["rerank_digest"] = digest(out.rr_ids, out.rr_score, out.rr_keep, out.refused, out.max_score)
+    dumped = host_outputs(out) if args.dump_outputs and rank == 0 else None
     qn = float(Q.float().norm(dim=1).max().item())
     xn = float(X[: min(hi - lo, 1 << 20)].float().norm(dim=1).max().item())
     cert_bound = dense_error_bound(D, qn, xn)
@@ -635,6 +679,8 @@ def main():
         except Exception as e:  # the baseline is a reported extra; never lose the GPU numbers over it
             line["cpu_baseline"] = {"value": None, "unit": "queries/s", "cores": None, "kind": "port",
                                     "sample": f"failed: {e!r}"}
+    if dumped is not None:
+        dump_outputs(dumped, args.dump_outputs)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -1,4 +1,4 @@
-"""pytest plugin for tests/test_ref_subclass_cpu.py (runs only where /root/reference exists, i.e. without a GPU):
+"""pytest plugin for tests/test_ref_subclass_cpu.py (runs only where THR_REFERENCE_DIR names a reference checkout):
 swaps the reference's RAG2Retriever for triple_hybrid_rag_b200's SUBCLASS of it, wired to a stub engine whose
 fuse_ranked / safety are the CPU oracle.  What this checks is the plumbing of the literal drop-in — that the
 subclass constructs like the reference class, that the reference's own retrieve() / _retrieve_candidates() call the

@@ -1,7 +1,8 @@
 """Literal boundary (VERDICT r01 item 5a): where the reference package is importable, GpuRAG2Retriever IS a subclass
 of the reference's RAG2Retriever and reads the reference's SETTINGS.  The reference's own two hot-path test files
-run here against that subclass (tests/ref_subclass_plugin.py supplies a stub engine: no GPU in this container).
-Skipped where /root/reference is absent (the GPU box)."""
+run here against that subclass (tests/ref_subclass_plugin.py supplies a stub engine, so no GPU is needed).
+The reference is third-party source and not part of this repository: point THR_REFERENCE_DIR at a checkout of it
+(the directory holding src/voice_agent and tests/) to run these; without it they skip."""
 import os
 import re
 import subprocess
@@ -10,10 +11,10 @@ from pathlib import Path
 
 import pytest
 
-REF = Path("/root/reference")
+REF = Path(os.environ["THR_REFERENCE_DIR"]) if os.environ.get("THR_REFERENCE_DIR") else None
 HERE = Path(__file__).resolve().parent
-pytestmark = pytest.mark.skipif(not (REF / "src" / "voice_agent" / "rag2" / "retrieval.py").exists(),
-                                reason="reference checkout not present")
+pytestmark = pytest.mark.skipif(REF is None or not (REF / "src" / "voice_agent" / "rag2" / "retrieval.py").is_file(),
+                                reason="THR_REFERENCE_DIR does not point at a checkout of the reference")
 
 
 def _env():
@@ -38,10 +39,10 @@ def test_subclass_binds_to_the_reference():
     assert out.returncode == 0, out.stdout + out.stderr
 
 
-def test_reference_tests_run_through_the_subclass():
+def test_reference_tests_run_through_the_subclass(tmp_path):
     files = [str(REF / "tests" / n) for n in ("test_rag2_triple_hybrid.py", "test_rag2_retrieval.py")]
     cmd = [sys.executable, "-m", "pytest", "-p", "asyncio_shim", "-p", "ref_subclass_plugin", "-p", "no:cacheprovider",
-           "-c", os.devnull, "--rootdir", "/tmp", "-q", "-rf"] + files
-    out = subprocess.run(cmd, capture_output=True, text=True, env=_env(), cwd="/tmp", timeout=900)
+           "-c", os.devnull, "--rootdir", str(tmp_path), "-q", "-rf"] + files
+    out = subprocess.run(cmd, capture_output=True, text=True, env=_env(), cwd=tmp_path, timeout=900)
     m = re.search(r"(\d+) passed", out.stdout)
     assert out.returncode == 0 and m and int(m.group(1)) == 51, out.stdout[-4000:] + out.stderr[-2000:]
