@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define THR_ABI_VERSION 10
+#define THR_ABI_VERSION 11
 
 enum {
   THR_OK = 0,
@@ -103,11 +103,11 @@ int thr_dense_index_set(thr_handle* h, const void* X, int64_t N, int D, int64_t 
  * fp32 scores select k + margin survivors, which are re-scored exactly before the final sort).
  *   out_ids    [B, k] int64   (id_base + row; -1 past out_count)
  *   out_scores [B, k] double
- *   out_count  [B]    int32   min(k, N)
+ *   out_count  [B]    int32   min(k, N live rows)
  *   out_gap    [B]    float, nullable: (exact k-th score) - (best tensor-core score that was
  *              NOT re-scored); the result is certified exact when gap > the fp32 accumulation
  *              error bound.  +inf when every chunk was re-scored.
- * 1 <= k, k + margin <= 256.
+ * 1 <= k, k + margin <= 256.  Rows marked in the deletion bitmap (thr_dense_deleted_set) are never returned.
  */
 int thr_dense_topk(thr_handle* h, const void* Q, int B, int k, int margin,
                    int64_t* out_ids, double* out_scores, int32_t* out_count, float* out_gap,
@@ -124,6 +124,15 @@ int thr_dense_tags_set(thr_handle* h, const uint16_t* tags);
 int thr_dense_topk_tagged(thr_handle* h, const void* Q, int B, int k, int margin, const int32_t* want,
                           int64_t* out_ids, double* out_scores, int32_t* out_count, float* out_gap,
                           void* stream);
+
+/* Deletion bitmap of the semantic channel: rows removed from the corpus without a rebuild.  bits
+ * [ceil(N / 32)] uint32 on the device (16-byte aligned, stays resident; NULL clears): bit i % 32 of word i / 32
+ * set = row i is deleted.  While it is set, every thr_dense_topk / thr_dense_topk_tagged call (every query, any
+ * want) skips deleted rows inside the scan: they are never returned, thresholds are learnt from live rows only,
+ * out_count = min(k, live eligible rows), and out_gap keeps its meaning over the eligible rows.  Like the tags,
+ * the bitmap is dropped by the next thr_dense_index_set.
+ */
+int thr_dense_deleted_set(thr_handle* h, const uint32_t* bits);
 
 /* ---- K2: lexical channel — BM25 top-k over a blocked CSR inverted index ----------
  * Replaces RAG2Retriever._lexical_search -> RPC rag2_lexical_search
@@ -157,7 +166,8 @@ int thr_bm25_index_set(thr_handle* h, const int64_t* skip, const void* postings,
  * definition, so results are bit-reproducible.  Only docs with score > 0 are eligible;
  * order is (score desc, id asc).
  *   out_ids [B,k] int64 (-1 past count), out_scores [B,k] float, out_count [B] int32.
- * 1 <= k <= 256, at most 32 terms per query.
+ * 1 <= k <= 256, at most 32 terms per query.  Docs marked in the deletion bitmap (thr_bm25_deleted_set) are never
+ * returned.
  */
 int thr_bm25_topk(thr_handle* h, const int32_t* q_terms, const int32_t* q_off, int B, int k,
                   int64_t* out_ids, float* out_scores, int32_t* out_count, void* stream);
@@ -168,6 +178,13 @@ int thr_bm25_tags_set(thr_handle* h, const uint16_t* tags);
 int thr_bm25_topk_tagged(thr_handle* h, const int32_t* q_terms, const int32_t* q_off, int B, int k,
                          const int32_t* want, int64_t* out_ids, float* out_scores, int32_t* out_count,
                          void* stream);
+
+/* Deletion bitmap of the lexical channel: same contract as thr_dense_deleted_set, over local doc ids; bits
+ * [ceil(n_docs / 32)] uint32 on the device, 16-byte aligned.  Applies to every thr_bm25_topk* call (OR and AND,
+ * any want); dropped by the next thr_bm25_index_set.  idf is the caller's: recompute it from the live docs and
+ * write it into the resident idf array when the live set changes.  The planner's cost estimates keep counting
+ * the postings of deleted docs. */
+int thr_bm25_deleted_set(thr_handle* h, const uint32_t* bits);
 
 /* AND semantics — the `tsv @@ plainto_tsquery(...)` predicate of rag2_lexical_search
  * (database/migrations/20260114_rag2_schema.sql:369: every lexeme of the query must match).  thr_bm25_topk_ex is

@@ -68,6 +68,7 @@ struct Bm25Args {
   int32_t* part_cnt;      // [max_units]
   const uint16_t* tags;   // [n_docs] nullable: per-doc tag (collection id) for filtered queries
   const int32_t* want;    // [B] nullable: tag a query's docs must carry, < 0 = any
+  const uint32_t* deleted;  // [ceil(n_docs / 32)] nullable: bit d % 32 of word d / 32 set = doc d is deleted
   uint64_t* wlists;       // [grid][warps][kListCap] per-warp candidate lists
   unsigned* tau_q;        // [B] running threshold per query (fp32 bits of a score >= 0), shared by its units
   int require_all;        // AND semantics: a doc must contain every (distinct, known) query term
@@ -280,7 +281,10 @@ __global__ void __launch_bounds__(kBlk == 2048 ? 768 : 1024, 1) bm25_range_kerne
         __syncwarp();
       }
     };
-    // Append the lanes' candidates (has) to the list; room for 32 entries is the caller's invariant.
+    // Append the lanes' candidates (has) to the list; room for 32 entries is the caller's invariant.  Every candidate
+    // passes here, so the tag filter acts on all of them.  The deletion bitmap is tested by the two callers (a test
+    // here costs the AND instantiations spills: the slow scan reads one word for a lane's four docs); either way a
+    // deleted doc never enters a list, and the threshold (the histogram of appended scores) is learnt from live docs.
     auto append = [&](bool has, float score, uint32_t doc) {
       if (has && want >= 0) has = (int)__ldg(a.tags + doc) == want;
       const unsigned m = __ballot_sync(0xffffffffu, has);
@@ -487,7 +491,9 @@ __global__ void __launch_bounds__(kBlk == 2048 ? 768 : 1024, 1) bm25_range_kerne
             if (kAnd) asm volatile("ld.shared.u8 %0, [%1];" : "=r"(hc) : "r"(hit0 + cross_doc));
           }
           const int before = n_list;
-          append(cross_doc != 0xffffffffu && v > tau && (!kAnd || hc == (uint32_t)need), v, cross_doc);
+          append(cross_doc != 0xffffffffu && v > tau && (!kAnd || hc == (uint32_t)need) &&
+                     !(a.deleted && ((__ldg(a.deleted + (cross_doc >> 5)) >> (cross_doc & 31u)) & 1u)),
+                 v, cross_doc);
           appended = n_list - before;
         }
       } else {
@@ -506,12 +512,14 @@ __global__ void __launch_bounds__(kBlk == 2048 ? 768 : 1024, 1) bm25_range_kerne
           uint32_t hc4 = 0u;
           if (kAnd) asm volatile("ld.shared.b32 %0, [%1];" : "=r"(hc4) : "r"(hit_u + (uint32_t)(j * 32 + lane) * 4u));
           if (__any_sync(0xffffffffu, m != 0u)) {
+            // the lane's four docs share a bitmap word; docs past n_docs (the last range's tail) have none
+            const uint32_t doc4 = doc0 + (uint32_t)(j * 32 + lane) * 4u;
+            const uint32_t dead4 = a.deleted && doc4 < a.n_docs ? __ldg(a.deleted + (doc4 >> 5)) >> (doc4 & 31u) : 0u;
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
               const float x = __uint_as_float(v[c]) * kAccUnscale;
-              const uint32_t doc = doc0 + (uint32_t)(j * 32 + lane) * 4u + c;
               const bool all = !kAnd || ((hc4 >> (8 * c)) & 255u) == (uint32_t)need;
-              append(x > tcur && x > 0.f && all, x, doc);
+              append(x > tcur && x > 0.f && all && !((dead4 >> c) & 1u), x, doc4 + c);
             }
           }
         }
@@ -792,6 +800,7 @@ struct thr_bm25_state {
   int64_t id_base;
   int64_t* df;  // [V] device
   const uint16_t* tags;  // [n_docs] device, nullable
+  const uint32_t* deleted;  // [ceil(n_docs / 32)] device, nullable
   // planner tuning (per handle; THR_BM25_* environment variables are read once, when the index is set)
   int units_per_cta;
   long long range_cost, term_cost;
@@ -867,6 +876,14 @@ int thr_bm25_tags_set(thr_handle* h, const uint16_t* tags) {
   if (!h->bm25) return thr_fail(h, THR_ENOINDEX, "thr_bm25_tags_set: call thr_bm25_index_set first");
   THR_REQUIRE(h, ((uintptr_t)tags & 7u) == 0, "thr_bm25_tags_set: tags must be 8-byte aligned");
   h->bm25->tags = tags;
+  return THR_OK;
+}
+
+int thr_bm25_deleted_set(thr_handle* h, const uint32_t* bits) {
+  if (!h) return THR_EINVAL;
+  if (!h->bm25) return thr_fail(h, THR_ENOINDEX, "thr_bm25_deleted_set: call thr_bm25_index_set first");
+  THR_REQUIRE(h, ((uintptr_t)bits & 15u) == 0, "thr_bm25_deleted_set: bits must be 16-byte aligned");
+  h->bm25->deleted = bits;
   return THR_OK;
 }
 
@@ -962,7 +979,7 @@ static int bm25_topk_impl(thr_handle* h, const int32_t* q_terms, const int32_t* 
   a.n_blk = st->n_blk; a.blk_docs = st->blk_docs; a.blk_shift = st->blk_shift; a.V = st->V;
   a.q_terms = q_terms; a.q_off = q_off; a.order = order; a.units = units; a.total_units = total_units;
   a.work_counter = counter; a.B = B; a.k = k; a.part_keys = part_keys; a.part_cnt = part_cnt;
-  a.tags = want ? st->tags : nullptr; a.want = want;
+  a.tags = want ? st->tags : nullptr; a.want = want; a.deleted = st->deleted;
   a.wlists = (uint64_t*)(ws + o_wl); a.tau_q = (unsigned*)(ws + o_tau); a.require_all = require_all;
   a.status = h->d_status;
   tok = thr_prof_begin(h, THR_PROF_BM25, s);

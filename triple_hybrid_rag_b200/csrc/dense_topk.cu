@@ -62,6 +62,7 @@ struct ScoreArgs {
   int seed_mode;          // seed pass: leave the lists uncompacted (<= kSeedTilesMax * kTileN entries each)
   const uint16_t* tags;   // [N] nullable: per-chunk tag (collection id) for filtered queries
   const int32_t* want;    // [B] nullable: tag a query's chunks must carry, < 0 = any
+  const uint32_t* deleted;  // [ceil(N / 32)] nullable: bit i % 32 of word i / 32 set = row i is deleted
   thr_dev_status* status;
 };
 
@@ -131,8 +132,8 @@ __device__ uint64_t warp_compact_topk(uint64_t* row, int n, int ksel, uint32_t l
   return mn;
 }
 
-// kSeed: the seed pass (a.seed_mode): thresholds stay at -inf, lists stay uncompacted, and without a tag filter every
-// score of a tile is stored — with 32-byte stores, four entries a time (the generic append path stores 8 bytes per lane
+// kSeed: the seed pass (a.seed_mode): thresholds stay at -inf, lists stay uncompacted, and without a tag filter or a
+// deletion bitmap every score of a tile is stored — with 32-byte stores, four entries a time (the generic append path stores 8 bytes per lane
 // per instruction into 32 different rows: at one wavefront per row that path alone was ~2/3 of the seed pass).
 template <int G, bool kSeed>
 __global__ void __launch_bounds__(kScoreThreads, 1)
@@ -275,6 +276,8 @@ dense_score_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
       // tag filter: a chunk outside the query's tag is never appended, so every threshold (seed pass included) is
       // learnt from eligible chunks only and the result is the exact top-k of the filtered corpus
       const int want = (row_valid && a.tags && a.want) ? a.want[row] : -1;
+      // deleted rows are dropped at the same place: thresholds, seed bound included, come from live rows only (the
+      // seed pass takes the filtered path below when a bitmap is set, so a deleted row never reaches its select)
       int cnt = 0;
       for (int64_t t = tile_lo; t < tile_hi && ok; ++t, ++tcount) {
         const int acc = tcount & 1;
@@ -296,7 +299,7 @@ dense_score_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         const int64_t col0 = t * kTileN;
         const int ncols = (int)min((int64_t)kTileN, a.N - col0);
         uint64_t* wptr = rowbuf + cnt;
-        if (kSeed && a.tags == nullptr && ncols == kTileN) {
+        if (kSeed && a.tags == nullptr && a.deleted == nullptr && ncols == kTileN) {
           // seed pass, full tile, no tag filter: all kTileN scores of the row, in column order
 #pragma unroll 1
           for (int c = 0; c < kTileN / 32; ++c) {
@@ -329,7 +332,7 @@ dense_score_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
 // Four columns at a time: max + one compare + one warp vote; the (predicated) appends run only when
 // some lane of the warp passes — after warm-up that is ~ 128*K'/seen of the groups.
 #define P1(j, tg)                                                                                  \
-  if (__uint_as_float(r[j]) > tau && (want < 0 || (int)(tg) == want))                              \
+  if (__uint_as_float(r[j]) > tau && (want < 0 || (int)(tg) == want) && !((dw >> (j)) & 1u))       \
     *wptr++ = ((uint64_t)r[j] << 32) | (uint64_t)(inv0 - (uint32_t)(j));
 #define P(j)                                                                                       \
   {                                                                                                \
@@ -339,6 +342,7 @@ dense_score_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
       asm volatile("" ::: "memory"); /* keep this a real (warp-uniform) branch */                  \
       ushort4 tg = make_ushort4(0, 0, 0, 0);                                                       \
       if (a.tags) tg = __ldg((const ushort4*)(a.tags + col0 + c * 32 + (j))); /* 8-byte aligned */ \
+      const uint32_t dw = a.deleted ? __ldg(a.deleted + ((col0 >> 5) + c)) : 0u; /* the c block's word */ \
       P1(j, tg.x) P1(j + 1, tg.y) P1(j + 2, tg.z) P1(j + 3, tg.w)                                  \
     }                                                                                              \
   }
@@ -358,7 +362,8 @@ dense_score_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
 #pragma unroll
               for (int j = 0; j < 32; ++j) {
                 const int col = c * 32 + j;
-                if (__uint_as_float(r[j]) > tau && col < ncols && (want < 0 || (int)a.tags[col0 + col] == want))
+                if (__uint_as_float(r[j]) > tau && col < ncols && (want < 0 || (int)a.tags[col0 + col] == want) &&
+                    !(a.deleted && ((a.deleted[(col0 + col) >> 5] >> ((col0 + col) & 31)) & 1u)))
                   *wptr++ = ((uint64_t)r[j] << 32) | (uint64_t)(~(uint32_t)(col0 + col));
               }
             }
@@ -779,6 +784,7 @@ struct thr_dense_state {
   CUtensorMap map_x;
   int cta_group;  // 2 (pair) or 1; THR_DENSE_CTA_GROUP overrides for bring-up
   const uint16_t* tags;  // [N] device, nullable
+  const uint32_t* deleted;  // [ceil(N / 32)] device, nullable
   // tuning knobs, read from the environment ONCE, when the index is set (THR_DENSE_SEED_TILES, THR_DENSE_NO_SEED)
   int seed_tiles;  // 0: the default for the shard size
   int no_seed;
@@ -848,6 +854,14 @@ int thr_dense_tags_set(thr_handle* h, const uint16_t* tags) {
   return THR_OK;
 }
 
+int thr_dense_deleted_set(thr_handle* h, const uint32_t* bits) {
+  if (!h) return THR_EINVAL;
+  if (!h->dense) return thr_fail(h, THR_ENOINDEX, "thr_dense_deleted_set: call thr_dense_index_set first");
+  THR_REQUIRE(h, ((uintptr_t)bits & 15u) == 0, "thr_dense_deleted_set: bits must be 16-byte aligned");
+  h->dense->deleted = bits;
+  return THR_OK;
+}
+
 int thr_dense_topk(thr_handle* h, const void* Q, int B, int k, int margin, int64_t* out_ids,
                    double* out_scores, int32_t* out_count, float* out_gap, void* stream) {
   return thr_dense_topk_tagged(h, Q, B, k, margin, nullptr, out_ids, out_scores, out_count, out_gap, stream);
@@ -892,6 +906,7 @@ int thr_dense_topk_tagged(thr_handle* h, const void* Q, int B, int k, int margin
   a.seed_mode = 0;
   a.tags = want ? st->tags : nullptr;
   a.want = want;
+  a.deleted = st->deleted;
   float* tau_seed = (float*)(ws + cand_bytes + cnt_bytes);
 
   FinalArgs f;

@@ -114,6 +114,16 @@ class Engine:
         self._keep["dense_tags"] = tags
         self._check(self._lib.thr_dense_tags_set(self._h, _ptr(tags)))
 
+    def dense_deleted_set(self, bits: Optional[torch.Tensor]):
+        """Deletion bitmap ([ceil(N / 32)] int32 words on the device, bit i % 32 of word i / 32 = row i deleted):
+        dense_topk never returns a deleted row; None clears."""
+        if bits is not None:
+            bits = self._dev(bits, torch.int32, "bits")
+            if bits.numel() * 32 < self._keep["X"].shape[0]:
+                raise ValueError("the bitmap needs one bit per chunk")
+        self._keep["dense_deleted"] = bits
+        self._check(self._lib.thr_dense_deleted_set(self._h, _ptr(bits)))
+
     def dense_topk(self, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None
                    ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
         """-> ids [B,k] int64, scores [B,k] float64, count [B] int32, gap [B] float32.
@@ -141,7 +151,7 @@ class Engine:
         n_blk = (n_docs + blk_docs - 1) // blk_docs
         if skip.numel() != V * n_blk + 1:
             raise ValueError("skip must have V * n_blk + 1 entries")
-        self._keep.update(skip=skip, postings=postings, idf=idf)
+        self._keep.update(skip=skip, postings=postings, idf=idf, bm25_n_docs=n_docs)
         self._check(self._lib.thr_bm25_index_set(self._h, _ptr(skip), _ptr(postings), _ptr(idf), n_docs, n_blk,
                                                  blk_docs, V, id_base))
 
@@ -151,6 +161,15 @@ class Engine:
             tags = self._dev(tags, torch.uint16, "tags")
         self._keep["bm25_tags"] = tags
         self._check(self._lib.thr_bm25_tags_set(self._h, _ptr(tags)))
+
+    def bm25_deleted_set(self, bits: Optional[torch.Tensor]):
+        """Deletion bitmap over the index's local doc ids (layout as in dense_deleted_set); None clears."""
+        if bits is not None:
+            bits = self._dev(bits, torch.int32, "bits")
+            if bits.numel() * 32 < self._keep["bm25_n_docs"]:
+                raise ValueError("the bitmap needs one bit per doc")
+        self._keep["bm25_deleted"] = bits
+        self._check(self._lib.thr_bm25_deleted_set(self._h, _ptr(bits)))
 
     def bm25_topk(self, q_terms: torch.Tensor, q_off: torch.Tensor, k: int, want: Optional[torch.Tensor] = None,
                   require_all: bool = False) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:

@@ -93,7 +93,7 @@ class GpuHybridSearcher:
         if q.shape[1] != ix.dim:
             raise ValueError(f"query embedding has {q.shape[1]} dimensions, the index {ix.dim}")
         q = q / q.norm(dim=1, keepdim=True).clamp_min(1e-30)
-        k = min(self.config.top_k_retrieve, len(ix.rows), 228)
+        k = max(1, min(self.config.top_k_retrieve, ix.n_live, 228))
         with eng.lock:
             ids, sc, cnt, gap = eng.dense_topk(pad_dim(q.to(torch.bfloat16)).to(eng.device), k, want=ix.want(category))
             eng.sync()
@@ -120,8 +120,8 @@ class GpuHybridSearcher:
             return []
         qt, qo = pack_queries([list(seen)], eng.device)
         with eng.lock:
-            ids, sc, cnt = eng.bm25_topk(qt, qo, min(self.config.top_k_retrieve, 256), want=ix.want(category), require_all=True)
-            eng.sync()
+            ids, sc, cnt = ix.bm25_topk(qt, qo, min(self.config.top_k_retrieve, 256), want=ix.want(category), require_all=True)
+            ix.sync()
         out = [self._result(i, "bm25", bm25_score=s) for i, s in zip(ids[0, :int(cnt[0])].tolist(), sc[0, :int(cnt[0])].tolist())]
         return [r for r in out if source_document is None or r.source_document == source_document]
 

@@ -75,6 +75,22 @@ def exchange_topk(group, world, B, k_sem, k_lex, d_ids, d_sc, d_cnt, l_ids, l_sc
             l_ids, l_sc, m_cnt[B:].clamp(max=k_lex))
 
 
+def bm25_topk_segments(engine: Engine, delta: Optional[Engine], q_terms: torch.Tensor, q_off: torch.Tensor, k: int,
+                       want: Optional[torch.Tensor] = None, require_all: bool = False):
+    """K2 over a main index and, when `delta` is a handle, a delta segment whose ids follow the main index's (its
+    id_base): each segment's top-k, merged by K5 (G = 2).  fp32 -> fp64 -> fp32 is exact and K5 orders by (score
+    desc, id asc) as K2 does, so the result is what one index over both segments returns.  -> Engine.bm25_topk's.
+    Sync both handles afterwards (ResidentIndex.sync): each reports its own device-side failures."""
+    ids, sc, cnt = engine.bm25_topk(q_terms, q_off, k, want=want, require_all=require_all)
+    if delta is None:
+        return ids, sc, cnt
+    d_ids, d_sc, d_cnt = delta.bm25_topk(q_terms, q_off, k, want=want, require_all=require_all)
+    m_sc, m_ids, m_cnt = engine.merge_topk(torch.stack([sc, d_sc]).to(torch.float64), torch.stack([ids, d_ids]),
+                                           torch.stack([cnt, d_cnt]), k)
+    m_sc = torch.where(m_ids < 0, torch.zeros_like(m_sc), m_sc).to(torch.float32)   # thr_bm25_topk pads with 0
+    return m_ids, m_sc, m_cnt
+
+
 @dataclass
 class SearchOutput:
     ids: torch.Tensor        # [B, top_k] int64, -1 padded
@@ -171,13 +187,17 @@ class TripleHybridSearcher:
                graph_ids: Optional[torch.Tensor], weights: Optional[torch.Tensor] = None,
                k_sem: int = 100, k_lex: int = 100, top_k: int = 100, margin: int = 28,
                tie_mode: int = _lib.TIE_CHUNK_ID, rrf_k: int = 60, want: Optional[torch.Tensor] = None,
-               require_all: bool = False) -> SearchOutput:
+               require_all: bool = False, lex_delta: Optional[Engine] = None) -> SearchOutput:
         """want: int32 [B] on the device — per query, the tag its semantic and lexical hits must carry (< 0: any);
-        needs set_tags.  require_all: AND semantics of the lexical channel (thr_bm25_topk_ex).  The graph list is an
+        needs set_tags.  require_all: AND semantics of the lexical channel (thr_bm25_topk_ex).  lex_delta: the handle
+        of a lexical delta segment (ResidentIndex.delta_engine), searched and merged with the main list; single GPU
+        only.  The graph list is an
         input and is taken as given.  SearchOutput.gap is K1's exactness certificate of THIS shard (compare with
         dense_error_bound; `certify` does it on the host)."""
         eng, dev = self.engine, self.engine.device
         B = Q.shape[0]
+        if lex_delta is not None and self.world > 1:
+            raise NotImplementedError("a lexical delta segment is not supported with a sharded corpus")
         if self.overlap:
             # The two channels do not depend on each other: K2's chain (plan, range kernel, unit merge) goes on a
             # second stream and K1's (seed, select, score, finalize) on a high-priority one.  Both big kernels take
@@ -190,7 +210,8 @@ class TripleHybridSearcher:
             s_dense.wait_stream(main)
             s_lex.wait_stream(main)
             with torch.cuda.stream(s_lex):
-                l_ids, l_sc, l_cnt = eng.bm25_topk(q_terms, q_off, k_lex, want=want, require_all=require_all)
+                l_ids, l_sc, l_cnt = bm25_topk_segments(eng, lex_delta, q_terms, q_off, k_lex, want=want,
+                                                        require_all=require_all)
             with torch.cuda.stream(s_dense):
                 d_ids, d_sc, d_cnt, gap = eng.dense_topk(Q, k_sem, margin, want=want)
             main.wait_stream(s_dense)
@@ -199,7 +220,8 @@ class TripleHybridSearcher:
                 t.record_stream(main)
         else:
             d_ids, d_sc, d_cnt, gap = eng.dense_topk(Q, k_sem, margin, want=want)
-            l_ids, l_sc, l_cnt = eng.bm25_topk(q_terms, q_off, k_lex, want=want, require_all=require_all)
+            l_ids, l_sc, l_cnt = bm25_topk_segments(eng, lex_delta, q_terms, q_off, k_lex, want=want,
+                                                    require_all=require_all)
         if self.world > 1:
             d_ids, d_sc, d_cnt, l_ids, l_sc, l_cnt = self._exchange(B, k_sem, k_lex, d_ids, d_sc, d_cnt,
                                                                     l_ids, l_sc, l_cnt)

@@ -33,11 +33,12 @@ import time
 from dataclasses import dataclass, field
 from typing import Any, Callable, Dict, List, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 
 from . import _lib
 from .engine import Engine
-from .index import BM25Index, pack_queries
+from .index import BM25Index, bm25_idf, pack_queries
 
 
 # ---- result / plan types: field-for-field the reference's (retrieval.py:26-63, query_planner.py:23-50) ----
@@ -211,67 +212,354 @@ class GraphSearchResult:
     source: str
 
 
+def pack_bitmap(dead) -> torch.Tensor:
+    """bool [n] -> int32 words (a multiple of four: 16 bytes): bit i % 32 of word i / 32 set = dead[i], the deletion
+    bitmap of thr_dense_deleted_set / thr_bm25_deleted_set."""
+    dead = np.asarray(dead, dtype=bool)
+    bits = np.zeros(max(1, (len(dead) + 127) // 128) * 128, dtype=bool)
+    bits[:len(dead)] = dead
+    return torch.from_numpy(np.packbits(bits, bitorder="little").view("<u4").astype(np.int32))
+
+
 class ResidentIndex:
     """Everything the scoring path keeps in HBM for one tenant: the bf16 embedding matrix, the BM25
     inverted index, optionally a per-chunk token store for MaxSim, plus the host-side row metadata the
-    retriever returns (the reference reads those columns from rag_child_chunks / rag_parent_chunks)."""
+    retriever returns (the reference reads those columns from rag_child_chunks / rag_parent_chunks).
+
+    Live updates (add_chunks / delete_chunks, a replace is both) keep the index in step with the tables without a
+    rebuild: deleted rows stay in place and are masked inside K1 / K2 by a deletion bitmap; appended rows extend the
+    embedding matrix (one corpus for K1) and go into a second BM25 index, the lexical delta segment, served by a second
+    handle and merged with the main segment's list by K5.  Every search answers exactly what a fresh index built over
+    the live rows, in this index's row order and with the frozen `avgdl`, answers (DESIGN.md §2: N and df follow the
+    live rows, avgdl is frozen at the last full build or compact())."""
 
     def __init__(self, engine: Engine, chunks: Sequence[Dict[str, Any]], embeddings: torch.Tensor,
                  parents: Optional[Dict[str, Dict[str, Any]]] = None, blk_docs: int = 1024,
                  token_store: Optional[torch.Tensor] = None, token_lens: Optional[torch.Tensor] = None,
-                 tokenizer: Optional[Callable[[str], List[str]]] = None):
+                 tokenizer: Optional[Callable[[str], List[str]]] = None, avgdl: Optional[float] = None):
         """chunks: rows with child_id, parent_id, document_id, text, page, modality (row i <-> embeddings[i]).
-        tokenizer: str -> tokens for the lexical channel (default: `tokenize`; see Tokenizer)."""
+        tokenizer: str -> tokens for the lexical channel (default: `tokenize`; see Tokenizer).
+        avgdl: BM25's average document length (default: the mean over these chunks)."""
         if len(chunks) != embeddings.shape[0]:
             raise ValueError("one embedding row per chunk")
         self.engine = engine
         self.tokenizer = tokenizer or tokenize
-        dev = engine.device
-        self.rows = list(chunks)
-        self.id_of = {r["child_id"]: i for i, r in enumerate(self.rows)}
         self.parents = dict(parents or {})
-        self.collections = [r.get("collection") for r in self.rows]
-        # dense (D is padded with zero columns to the kernel's multiple of 64: dot products do not change — this is how
-        # the RAG 1.0 halfvec(4000) column, database/migrations/20260113_halfvec_4000.sql:34-35, becomes 4032 wide)
+        self.blk_docs = blk_docs
+        self.dim = int(embeddings.shape[1])
+        self.version = 0
+        self._delta_engine: Optional[Engine] = None
+        dev = engine.device
+        self._build(list(chunks), self._unit_rows(embeddings).to(dev).contiguous(),
+                    None if token_store is None else token_store.to(torch.bfloat16).to(dev).contiguous(),
+                    None if token_lens is None else token_lens.to(torch.int32).to(dev).contiguous(), avgdl)
+
+    @staticmethod
+    def _unit_rows(embeddings: torch.Tensor) -> torch.Tensor:
+        """L2-normalised bf16 rows, D padded with zero columns to the kernel's multiple of 64: dot products do not
+        change — this is how the RAG 1.0 halfvec(4000) column, database/migrations/20260113_halfvec_4000.sql:34-35,
+        becomes 4032 wide.  Row by row, so appended rows are bit-identical to the same rows of a full build."""
         X = embeddings.to(torch.float32)
         X = X / X.norm(dim=1, keepdim=True).clamp_min(1e-30)
-        self.dim = int(X.shape[1])
-        self.X = pad_dim(X.to(torch.bfloat16)).to(dev).contiguous()
-        engine.dense_index_set(self.X)
-        # lexical
-        vocab: Dict[str, int] = {}
-        d_l, t_l, f_l, lens = [], [], [], []
-        for i, r in enumerate(self.rows):
+        return pad_dim(X.to(torch.bfloat16))
+
+    def _tokenize(self, rows: Sequence[Dict[str, Any]], vocab: Dict[str, int]):
+        """Rows -> (int32 term ids, int32 tf, distinct terms per row, doc lengths) in row order; new words extend
+        `vocab`.  The index keeps this COO on the host for its whole life (8 B per posting): deletes need a row's
+        terms for df, adds rebuild the delta segment from it."""
+        t_l, f_l, per_row, lens = [], [], [], []
+        for r in rows:
             toks = self.tokenizer(r.get("text", ""))
             lens.append(max(len(toks), 1))
             tf: Dict[int, int] = {}
             for w in toks:
                 t = vocab.setdefault(w, len(vocab))
                 tf[t] = tf.get(t, 0) + 1
-            for t, c in tf.items():
-                d_l.append(i); t_l.append(t); f_l.append(c)
-        self.vocab = vocab
-        V = max(len(vocab), 1)
-        self.bm25 = BM25Index.build(torch.tensor(d_l, dtype=torch.int64), torch.tensor(t_l, dtype=torch.int64),
-                                    torch.tensor(f_l, dtype=torch.int32), torch.tensor(lens, dtype=torch.int64), V,
-                                    blk_docs=blk_docs).to(dev)
-        engine.bm25_index_set(self.bm25.skip, self.bm25.postings, self.bm25.idf, self.bm25.n_docs, self.bm25.blk_docs, V)
-        # late-interaction token store (optional)
-        self.token_store = None if token_store is None else token_store.to(torch.bfloat16).to(dev).contiguous()
-        self.token_lens = None if token_lens is None else token_lens.to(torch.int32).to(dev).contiguous()
-        self._set_tags()
+            t_l.extend(tf.keys()); f_l.extend(tf.values()); per_row.append(len(tf))
+        return (np.array(t_l, dtype=np.int32), np.array(f_l, dtype=np.int32), np.array(per_row, dtype=np.int64),
+                np.array(lens, dtype=np.int64))
 
-    def _set_tags(self) -> None:
-        """Collection names -> uint16 tags resident next to the indexes: the reference's `collection` predicate
-        (20260114_rag2_schema.sql:368-370, :404-406) is evaluated inside K1 / K2 (thr_*_topk_tagged)."""
+    def _build(self, rows, X, token_store, token_lens, avgdl) -> None:
+        """A full build over `rows` (X: their unit rows on the device): the constructor and compact()."""
+        dev = self.engine.device
+        self.rows = rows
+        self.id_of = {r["child_id"]: i for i, r in enumerate(rows)}
+        self.collections = [r.get("collection") for r in rows]
+        self._Xbuf, self._tokbuf, self._lenbuf = X, token_store, token_lens
+        self.vocab: Dict[str, int] = {}
+        t, f, per_row, lens = self._tokenize(rows, self.vocab)
+        self._coo_t, self._coo_f, self._lens = t, f, lens
+        self._row_ptr = np.concatenate([[0], np.cumsum(per_row)])
+        V = max(len(self.vocab), 1)
+        doc = np.repeat(np.arange(len(rows), dtype=np.int64), per_row)
+        self.bm25 = BM25Index.build(torch.from_numpy(doc), torch.from_numpy(t), torch.from_numpy(f),
+                                    torch.from_numpy(lens), V, blk_docs=self.blk_docs, avgdl=avgdl).to(dev)
+        self.avgdl = self.bm25.avgdl
+        self.n_main = len(rows)
+        self._df = self.bm25.df.cpu().numpy().astype(np.int64)
+        self._dead = np.zeros(len(rows), dtype=bool)
         names = sorted({c for c in self.collections if c is not None})
         if len(names) >= 0xffff:
             raise ValueError("at most 65534 collections per resident index")
         self.tag_of = {c: i for i, c in enumerate(names)}
-        tags = torch.tensor([self.tag_of.get(c, 0xffff) for c in self.collections], dtype=torch.int32)
-        self.tags = tags.to(torch.uint16).to(self.engine.device).contiguous()
-        self.engine.dense_tags_set(self.tags)
-        self.engine.bm25_tags_set(self.tags)
+        self._tag = self._tags_of(self.collections)
+        self._delta = None
+        self._publish(main=True, delta=True)
+
+    def _tags_of(self, collections) -> np.ndarray:
+        """Collection names -> the uint16 tags resident next to the indexes (0xffff: none): the reference's
+        `collection` predicate (20260114_rag2_schema.sql:368-370, :404-406) is evaluated inside K1 / K2."""
+        return np.array([self.tag_of.get(c, 0xffff) for c in collections], dtype=np.int32)
+
+    # ---- what the kernels read: set after every build and update ----
+    def _publish(self, main: bool, delta: bool) -> None:
+        """Hand the current state to the handles.  main: the embedding matrix or main BM25 index changed (re-set them;
+        that drops tags and bitmaps, so those are always set again); delta: the delta segment's rows changed."""
+        eng, dev = self.engine, self.engine.device
+        N = len(self.rows)
+        self.X = self._Xbuf[:N]
+        self.token_store = None if self._tokbuf is None else self._tokbuf[:N]
+        self.token_lens = None if self._lenbuf is None else self._lenbuf[:N]
+        eng.dense_index_set(self.X)        # N may have grown and the matrix moved
+        if main:
+            b = self.bm25
+            eng.bm25_index_set(b.skip, b.postings, b.idf, b.n_docs, b.blk_docs, b.V)
+        self.tags = torch.from_numpy(self._tag).to(torch.uint16).to(dev).contiguous()
+        eng.dense_tags_set(self.tags)
+        eng.bm25_tags_set(self.tags)        # the main segment reads its prefix
+        idf = bm25_idf(torch.from_numpy(self._df), self.n_live)   # N and df follow the live rows
+        self.bm25.idf.copy_(idf[:self.bm25.V].to(dev))
+        self.bm25.df = torch.from_numpy(self._df[:self.bm25.V].copy()).to(dev)
+        eng.dense_deleted_set(pack_bitmap(self._dead).to(dev) if self._dead.any() else None)
+        eng.bm25_deleted_set(pack_bitmap(self._dead[:self.n_main]).to(dev) if self._dead[:self.n_main].any() else None)
+        if N == self.n_main:
+            self._delta = None
+        else:
+            de = self._delta_engine
+            if de is None:
+                de = self._delta_engine = type(eng)(eng.device)   # a second handle on the same GPU
+            if delta or self._delta is None:
+                lo = int(self._row_ptr[self.n_main])
+                per_row = np.diff(self._row_ptr[self.n_main:])
+                doc = np.repeat(np.arange(N - self.n_main, dtype=np.int64), per_row)
+                self._delta = BM25Index.build(torch.from_numpy(doc), torch.from_numpy(self._coo_t[lo:]),
+                                              torch.from_numpy(self._coo_f[lo:]), torch.from_numpy(self._lens[self.n_main:]),
+                                              len(self.vocab), blk_docs=self.blk_docs, avgdl=self.avgdl, idf=idf).to(dev)
+                d = self._delta
+                de.bm25_index_set(d.skip, d.postings, d.idf, d.n_docs, d.blk_docs, d.V, id_base=self.n_main)
+            else:
+                self._delta.idf.copy_(idf.to(dev))
+            self._delta_tags = self.tags[self.n_main:].clone()   # its own allocation: 8-byte aligned
+            de.bm25_tags_set(self._delta_tags)
+            dd = self._dead[self.n_main:]
+            de.bm25_deleted_set(pack_bitmap(dd).to(dev) if dd.any() else None)
+
+    @property
+    def n_live(self) -> int:
+        """Live chunks: the corpus size every search sees."""
+        return len(self.id_of)
+
+    @property
+    def delta_engine(self) -> Optional[Engine]:
+        """The handle of the lexical delta segment (None while there is none)."""
+        return None if self._delta is None else self._delta_engine
+
+    def sync(self) -> None:
+        """Engine.sync on every handle the index searches with (the delta segment has its own: its device-side
+        failures are reported here too)."""
+        self.engine.sync()
+        if self.delta_engine is not None:
+            self.delta_engine.sync()
+
+    def _host_terms(self) -> None:
+        """The per-row COO of a v1 file, recovered with the tokenizer on the first update (not at load: a v1 file
+        holds impacts, not tf, and re-tokenising the corpus costs as much as a build)."""
+        if self._coo_t is not None:
+            return
+        vocab = dict(self.vocab)
+        t, f, per_row, lens = self._tokenize(self.rows, vocab)
+        if len(vocab) != len(self.vocab):
+            raise ValueError("the tokenizer does not reproduce the index's vocabulary")
+        self._coo_t, self._coo_f, self._lens = t, f, lens
+        self._row_ptr = np.concatenate([[0], np.cumsum(per_row)])
+
+    def bm25_topk(self, q_terms: torch.Tensor, q_off: torch.Tensor, k: int, want: Optional[torch.Tensor] = None,
+                  require_all: bool = False):
+        """K2 over both lexical segments (Engine.bm25_topk's arguments and results)."""
+        from .pipeline import bm25_topk_segments
+        return bm25_topk_segments(self.engine, self.delta_engine, q_terms, q_off, k, want=want, require_all=require_all)
+
+    # ---- live updates ----
+    def add_chunks(self, chunks: Sequence[Dict[str, Any]], embeddings: torch.Tensor,
+                   token_rows: Optional[torch.Tensor] = None, token_lens: Optional[torch.Tensor] = None,
+                   parents: Optional[Dict[str, Dict[str, Any]]] = None) -> None:
+        """Append chunks (rows as in the constructor, row i <-> embeddings[i]).  A child_id already present is
+        replaced: its old row is deleted and the new one appended.  With a token store, token_rows [n, Td, 128] (and
+        token_lens [n] when the store has lengths) come with them.  parents are merged into the parent map."""
+        chunks = list(chunks)
+        n = len(chunks)
+        if n != embeddings.shape[0]:
+            raise ValueError("one embedding row per chunk")
+        if embeddings.dim() != 2 or int(embeddings.shape[1]) != self.dim:
+            raise ValueError(f"embeddings must be [n, {self.dim}]")
+        ids = [r["child_id"] for r in chunks]
+        if len(set(ids)) != n:
+            raise ValueError("a child_id appears twice in one add_chunks call")
+        if (self._tokbuf is None) != (token_rows is None):
+            raise ValueError("token_rows must be given exactly when the index has a token store")
+        if token_rows is not None and (token_rows.shape[0] != n or token_rows.shape[1:] != self._tokbuf.shape[1:]):
+            raise ValueError(f"token_rows must be [n, {self._tokbuf.shape[1]}, {self._tokbuf.shape[2]}]")
+        if (self._lenbuf is None) != (token_lens is None):
+            raise ValueError("token_lens must be given exactly when the index has token lengths")
+        if n == 0:
+            return
+        dev = self.engine.device
+        X = self._unit_rows(embeddings).to(dev)
+        with self.engine.lock:
+            # everything that can fail on the input runs before the first change (tags and vocabulary are read here,
+            # under the lock, so that concurrent adds never hand out a tag twice)
+            new_names = {r.get("collection") for r in chunks} - set(self.tag_of) - {None}
+            if len(self.tag_of) + len(new_names) >= 0xffff:
+                raise ValueError("at most 65534 collections per resident index")
+            self._host_terms()
+            vocab = dict(self.vocab)
+            t, f, per_row, lens = self._tokenize(chunks, vocab)
+            self._kill([self.id_of[c] for c in ids if c in self.id_of])
+            N = len(self.rows)
+            self._Xbuf = self._grow(self._Xbuf, N, n, X)
+            if self._tokbuf is not None:
+                self._tokbuf = self._grow(self._tokbuf, N, n, token_rows.to(torch.bfloat16).to(dev))
+            if self._lenbuf is not None:
+                self._lenbuf = self._grow(self._lenbuf, N, n, token_lens.to(torch.int32).to(dev))
+            for c in sorted(new_names):   # the next free tags; existing tags never change
+                self.tag_of[c] = len(self.tag_of)
+            self.vocab = vocab
+            self._coo_t = np.concatenate([self._coo_t, t])
+            self._coo_f = np.concatenate([self._coo_f, f])
+            self._lens = np.concatenate([self._lens, lens])
+            self._row_ptr = np.concatenate([self._row_ptr, self._row_ptr[-1] + np.cumsum(per_row)])
+            if len(self.vocab) > len(self._df):
+                self._df = np.concatenate([self._df, np.zeros(len(self.vocab) - len(self._df), dtype=np.int64)])
+            np.add.at(self._df, t, 1)
+            self.rows.extend(chunks)
+            self.collections.extend(r.get("collection") for r in chunks)
+            self._tag = np.concatenate([self._tag, self._tags_of(r.get("collection") for r in chunks)])
+            self._dead = np.concatenate([self._dead, np.zeros(n, dtype=bool)])
+            for i, c in enumerate(ids):
+                self.id_of[c] = N + i
+            self.parents.update(parents or {})
+            self.version += 1
+            self._publish(main=False, delta=True)
+
+    @staticmethod
+    def _grow(buf: torch.Tensor, N: int, n: int, new: torch.Tensor) -> torch.Tensor:
+        """Write `new` at rows [N, N + n) of `buf`, reallocating (with an eighth of spare rows) when it is full."""
+        if N + n > buf.shape[0]:
+            cap = N + n + max(n, N // 8)
+            big = torch.empty((cap,) + tuple(buf.shape[1:]), dtype=buf.dtype, device=buf.device)
+            big[:N] = buf[:N]
+            buf = big
+        buf[N:N + n] = new
+        return buf
+
+    def delete_chunks(self, child_ids: Sequence[str]) -> None:
+        """Remove chunks by child_id: K1 and K2 never return them again and N / df / idf follow.  An unknown (or
+        already deleted) id raises KeyError before anything changes."""
+        ids = list(dict.fromkeys(child_ids))
+        missing = [c for c in ids if c not in self.id_of]
+        if missing:
+            raise KeyError(f"unknown child_id(s): {missing[:5]}")
+        if not ids:
+            return
+        with self.engine.lock:
+            self._host_terms()
+            self._kill([self.id_of[c] for c in ids])
+            self.version += 1
+            self._publish(main=False, delta=False)
+
+    def _kill(self, rows: Sequence[int]) -> None:
+        for i in rows:
+            self._dead[i] = True
+            del self.id_of[self.rows[i]["child_id"]]
+            np.subtract.at(self._df, self._coo_t[self._row_ptr[i]:self._row_ptr[i + 1]], 1)
+
+    def compact(self) -> None:
+        """A full rebuild over the live rows: rows are renumbered (child_ids are stable), the delta segment is folded
+        in, the bitmaps are cleared and avgdl is recomputed."""
+        with self.engine.lock:
+            live = np.flatnonzero(~self._dead)
+            sel = torch.from_numpy(live).to(self.engine.device)
+            N = len(self.rows)
+            self.version += 1
+            if self._delta_engine is not None:      # no delta after a full build: free its handle and index
+                self._delta_engine.close()
+                self._delta_engine = self._delta = None
+            self._build([self.rows[i] for i in live], self._Xbuf[:N][sel].contiguous(),
+                        None if self._tokbuf is None else self._tokbuf[:N][sel].contiguous(),
+                        None if self._lenbuf is None else self._lenbuf[:N][sel].contiguous(), None)
+
+    # ---- persistence (SURVEY.md 8f row 1): start a retriever without re-reading / re-embedding the corpus ----
+    def save(self, path) -> None:
+        """thr-resident-v2: the v1 content plus the update state (deletion mask, appended rows, frozen avgdl, tags)."""
+        self._host_terms()
+        b = self.bm25
+        torch.save({"format": "thr-resident-v2", "rows": self.rows, "parents": self.parents, "vocab": self.vocab,
+                    "dim": self.dim,
+                    "X": self.X.cpu(), "token_store": None if self.token_store is None else self.token_store.cpu(),
+                    "token_lens": None if self.token_lens is None else self.token_lens.cpu(),
+                    "bm25": {"skip": b.skip.cpu(), "postings": b.postings.cpu(),
+                             "idf": b.idf.cpu(), "df": b.df.cpu(), "n_docs": b.n_docs,
+                             "blk_docs": b.blk_docs, "V": b.V, "nnz": b.nnz,
+                             "k1": b.k1, "b": b.b, "avgdl": b.avgdl},
+                    "n_main": self.n_main, "dead": torch.from_numpy(self._dead.copy()), "tag_of": self.tag_of,
+                    "df": torch.from_numpy(self._df.copy()), "coo_t": torch.from_numpy(self._coo_t),
+                    "coo_f": torch.from_numpy(self._coo_f), "lens": torch.from_numpy(self._lens),
+                    "row_ptr": torch.from_numpy(self._row_ptr.astype(np.int64))}, path)
+
+    @classmethod
+    def load(cls, engine: Engine, path, tokenizer: Optional[Callable[[str], List[str]]] = None) -> "ResidentIndex":
+        """tokenizer: the callable the index was built with (callables are not persisted; default `tokenize`).
+        Reads thr-resident-v2 and v1 files."""
+        d = torch.load(path, map_location="cpu", weights_only=True)
+        fmt = d.get("format")
+        if fmt not in ("thr-resident-v1", "thr-resident-v2"):
+            raise ValueError(f"{path}: not a ResidentIndex file")
+        self = cls.__new__(cls)
+        dev = engine.device
+        self.engine = engine
+        self.tokenizer = tokenizer or tokenize
+        self.version = 0
+        self._delta_engine = None
+        self._delta = None
+        self.dim = int(d.get("dim", d["X"].shape[1]))
+        self.rows = d["rows"]
+        self.parents = d["parents"]
+        self.collections = [r.get("collection") for r in self.rows]
+        self.vocab = d["vocab"]
+        self._Xbuf = d["X"].to(dev).contiguous()
+        self._tokbuf = None if d["token_store"] is None else d["token_store"].to(dev).contiguous()
+        self._lenbuf = None if d["token_lens"] is None else d["token_lens"].to(dev).contiguous()
+        b = d["bm25"]
+        self.bm25 = BM25Index(b["skip"], b["postings"], b["idf"], b["df"], int(b["n_docs"]), int(b["blk_docs"]),
+                              int(b["V"]), int(b["nnz"]), float(b["k1"]), float(b["b"]), float(b["avgdl"])).to(dev)
+        self.blk_docs, self.avgdl = self.bm25.blk_docs, self.bm25.avgdl
+        if fmt == "thr-resident-v2":
+            self.n_main = int(d["n_main"])
+            self._dead = d["dead"].numpy().copy()
+            self.tag_of = dict(d["tag_of"])
+            self._df = d["df"].numpy().copy()
+            self._coo_t, self._coo_f = d["coo_t"].numpy().astype(np.int32), d["coo_f"].numpy().copy()
+            self._lens, self._row_ptr = d["lens"].numpy().copy(), d["row_ptr"].numpy().copy()
+        else:   # v1: no updates yet; the per-row terms are recovered with the tokenizer
+            self.n_main = len(self.rows)
+            self._dead = np.zeros(len(self.rows), dtype=bool)
+            self.tag_of = {c: i for i, c in enumerate(sorted({c for c in self.collections if c is not None}))}
+            self._df = self.bm25.df.cpu().numpy().astype(np.int64)
+            self._coo_t = None                     # recovered by _host_terms on the first update
+        self.id_of = {r["child_id"]: i for i, r in enumerate(self.rows) if not self._dead[i]}
+        self._tag = self._tags_of(self.collections)
+        self._publish(main=True, delta=True)
+        return self
 
     def want(self, collection: Optional[str]) -> Optional[torch.Tensor]:
         """The per-query filter argument of the tagged kernels for one query (None: no filter).  A collection no
@@ -280,49 +568,10 @@ class ResidentIndex:
             return None
         return torch.tensor([self.tag_of.get(collection, 0xfffe)], dtype=torch.int32, device=self.engine.device)
 
-    # ---- persistence (SURVEY.md 8f row 1): start a retriever without re-reading / re-embedding the corpus ----
-    def save(self, path) -> None:
-        torch.save({"format": "thr-resident-v1", "rows": self.rows, "parents": self.parents, "vocab": self.vocab,
-                    "dim": self.dim,
-                    "X": self.X.cpu(), "token_store": None if self.token_store is None else self.token_store.cpu(),
-                    "token_lens": None if self.token_lens is None else self.token_lens.cpu(),
-                    "bm25": {"skip": self.bm25.skip.cpu(), "postings": self.bm25.postings.cpu(),
-                             "idf": self.bm25.idf.cpu(), "df": self.bm25.df.cpu(), "n_docs": self.bm25.n_docs,
-                             "blk_docs": self.bm25.blk_docs, "V": self.bm25.V, "nnz": self.bm25.nnz,
-                             "k1": self.bm25.k1, "b": self.bm25.b, "avgdl": self.bm25.avgdl}}, path)
-
-    @classmethod
-    def load(cls, engine: Engine, path, tokenizer: Optional[Callable[[str], List[str]]] = None) -> "ResidentIndex":
-        """tokenizer: the callable the index was built with (callables are not persisted; default `tokenize`)."""
-        d = torch.load(path, map_location="cpu", weights_only=True)
-        if d.get("format") != "thr-resident-v1":
-            raise ValueError(f"{path}: not a ResidentIndex file")
-        self = cls.__new__(cls)
-        dev = engine.device
-        self.engine = engine
-        self.tokenizer = tokenizer or tokenize
-        self.dim = int(d.get("dim", d["X"].shape[1]))
-        self.rows = d["rows"]
-        self.id_of = {r["child_id"]: i for i, r in enumerate(self.rows)}
-        self.parents = d["parents"]
-        self.collections = [r.get("collection") for r in self.rows]
-        self.vocab = d["vocab"]
-        self.X = d["X"].to(dev).contiguous()
-        engine.dense_index_set(self.X)
-        b = d["bm25"]
-        self.bm25 = BM25Index(b["skip"], b["postings"], b["idf"], b["df"], int(b["n_docs"]), int(b["blk_docs"]),
-                              int(b["V"]), int(b["nnz"]), float(b["k1"]), float(b["b"]), float(b["avgdl"])).to(dev)
-        engine.bm25_index_set(self.bm25.skip, self.bm25.postings, self.bm25.idf, self.bm25.n_docs, self.bm25.blk_docs,
-                              self.bm25.V)
-        self.token_store = None if d["token_store"] is None else d["token_store"].to(dev).contiguous()
-        self.token_lens = None if d["token_lens"] is None else d["token_lens"].to(dev).contiguous()
-        self._set_tags()
-        return self
-
     def _rows_first(self, text: str) -> int:
-        """Row of the first chunk whose text is `text` (-1: none)."""
+        """Row of the first live chunk whose text is `text` (-1: none)."""
         for i, r in enumerate(self.rows):
-            if r.get("text", "") == text:
+            if r.get("text", "") == text and not self._dead[i]:
                 return i
         return -1
 
@@ -386,9 +635,10 @@ class _GpuScoring:
         if not terms:
             return []
         qt, qo = pack_queries([terms], eng.device)
-        ids, sc, cnt = eng.bm25_topk(qt, qo, max(1, limit), want=ix.want(collection),          # predicate inside K2
-                                     require_all=self.lexical_match == "all")
-        eng.sync()
+        with eng.lock:     # one state of the index (updates hold the same lock)
+            ids, sc, cnt = ix.bm25_topk(qt, qo, max(1, limit), want=ix.want(collection),     # predicate inside K2
+                                        require_all=self.lexical_match == "all")
+            ix.sync()
         n = int(cnt[0])
         return [ix.row_dict(i, rank=r) for i, r in zip(ids[0, :n].tolist(), sc[0, :n].tolist())]
 
@@ -402,15 +652,16 @@ class _GpuScoring:
         if q.shape[1] != ix.dim:
             raise ValueError(f"query embedding has {q.shape[1]} dimensions, the index {ix.dim}")
         q = q / q.norm(dim=1, keepdim=True).clamp_min(1e-30)
-        k = min(limit, len(ix.rows))
+        k = min(limit, ix.n_live)
         if k > 252:
             raise ValueError(f"semantic limit {limit} > 252 (K1 re-scores k + margin <= 256 survivors)")
         qd = pad_dim(q.to(torch.bfloat16)).to(eng.device)
         want = ix.want(collection)
         bound = dense_error_bound(ix.X.shape[1], 1.01, 1.01)
         for margin in (min(28, 256 - k), 256 - k):
-            ids, sc, cnt, gap = eng.dense_topk(qd, k, margin, want=want)                       # predicate inside K1
-            eng.sync()
+            with eng.lock:
+                ids, sc, cnt, gap = eng.dense_topk(qd, max(k, 1), margin, want=want)           # predicate inside K1
+                eng.sync()
             if float(gap[0]) > bound:
                 break
         else:
@@ -567,9 +818,9 @@ class _GpuScoring:
         if collections is not None and any(c is not None for c in collections):
             want = torch.tensor([-1 if c is None else ix.tag_of.get(c, 0xfffe) for c in collections], dtype=torch.int32,
                                 device=eng.device)
-        out = s.search(Q, qt, qo, g, weights=wt, k_sem=min(k_sem, len(ix.rows)), k_lex=k_lex, top_k=top_k, want=want,
-                       require_all=self.lexical_match == "all", tie_mode=tie_mode)
-        eng.sync()
+        out = s.search(Q, qt, qo, g, weights=wt, k_sem=max(1, min(k_sem, ix.n_live)), k_lex=k_lex, top_k=top_k,
+                       want=want, require_all=self.lexical_match == "all", tie_mode=tie_mode, lex_delta=ix.delta_engine)
+        ix.sync()
         ids, rrf, rk, cnt = out.ids.tolist(), out.rrf.tolist(), out.ranks.tolist(), out.count.tolist()
         res = []
         for b in range(B):
@@ -704,18 +955,21 @@ class GpuMaxSimReranker:
         self.top_k = top_k
         self.enabled = enabled
         self._rows_of_text: Optional[Dict[str, List[int]]] = None
+        self._rows_version = -1
 
     def _text_rows(self) -> Dict[str, List[int]]:
-        if self._rows_of_text is None:
+        ix = self.index
+        if self._rows_of_text is None or self._rows_version != ix.version:   # rebuilt after an update of the index
             m: Dict[str, List[int]] = {}
-            ix = self.index
-            for i, r in enumerate(ix.rows):
-                m.setdefault(r.get("text", ""), []).append(i)
-            for i, r in enumerate(ix.rows):
+            live = sorted(ix.id_of.values())
+            for i in live:
+                m.setdefault(ix.rows[i].get("text", ""), []).append(i)
+            for i in live:
+                r = ix.rows[i]
                 p = ix.parents.get(r.get("parent_id"))
                 if p is not None and p.get("text") is not None:
                     m.setdefault(p["text"], []).append(i)
-            self._rows_of_text = m
+            self._rows_of_text, self._rows_version = m, ix.version
         return self._rows_of_text
 
     def score_rows(self, query: str, rows: Sequence[int]) -> List[float]:
