@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define THR_ABI_VERSION 11
+#define THR_ABI_VERSION 12
 
 enum {
   THR_OK = 0,
@@ -266,6 +266,24 @@ int thr_safety(thr_handle* h, int B, const int32_t* off, const double* rerank,
 int thr_maxsim(thr_handle* h, const void* Qtok, const int32_t* q_len, int B, int Tq, int d,
                const void* Dtok, const int32_t* d_len, int64_t n_docs, int Td,
                const int64_t* cand, int C, float* out, void* stream);
+
+/* thr_maxsim on a residual-compressed token store (the ColBERTv2 / PLAID layout, 2-bit codes): 36 B per token
+ * instead of 256 B.  Every array is on the device; d == 128, Td in {64, 128}:
+ *   centroids bf16 [n_centroids, 128]  the codebook (16-byte aligned; read through L2)
+ *   weights   fp32 [128, 4]            weights[k, c] = reconstruction value of code c in dimension k (16-byte aligned)
+ *   cids      int32 [n_rows, Td]       centroid of each token, in [0, n_centroids)
+ *   codes     uint32 [n_rows, Td, 8]   2-bit code of dimension k = bits 2*(k % 16), 2*(k % 16) + 1 of word k / 16
+ *   d_len     int32 [n_rows], nullable tokens per row, as in thr_maxsim
+ * Token j of row r decodes to x[k] = bf16_rn(fp32(centroids[cids[r, j], k]) + weights[k, code]) (one fp32 add,
+ * round to nearest, no FMA; no renormalisation), and the score is thr_maxsim's on the decoded store: for the same
+ * inputs the outputs are bit-identical to thr_maxsim(Qtok, decode(store), ...).  Constraints are thr_maxsim's
+ * except that n_rows * Td may exceed 2^31.  A candidate < 0 or >= n_rows scores -inf.  The caller guarantees cids in
+ * range (a cid outside the table is clamped, never dereferenced).  Timed in the THR_PROF_MAXSIM slot.
+ */
+int thr_maxsim_packed(thr_handle* h, const void* Qtok, const int32_t* q_len, int B, int Tq, int d,
+                      const uint32_t* codes, const int32_t* cids, const void* centroids, int64_t n_centroids,
+                      const float* weights, const int32_t* d_len, int64_t n_rows, int Td,
+                      const int64_t* cand, int C, float* out, void* stream);
 
 /* The batched rerank stage around thr_maxsim — RAG2Retriever.retrieve steps 4-6, src/voice_agent/rag2/retrieval.py:175-191,
  * for B queries at once (the reference runs them one query at a time in Python).

@@ -18,7 +18,7 @@ THR_EINVAL, THR_ECUDA, THR_EUNSUPPORTED, THR_ENOINDEX, THR_EOVERFLOW, THR_ETIMEO
 FUSE_RAG2, FUSE_LIB, FUSE_RAG1 = 0, 1, 2
 TIE_INSERTION, TIE_CHUNK_ID = 0, 1
 BM25_REQUIRE_ALL = 1
-ABI_VERSION = 11
+ABI_VERSION = 12
 PROF_SLOTS = ("dense_score", "dense_finalize", "bm25", "fuse", "maxsim", "merge", "safety", "bm25_prep", "dense_seed", "rerank")
 
 _p, _i, _i64, _d = C.c_void_p, C.c_int, C.c_int64, C.c_double
@@ -51,6 +51,7 @@ SIGNATURES = {
     "thr_fuse_ranked": (_i, [_p, _i, _p, _p, _p, _i, _p, _p, _p]),
     "thr_safety": (_i, [_p, _i, _p, _p, _p, _p, _d, _d, _i, _p, _p, _p, _p]),
     "thr_maxsim": (_i, [_p, _p, _p, _i, _i, _i, _p, _p, _i64, _i, _p, _i, _p, _p]),
+    "thr_maxsim_packed": (_i, [_p, _p, _p, _i, _i, _i, _p, _p, _p, _i64, _p, _p, _i64, _i, _p, _i, _p, _p]),
     "thr_rerank_rows": (_i, [_p, _p, _p, _i, _i, _i, _i64, _i64, _i64, _i64, _p, _p]),
     "thr_rerank_finish": (_i, [_p, _i, _i, _i, _p, _p, _p, _p, _i, _d, _d, _i, _p, _p, _p, _p, _p, _p, _p, _p]),
     "thr_merge_topk": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _p, _p, _p, _p]),

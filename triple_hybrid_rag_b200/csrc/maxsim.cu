@@ -15,6 +15,12 @@
 // scans only a quarter (half) of the doc-token columns; partial maxima meet in shared memory.
 // The scores matrix [Tq x Td] never leaves the SM.  At Tq = 32 the kernel is HBM-bound
 // (2*Tq = 64 FLOP per byte of candidate tokens).
+//
+// maxsim_kernel<true> scores a residual-compressed store (thr_maxsim_packed, format in include/thr.h): the query
+// tile still arrives by TMA, but eight decoder warps replace the candidates' TMA loads.  They rebuild each candidate's
+// bf16 tokens (centroid row through L2 + 2-bit residual code, fp32 add, round to bf16) into the same swizzled stage
+// layout TMA writes, so the MMA and epilogue below are shared and the packed score is bit-identical to thr_maxsim on
+// the decoded store.
 #include <math_constants.h>
 
 #include "common.cuh"
@@ -25,6 +31,9 @@ constexpr int kD = 128;             // token embedding width
 constexpr int kStagesM = 5;
 constexpr int kAccM = 4;            // TMEM accumulators, 128 columns apart
 constexpr int kThreadsM = 192;      // warps 0-3 epilogue, 4 producer, 5 MMA
+constexpr int kDecGroupThreads = 128;                     // packed: one decoder group = 4 warps, fills every other stage
+constexpr int kDecGroups = 2;
+constexpr int kThreadsPacked = kThreadsM + kDecGroups * kDecGroupThreads;   // warps 6-13 decode
 constexpr int kATileBytes = 128 * kD * 2;                 // 32 KB (two 64-wide halves)
 constexpr int kMaxStageBytes = 128 * kD * 2;              // Td <= 128
 constexpr int kSmemM = kATileBytes + kStagesM * kMaxStageBytes + 1024 + 512;
@@ -40,9 +49,92 @@ struct MaxSimArgs {
   int per_slice;    // candidates per slice
   int reps;         // copies of the query tile stacked in the 128 MMA rows (4 for Tq <= 32, 2 for Tq <= 64, else 1)
   thr_dev_status* status;
+  // packed store (maxsim_kernel<true> only); n_docs is its row count
+  const uint32_t* codes;      // [n_docs, Td, 8]
+  const int32_t* cids;        // [n_docs, Td]
+  const uint4* centroids;     // [n_centroids, 128] bf16, 16 rows of 16 B per centroid
+  const float* weights;       // [128, 4]
+  int64_t n_centroids;
 };
 
-__global__ void __launch_bounds__(kThreadsM, 1)
+// Decoder group `grp` of maxsim_kernel<true>: rebuilds the candidates of stage iterations it = grp (mod kDecGroups)
+// into their ring stage, exactly as TMA would have written the decoded bf16 store (SWIZZLE_128B, K-major: 16-byte
+// chunk c of token j in chunk slot c ^ (j & 7) of the token's 128-byte row in each 64-column half).  Thread t owns
+// the 8 dimensions of 16-byte chunk q = t % 16 for every token it touches, so its 32 reconstruction values stay in
+// registers.
+__device__ __forceinline__ void maxsim_decode_stages(const MaxSimArgs& a, int grp, int t, uint32_t stage_base,
+                                                     uint32_t stage_stride, uint32_t bar_full0, uint32_t bar_empty0,
+                                                     int units) {
+  const int q = t & 15;               // chunk: dims 8q .. 8q+7, code word q / 2, bits 16 * (q & 1) + 2e
+  const int tok0 = t >> 4;            // tokens tok0, tok0 + 8, ...
+  float w0[8], w1[8], w2[8], w3[8];
+#pragma unroll
+  for (int e = 0; e < 8; ++e) {
+    const float4 v = reinterpret_cast<const float4*>(a.weights)[8 * q + e];
+    w0[e] = v.x; w1[e] = v.y; w2[e] = v.z; w3[e] = v.w;
+  }
+  const uint32_t half_bytes = (uint32_t)a.Td * 128u;
+  const uint32_t dst_q = (uint32_t)(q >> 3) * half_bytes;
+  const uint32_t cmax = (uint32_t)(a.n_centroids - 1);
+  uint32_t it = 0;
+  for (int u = blockIdx.x; u < units; u += gridDim.x) {
+    const int b = u / a.slices, sl = u % a.slices;
+    const int c_lo = sl * a.per_slice, c_hi = min(a.C, c_lo + a.per_slice);
+    for (int c = c_lo; c < c_hi; ++c, ++it) {
+      if ((int)(it % kDecGroups) != grp) continue;
+      const int s = it % kStagesM;
+      const uint32_t ph = (it / kStagesM) & 1u;
+      int64_t doc = a.cand[(size_t)b * a.C + c];
+      if (doc < 0 || doc >= a.n_docs) doc = 0;  // slot is skipped by the epilogue
+      const int64_t tok_base = doc * a.Td;      // 64-bit: the packed store has no 2^31-token limit
+      const uint32_t dst = stage_base + (uint32_t)s * stage_stride + dst_q;
+      mbar_wait_relaxed(bar_empty0 + 8u * s, ph ^ 1u, a.status, 530);
+      for (int j0 = 0; j0 < a.Td; j0 += 64) {
+        uint32_t cid[8], word[8];
+        uint4 cen[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const int64_t tok = tok_base + j0 + tok0 + 8 * i;
+          cid[i] = min((uint32_t)__ldcs(a.cids + tok), cmax);   // never dereference a cid outside the table
+          word[i] = __ldcs(a.codes + tok * 8 + (q >> 1)) >> (16 * (q & 1));
+        }
+#pragma unroll
+        for (int i = 0; i < 8; ++i) cen[i] = __ldg(a.centroids + (int64_t)cid[i] * 16 + q);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const uint32_t in[4] = {cen[i].x, cen[i].y, cen[i].z, cen[i].w};
+          uint32_t outw[4];
+#pragma unroll
+          for (int p = 0; p < 4; ++p) {
+            float x[2];
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+              const int e = 2 * p + h;
+              const uint32_t code = (word[i] >> (2 * e)) & 3u;
+              const float wv = (code & 2u) ? ((code & 1u) ? w3[e] : w2[e]) : ((code & 1u) ? w1[e] : w0[e]);
+              const float cv = __uint_as_float(h ? (in[p] & 0xffff0000u) : (in[p] << 16));
+              x[h] = __fadd_rn(cv, wv);
+            }
+            const __nv_bfloat162 r2 = __floats2bfloat162_rn(x[0], x[1]);
+            outw[p] = *reinterpret_cast<const uint32_t*>(&r2);
+          }
+          const int j = j0 + tok0 + 8 * i;
+          const uint32_t addr = dst + (uint32_t)j * 128u + ((uint32_t)((q & 7) ^ (j & 7)) << 4);
+          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(outw[0]), "r"(outw[1]),
+                       "r"(outw[2]), "r"(outw[3])
+                       : "memory");
+        }
+      }
+      fence_proxy_async_smem();   // generic-proxy stores -> visible to the tensor core's async proxy
+      mbar_arrive(bar_full0 + 8u * s);
+    }
+  }
+}
+
+// kPacked = false: candidates arrive by TMA from a bf16 store (map_d); true: decoder warps build them from the packed
+// store in `a` (map_d unused).  Everything else is one code path.
+template <bool kPacked>
+__global__ void __launch_bounds__(kPacked ? kThreadsPacked : kThreadsM, 1)
 maxsim_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_d,
               const MaxSimArgs a) {
   extern __shared__ uint8_t smem_raw[];
@@ -64,13 +156,14 @@ maxsim_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__
   const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   if (threadIdx.x == 0) {
-    for (int s = 0; s < kStagesM; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
+    // a packed stage is full once every thread of its decoder group has arrived
+    for (int s = 0; s < kStagesM; ++s) { mbar_init(full_bar(s), kPacked ? kDecGroupThreads : 1); mbar_init(empty_bar(s), 1); }
     for (int s = 0; s < kAccM; ++s) { mbar_init(tfull_bar(s), 1); mbar_init(tempty_bar(s), 1); }
     mbar_init(qfull_bar, 1);
     mbar_init(qempty_bar, 1);
     fence_mbar_init_cluster();
   }
-  if (warp == 4 && lane == 0) { tma_prefetch_desc(&map_q); tma_prefetch_desc(&map_d); }
+  if (warp == 4 && lane == 0) { tma_prefetch_desc(&map_q); if (!kPacked) tma_prefetch_desc(&map_d); }
   if (warp == 5) { tmem_alloc<1>(tmem_slot, 512); tmem_relinquish<1>(); }
   tc_fence_before_sync();
   __syncthreads();
@@ -97,16 +190,18 @@ maxsim_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__
           tma_load_2d(dst, &map_q, qfull_bar, 0, b * a.Tq, THR_L2_EVICT_LAST);
           tma_load_2d(dst + 128 * 64 * 2, &map_q, qfull_bar, 64, b * a.Tq, THR_L2_EVICT_LAST);
         }
-        for (int c = c_lo; c < c_hi; ++c, ++it) {
-          const int s = it % kStagesM;
-          const uint32_t ph = (it / kStagesM) & 1u;
-          int64_t doc = a.cand[(size_t)b * a.C + c];
-          if (doc < 0 || doc >= a.n_docs) doc = 0;  // slot is skipped by the epilogue
-          mbar_wait(empty_bar(s), ph ^ 1u, a.status, 501);
-          mbar_arrive_expect_tx(full_bar(s), stage_bytes);
-          const int32_t row = (int32_t)(doc * a.Td);
-          tma_load_2d(b_smem(s), &map_d, full_bar(s), 0, row, THR_L2_EVICT_FIRST);
-          tma_load_2d(b_smem(s) + half_bytes_b, &map_d, full_bar(s), 64, row, THR_L2_EVICT_FIRST);
+        if constexpr (!kPacked) {   // packed: the decoder warps fill the candidate stages
+          for (int c = c_lo; c < c_hi; ++c, ++it) {
+            const int s = it % kStagesM;
+            const uint32_t ph = (it / kStagesM) & 1u;
+            int64_t doc = a.cand[(size_t)b * a.C + c];
+            if (doc < 0 || doc >= a.n_docs) doc = 0;  // slot is skipped by the epilogue
+            mbar_wait(empty_bar(s), ph ^ 1u, a.status, 501);
+            mbar_arrive_expect_tx(full_bar(s), stage_bytes);
+            const int32_t row = (int32_t)(doc * a.Td);
+            tma_load_2d(b_smem(s), &map_d, full_bar(s), 0, row, THR_L2_EVICT_FIRST);
+            tma_load_2d(b_smem(s) + half_bytes_b, &map_d, full_bar(s), 64, row, THR_L2_EVICT_FIRST);
+          }
         }
       }
     }
@@ -141,6 +236,13 @@ maxsim_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__
         }
         umma_commit_1cta(qempty_bar);  // query tile reusable once this unit's MMAs are done
       }
+    }
+  } else if (warp >= 6) {
+    // ===================== decoders (packed store only) =====================
+    if constexpr (kPacked) {
+      const int t = (int)threadIdx.x - kThreadsM;
+      maxsim_decode_stages(a, t / kDecGroupThreads, t % kDecGroupThreads, b_smem(0), kMaxStageBytes, full_bar(0),
+                           empty_bar(0), units);
     }
   } else {
     // ===================== epilogue: row max over doc tokens, sum over query tokens =====================
@@ -208,6 +310,29 @@ maxsim_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__
   }
 }
 
+// Work split and launch shared by both entry points (the candidates of a query are cut into slices so that every SM
+// has units).
+template <bool kPacked>
+int maxsim_launch(thr_handle* h, const CUtensorMap& map_q, const CUtensorMap& map_d, MaxSimArgs& a, int B, int C,
+                  void* stream) {
+  a.status = h->d_status;
+  a.reps = a.Tq <= 32 ? 4 : (a.Tq <= 64 ? 2 : 1);
+  int slices = (4 * h->num_sms + B - 1) / B;
+  if (slices < 1) slices = 1;
+  if (slices > C) slices = C;
+  a.per_slice = (C + slices - 1) / slices;
+  a.slices = (C + a.per_slice - 1) / a.per_slice;
+  const int units = B * a.slices;
+  constexpr int threads = kPacked ? kThreadsPacked : kThreadsM;
+  THR_CUDA(h, cudaFuncSetAttribute(maxsim_kernel<kPacked>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemM));
+  int grid = units < h->num_sms ? units : h->num_sms;
+  const int tok = thr_prof_begin(h, THR_PROF_MAXSIM, (cudaStream_t)stream);
+  maxsim_kernel<kPacked><<<grid, threads, kSmemM, (cudaStream_t)stream>>>(map_q, map_d, a);
+  thr_prof_end(h, tok, (cudaStream_t)stream);
+  THR_CHECK_LAUNCH(h, kPacked ? "maxsim_kernel<packed>" : "maxsim_kernel");
+  return THR_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -230,23 +355,40 @@ int thr_maxsim(thr_handle* h, const void* Qtok, const int32_t* q_len, int B, int
   if (rc != THR_OK) return rc;
   rc = thr_encode_tma_2d_bf16(h, &map_d, Dtok, (uint64_t)n_docs * Td, kD, (uint32_t)Td, 64);
   if (rc != THR_OK) return rc;
-  MaxSimArgs a;
+  MaxSimArgs a = {};
   a.B = B; a.Tq = Tq; a.Td = Td; a.C = C; a.n_docs = n_docs; a.q_len = q_len; a.d_len = d_len;
-  a.cand = cand; a.out = out; a.status = h->d_status;
-  a.reps = Tq <= 32 ? 4 : (Tq <= 64 ? 2 : 1);
-  int slices = (4 * h->num_sms + B - 1) / B;
-  if (slices < 1) slices = 1;
-  if (slices > C) slices = C;
-  a.per_slice = (C + slices - 1) / slices;
-  a.slices = (C + a.per_slice - 1) / a.per_slice;
-  const int units = B * a.slices;
-  THR_CUDA(h, cudaFuncSetAttribute(maxsim_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemM));
-  int grid = units < h->num_sms ? units : h->num_sms;
-  const int tok = thr_prof_begin(h, THR_PROF_MAXSIM, (cudaStream_t)stream);
-  maxsim_kernel<<<grid, kThreadsM, kSmemM, (cudaStream_t)stream>>>(map_q, map_d, a);
-  thr_prof_end(h, tok, (cudaStream_t)stream);
-  THR_CHECK_LAUNCH(h, "maxsim_kernel");
-  return THR_OK;
+  a.cand = cand; a.out = out;
+  return maxsim_launch<false>(h, map_q, map_d, a, B, C, stream);
+}
+
+int thr_maxsim_packed(thr_handle* h, const void* Qtok, const int32_t* q_len, int B, int Tq, int d,
+                      const uint32_t* codes, const int32_t* cids, const void* centroids, int64_t n_centroids,
+                      const float* weights, const int32_t* d_len, int64_t n_rows, int Td, const int64_t* cand,
+                      int C, float* out, void* stream) {
+  if (!h) return THR_EINVAL;
+  cudaSetDevice(h->device);
+  THR_REQUIRE(h, B >= 0 && C >= 0, "thr_maxsim_packed: negative sizes");
+  if (B == 0 || C == 0) return THR_OK;
+  THR_REQUIRE(h, Qtok && codes && cids && centroids && weights && cand && out, "thr_maxsim_packed: NULL argument");
+  if (d != kD) return thr_fail(h, THR_EUNSUPPORTED, "thr_maxsim_packed: d = %d, kernels are built for d = %d", d, kD);
+  if (Td != 64 && Td != 128) return thr_fail(h, THR_EUNSUPPORTED, "thr_maxsim_packed: Td = %d must be 64 or 128", Td);
+  if (Tq < 1 || Tq > 128) return thr_fail(h, THR_EUNSUPPORTED, "thr_maxsim_packed: Tq = %d must be in [1, 128]", Tq);
+  THR_REQUIRE(h, n_rows >= 1 && n_centroids >= 1 && n_centroids <= ((int64_t)1 << 31),
+              "thr_maxsim_packed: need n_rows >= 1 and 1 <= n_centroids <= 2^31");
+  THR_REQUIRE(h, ((uintptr_t)centroids & 15) == 0 && ((uintptr_t)weights & 15) == 0 && ((uintptr_t)codes & 3) == 0 &&
+                     ((uintptr_t)cids & 3) == 0,
+              "thr_maxsim_packed: centroids and weights must be 16-byte aligned, codes and cids 4-byte aligned");
+  CUtensorMap map_q, map_unused;
+  memset(&map_unused, 0, sizeof(map_unused));
+  const uint32_t q_box_rows = Tq <= 32 ? 32u : (Tq <= 64 ? 64u : 128u);
+  int rc = thr_encode_tma_2d_bf16(h, &map_q, Qtok, (uint64_t)B * Tq, kD, q_box_rows, 64);
+  if (rc != THR_OK) return rc;
+  MaxSimArgs a = {};
+  a.B = B; a.Tq = Tq; a.Td = Td; a.C = C; a.n_docs = n_rows; a.q_len = q_len; a.d_len = d_len;
+  a.cand = cand; a.out = out;
+  a.codes = codes; a.cids = cids; a.centroids = (const uint4*)centroids; a.weights = weights;
+  a.n_centroids = n_centroids;
+  return maxsim_launch<true>(h, map_q, map_unused, a, B, C, stream);
 }
 
 }  // extern "C"

@@ -284,6 +284,35 @@ class Engine:
                                          Td, _ptr(cand), Cc, _ptr(out), self._stream()))
         return out
 
+    def maxsim_packed(self, Qtok: torch.Tensor, store, cand: torch.Tensor,
+                      q_len: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """maxsim on a residual-compressed store (tokpack.PackedTokenStore; d_len = store.lens): Qtok [B,Tq,d] bf16,
+        cand [B,C] int64 rows of the store -> scores [B,C] float32, bit-identical to maxsim on the decoded store."""
+        from .tokpack import PackedTokenStore
+        if not isinstance(store, PackedTokenStore):
+            raise TypeError("store: expected a tokpack.PackedTokenStore")
+        Qtok = self._dev(Qtok, torch.bfloat16, "Qtok")
+        cand = self._dev(cand, torch.int64, "cand")
+        centroids = self._dev(store.centroids, torch.bfloat16, "centroids")
+        weights = self._dev(store.weights, torch.float32, "weights")
+        cids = self._dev(store.cids, torch.int32, "cids")
+        codes = self._dev(store.codes, torch.int32, "codes")
+        lens = None if store.lens is None else self._dev(store.lens, torch.int32, "lens")
+        if q_len is not None:
+            q_len = self._dev(q_len, torch.int32, "q_len")
+        if Qtok.dim() != 3 or cand.dim() != 2:
+            raise ValueError("Qtok must be [B, Tq, d] and cand [B, C]")
+        B, Tq, d = Qtok.shape
+        n_rows, Td = cids.shape
+        if d != centroids.shape[1] or cand.shape[0] != B:
+            raise ValueError("shape mismatch")
+        Cc = cand.shape[1]
+        out = torch.empty((B, Cc), dtype=torch.float32, device=self.device)
+        self._check(self._lib.thr_maxsim_packed(self._h, _ptr(Qtok), _ptr(q_len), B, Tq, d, _ptr(codes), _ptr(cids),
+                                                _ptr(centroids), centroids.shape[0], _ptr(weights), _ptr(lens), n_rows,
+                                                Td, _ptr(cand), Cc, _ptr(out), self._stream()))
+        return out
+
     # -- the batched rerank stage around K4 ---------------------------------------------------
     def rerank_rows(self, ids: torch.Tensor, count: torch.Tensor, C: int, id_lo: int, id_hi: int, period: int = 0,
                     row_off: int = 0) -> torch.Tensor:

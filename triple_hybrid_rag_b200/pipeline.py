@@ -161,9 +161,18 @@ class TripleHybridSearcher:
         """This rank's late-interaction token store for the rerank stage: store [rows, Td, 128] bf16 holds the token
         embeddings of the chunks [id_lo, id_hi) this rank owns, chunk id -> row (id - id_lo + row_off), modulo `period`
         when period > 0 (synthetic stores that repeat; period == rows then, and row_off = id_lo % period makes the row a
-        function of the global id, so every sharding sees the same token embeddings for a chunk)."""
-        self.tok_store = self.engine._dev(store, torch.bfloat16, "token store")
-        self.tok_lens = None if lens is None else self.engine._dev(lens, torch.int32, "token lens")
+        function of the global id, so every sharding sees the same token embeddings for a chunk).
+        store may also be a tokpack.PackedTokenStore (residual-compressed rows of the same chunks, the codebook
+        replicated on every rank; its own lens are used, so `lens` must be None): rerank then scores with
+        maxsim_packed."""
+        from .tokpack import PackedTokenStore
+        if isinstance(store, PackedTokenStore):
+            if lens is not None:
+                raise ValueError("a packed token store carries its own lens")
+            self.tok_store, self.tok_lens = store, None
+        else:
+            self.tok_store = self.engine._dev(store, torch.bfloat16, "token store")
+            self.tok_lens = None if lens is None else self.engine._dev(lens, torch.int32, "token lens")
         self.tok_lo, self.tok_hi, self.tok_period, self.tok_off = int(id_lo), int(id_hi), int(period), int(row_off)
 
     def rerank(self, out: "SearchOutput", Qtok: torch.Tensor, C: int, threshold: float, alpha: float, final_top_k: int,
@@ -174,7 +183,10 @@ class TripleHybridSearcher:
         thr_rerank_finish orders by rerank score and applies the safety threshold / denoise on every rank."""
         eng = self.engine
         rows = eng.rerank_rows(out.ids, out.count, C, self.tok_lo, self.tok_hi, self.tok_period, self.tok_off)
-        raw = eng.maxsim(Qtok, self.tok_store, rows, q_len=q_len, d_len=self.tok_lens)
+        if isinstance(self.tok_store, torch.Tensor):
+            raw = eng.maxsim(Qtok, self.tok_store, rows, q_len=q_len, d_len=self.tok_lens)
+        else:
+            raw = eng.maxsim_packed(Qtok, self.tok_store, rows, q_len=q_len)
         if self.world > 1:
             import torch.distributed as dist
             dist.all_reduce(raw, op=dist.ReduceOp.MAX, group=self.group)

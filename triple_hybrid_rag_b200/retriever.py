@@ -39,6 +39,7 @@ import torch
 from . import _lib
 from .engine import Engine
 from .index import BM25Index, bm25_idf, pack_queries
+from .tokpack import Codebook, PackedTokenStore, encode as encode_tokens
 
 
 # ---- result / plan types: field-for-field the reference's (retrieval.py:26-63, query_planner.py:23-50) ----
@@ -235,9 +236,12 @@ class ResidentIndex:
 
     def __init__(self, engine: Engine, chunks: Sequence[Dict[str, Any]], embeddings: torch.Tensor,
                  parents: Optional[Dict[str, Dict[str, Any]]] = None, blk_docs: int = 1024,
-                 token_store: Optional[torch.Tensor] = None, token_lens: Optional[torch.Tensor] = None,
+                 token_store: Optional[torch.Tensor | PackedTokenStore] = None, token_lens: Optional[torch.Tensor] = None,
                  tokenizer: Optional[Callable[[str], List[str]]] = None, avgdl: Optional[float] = None):
         """chunks: rows with child_id, parent_id, document_id, text, page, modality (row i <-> embeddings[i]).
+        token_store: the MaxSim rerank's token rows (row i <-> chunk i): bf16 [n, Td, 128] (+ token_lens [n]), or a
+        tokpack.PackedTokenStore (residual-compressed; it carries its own lens, and its codebook stays frozen: rows
+        added later are encoded with it).
         tokenizer: str -> tokens for the lexical channel (default: `tokenize`; see Tokenizer).
         avgdl: BM25's average document length (default: the mean over these chunks)."""
         if len(chunks) != embeddings.shape[0]:
@@ -250,8 +254,15 @@ class ResidentIndex:
         self.version = 0
         self._delta_engine: Optional[Engine] = None
         dev = engine.device
-        self._build(list(chunks), self._unit_rows(embeddings).to(dev).contiguous(),
-                    None if token_store is None else token_store.to(torch.bfloat16).to(dev).contiguous(),
+        if isinstance(token_store, PackedTokenStore):
+            if token_lens is not None:
+                raise ValueError("a packed token store carries its own lens")
+            if token_store.n_rows != len(chunks):
+                raise ValueError("one token-store row per chunk")
+            token_store = token_store.to(dev)
+        elif token_store is not None:
+            token_store = token_store.to(torch.bfloat16).to(dev).contiguous()
+        self._build(list(chunks), self._unit_rows(embeddings).to(dev).contiguous(), token_store,
                     None if token_lens is None else token_lens.to(torch.int32).to(dev).contiguous(), avgdl)
 
     @staticmethod
@@ -285,7 +296,8 @@ class ResidentIndex:
         self.rows = rows
         self.id_of = {r["child_id"]: i for i, r in enumerate(rows)}
         self.collections = [r.get("collection") for r in rows]
-        self._Xbuf, self._tokbuf, self._lenbuf = X, token_store, token_lens
+        self._Xbuf = X
+        self._set_tokens(token_store, token_lens)
         self.vocab: Dict[str, int] = {}
         t, f, per_row, lens = self._tokenize(rows, self.vocab)
         self._coo_t, self._coo_f, self._lens = t, f, lens
@@ -306,6 +318,19 @@ class ResidentIndex:
         self._delta = None
         self._publish(main=True, delta=True)
 
+    def _set_tokens(self, token_store, token_lens) -> None:
+        """The row buffers of the token store that updates grow: a bf16 [N, Td, 128] tensor (+ lens), or the cids /
+        codes of a PackedTokenStore (its lens become the index's token_lens; its codebook is kept as is)."""
+        packed = isinstance(token_store, PackedTokenStore)
+        self._codebook = token_store.codebook if packed else None
+        self._tokbuf = None if packed else token_store
+        self._cidbuf, self._codebuf = (token_store.cids, token_store.codes) if packed else (None, None)
+        self._lenbuf = token_store.lens if packed else token_lens
+
+    @property
+    def _has_tokens(self) -> bool:
+        return self._tokbuf is not None or self._codebook is not None
+
     def _tags_of(self, collections) -> np.ndarray:
         """Collection names -> the uint16 tags resident next to the indexes (0xffff: none): the reference's
         `collection` predicate (20260114_rag2_schema.sql:368-370, :404-406) is evaluated inside K1 / K2."""
@@ -318,8 +343,12 @@ class ResidentIndex:
         eng, dev = self.engine, self.engine.device
         N = len(self.rows)
         self.X = self._Xbuf[:N]
-        self.token_store = None if self._tokbuf is None else self._tokbuf[:N]
         self.token_lens = None if self._lenbuf is None else self._lenbuf[:N]
+        if self._codebook is not None:
+            self.token_store = PackedTokenStore(self._codebook, self._cidbuf[:N], self._codebuf[:N], self.token_lens,
+                                                _checked=True)
+        else:
+            self.token_store = None if self._tokbuf is None else self._tokbuf[:N]
         eng.dense_index_set(self.X)        # N may have grown and the matrix moved
         if main:
             b = self.bm25
@@ -395,7 +424,8 @@ class ResidentIndex:
                    parents: Optional[Dict[str, Dict[str, Any]]] = None) -> None:
         """Append chunks (rows as in the constructor, row i <-> embeddings[i]).  A child_id already present is
         replaced: its old row is deleted and the new one appended.  With a token store, token_rows [n, Td, 128] (and
-        token_lens [n] when the store has lengths) come with them.  parents are merged into the parent map."""
+        token_lens [n] when the store has lengths) come with them; a packed store encodes them with its frozen
+        codebook.  parents are merged into the parent map."""
         chunks = list(chunks)
         n = len(chunks)
         if n != embeddings.shape[0]:
@@ -405,10 +435,14 @@ class ResidentIndex:
         ids = [r["child_id"] for r in chunks]
         if len(set(ids)) != n:
             raise ValueError("a child_id appears twice in one add_chunks call")
-        if (self._tokbuf is None) != (token_rows is None):
+        if self._has_tokens != (token_rows is not None):
             raise ValueError("token_rows must be given exactly when the index has a token store")
-        if token_rows is not None and (token_rows.shape[0] != n or token_rows.shape[1:] != self._tokbuf.shape[1:]):
-            raise ValueError(f"token_rows must be [n, {self._tokbuf.shape[1]}, {self._tokbuf.shape[2]}]")
+        if token_rows is not None:
+            Td = int((self._tokbuf if self._codebook is None else self._cidbuf).shape[1])
+            if tuple(token_rows.shape) != (n, Td, 128):
+                raise ValueError(f"token_rows must be [n, {Td}, 128]")
+            if self._codebook is not None and self._codebook.cutoffs is None:
+                raise ValueError("the packed token store's codebook has no cutoffs: new rows cannot be encoded")
         if (self._lenbuf is None) != (token_lens is None):
             raise ValueError("token_lens must be given exactly when the index has token lengths")
         if n == 0:
@@ -424,11 +458,16 @@ class ResidentIndex:
             self._host_terms()
             vocab = dict(self.vocab)
             t, f, per_row, lens = self._tokenize(chunks, vocab)
+            if self._codebook is not None:
+                enc = encode_tokens(token_rows.to(dev), None, self._codebook)
             self._kill([self.id_of[c] for c in ids if c in self.id_of])
             N = len(self.rows)
             self._Xbuf = self._grow(self._Xbuf, N, n, X)
             if self._tokbuf is not None:
                 self._tokbuf = self._grow(self._tokbuf, N, n, token_rows.to(torch.bfloat16).to(dev))
+            if self._codebook is not None:
+                self._cidbuf = self._grow(self._cidbuf, N, n, enc.cids)
+                self._codebuf = self._grow(self._codebuf, N, n, enc.codes)
             if self._lenbuf is not None:
                 self._lenbuf = self._grow(self._lenbuf, N, n, token_lens.to(torch.int32).to(dev))
             for c in sorted(new_names):   # the next free tags; existing tags never change
@@ -485,7 +524,7 @@ class ResidentIndex:
 
     def compact(self) -> None:
         """A full rebuild over the live rows: rows are renumbered (child_ids are stable), the delta segment is folded
-        in, the bitmaps are cleared and avgdl is recomputed."""
+        in, the bitmaps are cleared and avgdl is recomputed.  A packed token store keeps its codebook."""
         with self.engine.lock:
             live = np.flatnonzero(~self._dead)
             sel = torch.from_numpy(live).to(self.engine.device)
@@ -494,35 +533,47 @@ class ResidentIndex:
             if self._delta_engine is not None:      # no delta after a full build: free its handle and index
                 self._delta_engine.close()
                 self._delta_engine = self._delta = None
-            self._build([self.rows[i] for i in live], self._Xbuf[:N][sel].contiguous(),
-                        None if self._tokbuf is None else self._tokbuf[:N][sel].contiguous(),
-                        None if self._lenbuf is None else self._lenbuf[:N][sel].contiguous(), None)
+            if self._codebook is not None:
+                tok, lens = self.token_store.select(sel), None
+            else:
+                tok = None if self._tokbuf is None else self._tokbuf[:N][sel].contiguous()
+                lens = None if self._lenbuf is None else self._lenbuf[:N][sel].contiguous()
+            self._build([self.rows[i] for i in live], self._Xbuf[:N][sel].contiguous(), tok, lens, None)
 
     # ---- persistence (SURVEY.md 8f row 1): start a retriever without re-reading / re-embedding the corpus ----
     def save(self, path) -> None:
-        """thr-resident-v2: the v1 content plus the update state (deletion mask, appended rows, frozen avgdl, tags)."""
+        """thr-resident-v2: the v1 content plus the update state (deletion mask, appended rows, frozen avgdl, tags).
+        An index with a packed token store is written as thr-resident-v3: v2 plus `packed_store` (codebook, cids,
+        codes; its lens are `token_lens`)."""
         self._host_terms()
         b = self.bm25
-        torch.save({"format": "thr-resident-v2", "rows": self.rows, "parents": self.parents, "vocab": self.vocab,
-                    "dim": self.dim,
-                    "X": self.X.cpu(), "token_store": None if self.token_store is None else self.token_store.cpu(),
-                    "token_lens": None if self.token_lens is None else self.token_lens.cpu(),
-                    "bm25": {"skip": b.skip.cpu(), "postings": b.postings.cpu(),
-                             "idf": b.idf.cpu(), "df": b.df.cpu(), "n_docs": b.n_docs,
-                             "blk_docs": b.blk_docs, "V": b.V, "nnz": b.nnz,
-                             "k1": b.k1, "b": b.b, "avgdl": b.avgdl},
-                    "n_main": self.n_main, "dead": torch.from_numpy(self._dead.copy()), "tag_of": self.tag_of,
-                    "df": torch.from_numpy(self._df.copy()), "coo_t": torch.from_numpy(self._coo_t),
-                    "coo_f": torch.from_numpy(self._coo_f), "lens": torch.from_numpy(self._lens),
-                    "row_ptr": torch.from_numpy(self._row_ptr.astype(np.int64))}, path)
+        packed = self._codebook is not None
+        d = {"format": "thr-resident-v3" if packed else "thr-resident-v2", "rows": self.rows, "parents": self.parents,
+             "vocab": self.vocab, "dim": self.dim,
+             "X": self.X.cpu(), "token_store": None if packed or self.token_store is None else self.token_store.cpu(),
+             "token_lens": None if self.token_lens is None else self.token_lens.cpu(),
+             "bm25": {"skip": b.skip.cpu(), "postings": b.postings.cpu(),
+                      "idf": b.idf.cpu(), "df": b.df.cpu(), "n_docs": b.n_docs,
+                      "blk_docs": b.blk_docs, "V": b.V, "nnz": b.nnz,
+                      "k1": b.k1, "b": b.b, "avgdl": b.avgdl},
+             "n_main": self.n_main, "dead": torch.from_numpy(self._dead.copy()), "tag_of": self.tag_of,
+             "df": torch.from_numpy(self._df.copy()), "coo_t": torch.from_numpy(self._coo_t),
+             "coo_f": torch.from_numpy(self._coo_f), "lens": torch.from_numpy(self._lens),
+             "row_ptr": torch.from_numpy(self._row_ptr.astype(np.int64))}
+        if packed:
+            cb, st = self._codebook, self.token_store
+            d["packed_store"] = {"centroids": cb.centroids.cpu(), "weights": cb.weights.cpu(),
+                                 "cutoffs": None if cb.cutoffs is None else cb.cutoffs.cpu(),
+                                 "cids": st.cids.cpu(), "codes": st.codes.cpu()}
+        torch.save(d, path)
 
     @classmethod
     def load(cls, engine: Engine, path, tokenizer: Optional[Callable[[str], List[str]]] = None) -> "ResidentIndex":
         """tokenizer: the callable the index was built with (callables are not persisted; default `tokenize`).
-        Reads thr-resident-v2 and v1 files."""
+        Reads thr-resident-v3, v2 and v1 files."""
         d = torch.load(path, map_location="cpu", weights_only=True)
         fmt = d.get("format")
-        if fmt not in ("thr-resident-v1", "thr-resident-v2"):
+        if fmt not in ("thr-resident-v1", "thr-resident-v2", "thr-resident-v3"):
             raise ValueError(f"{path}: not a ResidentIndex file")
         self = cls.__new__(cls)
         dev = engine.device
@@ -537,13 +588,19 @@ class ResidentIndex:
         self.collections = [r.get("collection") for r in self.rows]
         self.vocab = d["vocab"]
         self._Xbuf = d["X"].to(dev).contiguous()
-        self._tokbuf = None if d["token_store"] is None else d["token_store"].to(dev).contiguous()
-        self._lenbuf = None if d["token_lens"] is None else d["token_lens"].to(dev).contiguous()
+        lens = None if d["token_lens"] is None else d["token_lens"].to(dev).contiguous()
+        if fmt == "thr-resident-v3":
+            p = d["packed_store"]
+            tok = PackedTokenStore(Codebook(p["centroids"], p["weights"], p["cutoffs"]), p["cids"], p["codes"],
+                                   None if lens is None else lens.cpu()).to(dev)
+        else:
+            tok = None if d["token_store"] is None else d["token_store"].to(dev).contiguous()
+        self._set_tokens(tok, lens)
         b = d["bm25"]
         self.bm25 = BM25Index(b["skip"], b["postings"], b["idf"], b["df"], int(b["n_docs"]), int(b["blk_docs"]),
                               int(b["V"]), int(b["nnz"]), float(b["k1"]), float(b["b"]), float(b["avgdl"])).to(dev)
         self.blk_docs, self.avgdl = self.bm25.blk_docs, self.bm25.avgdl
-        if fmt == "thr-resident-v2":
+        if fmt != "thr-resident-v1":
             self.n_main = int(d["n_main"])
             self._dead = d["dead"].numpy().copy()
             self.tag_of = dict(d["tag_of"])
@@ -985,7 +1042,10 @@ class GpuMaxSimReranker:
         qtok = qtok / qtok.norm(dim=-1, keepdim=True).clamp_min(1e-30)
         qtok = qtok.to(torch.bfloat16).to(eng.device).unsqueeze(0).contiguous()
         cand = torch.tensor([list(rows)], dtype=torch.int64, device=eng.device)
-        raw = eng.maxsim(qtok, ix.token_store, cand, d_len=ix.token_lens)
+        if isinstance(ix.token_store, PackedTokenStore):
+            raw = eng.maxsim_packed(qtok, ix.token_store, cand)
+        else:
+            raw = eng.maxsim(qtok, ix.token_store, cand, d_len=ix.token_lens)
         eng.sync()
         tq = qtok.shape[1]
         return [0.5 if r < 0 else min(1.0, max(0.0, 0.5 * (float(s) / tq + 1.0))) for r, s in zip(rows, raw[0].tolist())]
