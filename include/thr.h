@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define THR_ABI_VERSION 12
+#define THR_ABI_VERSION 13
 
 enum {
   THR_OK = 0,
@@ -66,6 +66,10 @@ const char* thr_last_error(const thr_handle* h);
 int thr_sync(thr_handle* h, void* stream);
 /* Number of kernels this handle has launched since creation (bench.py's gpu_launches). */
 int64_t thr_launch_count(const thr_handle* h);
+/* Let kernels launched through `h` read memory of `peer_device` (cudaDeviceCanAccessPeer, then
+ * cudaDeviceEnablePeerAccess in the handle's device context; a runtime setting of this process only).  Already
+ * enabled, or peer_device == the handle's device: THR_OK.  THR_EUNSUPPORTED when the pair cannot peer. */
+int thr_peer_enable(thr_handle* h, int peer_device);
 
 /* Per-kernel device timing.  When enabled, every kernel launch is bracketed by CUDA events on the
  * launch stream; thr_prof_read synchronises the device, adds up the elapsed times recorded for
@@ -356,6 +360,35 @@ int thr_exchange_push(thr_handle* h, const int64_t* d_ids, const double* d_sc, c
 int thr_exchange_merge_pushed(thr_handle* h, const void* gathered, const uint64_t* signals, uint64_t seq,
                               int G, int B, int k_sem, int k_lex, int64_t* d_ids, double* d_sc,
                               int32_t* d_cnt, int64_t* l_ids, float* l_sc, int32_t* l_cnt, void* stream);
+
+/* ---- in-process sharding: one index over several handles (ShardedSearcher) -------------
+ * thr_shard_merge: the merge step of a sharded search in ONE process, without a message: the home handle reads every
+ * shard's K1 / K2 outputs where they are (peer memory, or local copies) through device arrays of pointers:
+ *   semantic sources s < S_sem: d_ids_src[s] [B, k_sem] int64, d_sc_src[s] [B, k_sem] double, d_cnt_src[s] [B] int32,
+ *     d_gap_src[s] [B] float (nullable table when d_gap is NULL) — thr_dense_topk outputs;
+ *   lexical sources s < S_lex: l_ids_src[s] [B, k_lex] int64, l_sc_src[s] [B, k_lex] float, l_cnt_src[s] [B] int32 —
+ *     thr_bm25_topk outputs (a shard with a lexical delta segment contributes two sources).
+ * Outputs, on the handle's GPU, are both channels' merged lists in exactly the formats thr_dense_topk /
+ * thr_bm25_topk write (thr_fuse runs on them unchanged), ordered by (score desc, id asc), placed by rank as
+ * thr_exchange_merge does; d_gap [B] (nullable) = min over the semantic sources' gaps, the certificate of the merged
+ * list (the global top-k is a subset of the union of exact per-shard top-k lists).  One launch for both channels;
+ * each row's lists are staged in shared memory with coalesced loads before any search.
+ * 1 <= S_sem, S_lex <= 64, 1 <= k <= 256; THR_EUNSUPPORTED when S * k of a channel exceeds 12288.  Timed in the
+ * THR_PROF_MERGE slot.
+ *
+ * thr_rerank_finish_shards: thr_rerank_finish on the element-wise max of S raw [B, C] float arrays (raws: device
+ * array of S pointers; exactly one shard scores a candidate, the others report -inf).  S == 1 is bit-identical to
+ * thr_rerank_finish.  Replaces the all-reduce(MAX) of the multi-process stage.  Timed in THR_PROF_RERANK.
+ */
+int thr_shard_merge(thr_handle* h, int B, int k_sem, int k_lex, int S_sem, const int64_t* const* d_ids_src,
+                    const double* const* d_sc_src, const int32_t* const* d_cnt_src, const float* const* d_gap_src,
+                    int S_lex, const int64_t* const* l_ids_src, const float* const* l_sc_src,
+                    const int32_t* const* l_cnt_src, int64_t* d_ids, double* d_sc, int32_t* d_cnt, float* d_gap,
+                    int64_t* l_ids, float* l_sc, int32_t* l_cnt, void* stream);
+int thr_rerank_finish_shards(thr_handle* h, int B, int C, int stride, const int64_t* ids, const double* rrf,
+                             const int32_t* count, const float* const* raws, int S, int Tq, double threshold,
+                             double alpha, int top_k, int64_t* out_ids, double* out_rerank, double* out_rrf,
+                             uint8_t* out_keep, int32_t* out_n, uint8_t* refused, double* max_score, void* stream);
 
 #ifdef __cplusplus
 }

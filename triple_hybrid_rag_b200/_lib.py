@@ -18,7 +18,7 @@ THR_EINVAL, THR_ECUDA, THR_EUNSUPPORTED, THR_ENOINDEX, THR_EOVERFLOW, THR_ETIMEO
 FUSE_RAG2, FUSE_LIB, FUSE_RAG1 = 0, 1, 2
 TIE_INSERTION, TIE_CHUNK_ID = 0, 1
 BM25_REQUIRE_ALL = 1
-ABI_VERSION = 12
+ABI_VERSION = 13
 PROF_SLOTS = ("dense_score", "dense_finalize", "bm25", "fuse", "maxsim", "merge", "safety", "bm25_prep", "dense_seed", "rerank")
 
 _p, _i, _i64, _d = C.c_void_p, C.c_int, C.c_int64, C.c_double
@@ -31,6 +31,7 @@ SIGNATURES = {
     "thr_last_error": (C.c_char_p, [_p]),
     "thr_sync": (_i, [_p, _p]),
     "thr_launch_count": (_i64, [_p]),
+    "thr_peer_enable": (_i, [_p, _i]),
     "thr_prof_enable": (_i, [_p, _i]),
     "thr_prof_select": (_i, [_p, C.c_uint]),
     "thr_prof_reset": (_i, [_p]),
@@ -60,6 +61,9 @@ SIGNATURES = {
     "thr_exchange_merge": (_i, [_p, _p, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p]),
     "thr_exchange_push": (_i, [_p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p, _i64, _p, _i64, _i, _i, C.c_uint64, _p, _p]),
     "thr_exchange_merge_pushed": (_i, [_p, _p, _p, C.c_uint64, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p]),
+    "thr_shard_merge": (_i, [_p, _i, _i, _i, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
+    "thr_rerank_finish_shards": (_i, [_p, _i, _i, _i, _p, _p, _p, _p, _i, _i, _d, _d, _i, _p, _p, _p, _p, _p, _p, _p,
+                                      _p]),
 }
 
 _lib = None

@@ -190,6 +190,28 @@ const char* thr_last_error(const thr_handle* h) { return h ? h->err : g_create_e
 
 int64_t thr_launch_count(const thr_handle* h) { return h ? h->launches : 0; }
 
+int thr_peer_enable(thr_handle* h, int peer_device) {
+  if (!h) return THR_EINVAL;
+  THR_CUDA(h, cudaSetDevice(h->device));
+  int count = 0;
+  THR_CUDA(h, cudaGetDeviceCount(&count));
+  THR_REQUIRE(h, peer_device >= 0 && peer_device < count, "thr_peer_enable: device %d out of range [0,%d)", peer_device, count);
+  if (peer_device == h->device) return THR_OK;
+  int can = 0;
+  THR_CUDA(h, cudaDeviceCanAccessPeer(&can, h->device, peer_device));
+  if (!can)
+    return thr_fail(h, THR_EUNSUPPORTED, "thr_peer_enable: device %d cannot access device %d", h->device, peer_device);
+  const cudaError_t e = cudaDeviceEnablePeerAccess(peer_device, 0);
+  if (e == cudaErrorPeerAccessAlreadyEnabled) {
+    cudaGetLastError();   // clear the sticky-free "already enabled" status: it is success here
+    return THR_OK;
+  }
+  if (e != cudaSuccess)
+    return thr_fail(h, THR_ECUDA, "cudaDeviceEnablePeerAccess(%d) on device %d: %s", peer_device, h->device,
+                    cudaGetErrorString(e));
+  return THR_OK;
+}
+
 int thr_sync(thr_handle* h, void* stream) {
   if (!h) return THR_EINVAL;
   cudaSetDevice(h->device);

@@ -534,6 +534,71 @@ __global__ void __launch_bounds__(256) exchange_push_kernel(const int64_t* d_ids
   }
 }
 
+// The merge step of K5's exchange and of thr_shard_merge: one CTA holds one (channel, query) row's G lists in shared
+// memory (list g at s_sc + g * k / s_id + g * k, its first s_cnt[g] <= k entries valid), each sorted by (score desc, id
+// asc), and writes the channel's merged list in the channel's own output format (semantic: f64 scores, -inf padding;
+// lexical: f32 scores, 0 padding as thr_bm25_topk writes them).  Rows [0, B) are semantic, [B, 2B) lexical.
+// Every list is sorted already: merge by RANK instead of sorting — an entry's place in the merged list is its place in
+// its own list plus, for every other list, the number of entries that precede it there (a binary search).  No
+// exchange network, no barrier between the staging and the output.
+__device__ __forceinline__ void merge_staged_write(const double* s_sc, const int64_t* s_id, const int* s_cnt, int G,
+                                                  int k, int row, int B, int k_sem, int k_lex, int64_t* d_ids,
+                                                  double* d_sc, int32_t* d_cnt, int64_t* l_ids, float* l_sc,
+                                                  int32_t* l_cnt) {
+  const int n = G * k;
+  int total = 0;
+  for (int g = 0; g < G; ++g) total += s_cnt[g];
+  const int k_out = row < B ? k_sem : k_lex;
+  const int nout = min(total, k_out);
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    const int g = i / k, j = i - g * k;
+    if (j >= s_cnt[g] || j >= nout) continue;   // an entry's merged place is at least its place in its own list
+    const double s = s_sc[i];
+    const int64_t id = s_id[i];
+    int rank = j;
+    for (int g2 = 0; g2 < G && rank < nout; ++g2) {
+      if (g2 == g) continue;
+      // entries of list g2 that precede (s, id); equal (score, id) pairs cannot come from two lists of a sharded
+      // corpus — if they ever do, the lower list goes first, so the merged places stay a permutation
+      int lo = 0, hi = s_cnt[g2];
+      const double* sc2 = s_sc + g2 * k;
+      const int64_t* id2 = s_id + g2 * k;
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        const double sm = sc2[mid];
+        const int64_t im = id2[mid];
+        const bool before = sm > s || (sm == s && (im < id || (im == id && g2 < g)));
+        if (before) lo = mid + 1; else hi = mid;
+      }
+      rank += lo;
+    }
+    if (rank < nout) {
+      if (row < B) {
+        d_sc[(size_t)row * k_sem + rank] = s;
+        d_ids[(size_t)row * k_sem + rank] = id;
+      } else {
+        const int q = row - B;
+        l_sc[(size_t)q * k_lex + rank] = (float)s;
+        l_ids[(size_t)q * k_lex + rank] = id;
+      }
+    }
+  }
+  if (row < B) {
+    if (threadIdx.x == 0) d_cnt[row] = nout;
+    for (int i = nout + threadIdx.x; i < k_sem; i += blockDim.x) {
+      d_sc[(size_t)row * k_sem + i] = -INFINITY;
+      d_ids[(size_t)row * k_sem + i] = -1;
+    }
+  } else {
+    const int q = row - B;
+    if (threadIdx.x == 0) l_cnt[q] = nout;
+    for (int i = nout + threadIdx.x; i < k_lex; i += blockDim.x) {
+      l_sc[(size_t)q * k_lex + i] = 0.f;
+      l_ids[(size_t)q * k_lex + i] = -1;
+    }
+  }
+}
+
 // One CTA per (channel, query): merge the G lists out of the gathered messages, write the channel's final list in
 // the channel's own output format (semantic: f64 scores, -inf padding; lexical: f32 scores, 0 padding as
 // thr_bm25_topk writes them).
@@ -585,59 +650,55 @@ __global__ void __launch_bounds__(256) exchange_merge_kernel(const uint8_t* gath
     }
   }
   __syncthreads();
-  int total = 0;
-  for (int g = 0; g < G; ++g) total += s_cnt[g];
-  const int k_out = row < B ? k_sem : k_lex;
-  const int nout = min(total, k_out);
-  for (int i = tid; i < n; i += 256) {
-    const int g = i / k, j = i - g * k;
-    if (j >= s_cnt[g] || j >= nout) continue;   // an entry's merged place is at least its place in its own list
-    const double s = s_sc[i];
-    const int64_t id = s_id[i];
-    int rank = j;
-    for (int g2 = 0; g2 < G && rank < nout; ++g2) {
-      if (g2 == g) continue;
-      // entries of list g2 that precede (s, id); equal (score, id) pairs cannot come from two ranks of a sharded
-      // corpus — if they ever do, the lower rank goes first, so the merged places stay a permutation
-      int lo = 0, hi = s_cnt[g2];
-      const double* sc2 = s_sc + g2 * k;
-      const int64_t* id2 = s_id + g2 * k;
-      while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        const double sm = sc2[mid];
-        const int64_t im = id2[mid];
-        const bool before = sm > s || (sm == s && (im < id || (im == id && g2 < g)));
-        if (before) lo = mid + 1; else hi = mid;
-      }
-      rank += lo;
-    }
-    if (rank < nout) {
-      if (row < B) {
-        d_sc[(size_t)row * k_sem + rank] = s;
-        d_ids[(size_t)row * k_sem + rank] = id;
-      } else {
-        const int q = row - B;
-        l_sc[(size_t)q * k_lex + rank] = (float)s;
-        l_ids[(size_t)q * k_lex + rank] = id;
-      }
-    }
-  }
-  if (row < B) {
-    if (tid == 0) d_cnt[row] = nout;
-    for (int i = nout + tid; i < k_sem; i += 256) {
-      d_sc[(size_t)row * k_sem + i] = -INFINITY;
-      d_ids[(size_t)row * k_sem + i] = -1;
-    }
-  } else {
-    const int q = row - B;
-    if (tid == 0) l_cnt[q] = nout;
-    for (int i = nout + tid; i < k_lex; i += 256) {
-      l_sc[(size_t)q * k_lex + i] = 0.f;
-      l_ids[(size_t)q * k_lex + i] = -1;
-    }
-  }
+  merge_staged_write(s_sc, s_id, s_cnt, G, k, row, B, k_sem, k_lex, d_ids, d_sc, d_cnt, l_ids, l_sc, l_cnt);
 }
 
+// thr_shard_merge: one CTA per (channel, query) row.  The sources are other handles' K1 / K2 outputs, possibly on other
+// GPUs (every load a peer round trip), so the row's S lists are first staged into shared memory with coalesced loads
+// (one pass over counts, one over entries, lexical f32 scores widened to f64 exactly); the binary searches of the
+// rank merge then run on shared memory only.  Dynamic shared memory: S_max * k * 16 bytes.
+constexpr int kShardMergeMax = 12288;   // entries staged per row: 192 KB of shared memory
+struct ShardSources {
+  const int64_t* const* d_ids; const double* const* d_sc; const int32_t* const* d_cnt; const float* const* d_gap;
+  const int64_t* const* l_ids; const float* const* l_sc; const int32_t* const* l_cnt;
+  int S_sem, S_lex;
+};
+
+__global__ void __launch_bounds__(256) shard_merge_kernel(const ShardSources src, int B, int k_sem, int k_lex,
+                                                          int64_t* d_ids, double* d_sc, int32_t* d_cnt, float* d_gap,
+                                                          int64_t* l_ids, float* l_sc, int32_t* l_cnt) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  __shared__ int s_cnt[64];
+  const int row = blockIdx.x, tid = threadIdx.x;
+  const bool sem = row < B;
+  const int q = sem ? row : row - B;
+  const int S = sem ? src.S_sem : src.S_lex;
+  const int k = sem ? k_sem : k_lex;
+  double* s_sc = (double*)smem;
+  int64_t* s_id = (int64_t*)(smem + (size_t)S * k * sizeof(double));
+  __shared__ float s_gap[64];
+  if (tid < S) {
+    s_cnt[tid] = min(max(sem ? src.d_cnt[tid][q] : src.l_cnt[tid][q], 0), k);
+    if (sem && d_gap) s_gap[tid] = src.d_gap[tid][q];
+  }
+  __syncthreads();
+  if (sem && d_gap && tid == 0) {   // certificate of the merged list: if every source's top-k is exact, so is theirs
+    float g = INFINITY;
+    for (int s = 0; s < S; ++s) g = fminf(g, s_gap[s]);
+    d_gap[q] = g;
+  }
+  const int n = S * k;
+  for (int i = tid; i < n; i += blockDim.x) {
+    const int g = i / k, j = i - g * k;
+    if (j < s_cnt[g]) {
+      const size_t o = (size_t)q * k + j;
+      s_sc[i] = sem ? src.d_sc[g][o] : (double)src.l_sc[g][o];
+      s_id[i] = sem ? src.d_ids[g][o] : src.l_ids[g][o];
+    }
+  }
+  __syncthreads();
+  merge_staged_write(s_sc, s_id, s_cnt, S, k, row, B, k_sem, k_lex, d_ids, d_sc, d_cnt, l_ids, l_sc, l_cnt);
+}
 }  // namespace
 
 extern "C" {
@@ -810,5 +871,35 @@ int thr_exchange_push(thr_handle* h, const int64_t* d_ids, const double* d_sc, c
   return THR_OK;
 }
 
+
+int thr_shard_merge(thr_handle* h, int B, int k_sem, int k_lex, int S_sem, const int64_t* const* d_ids_src,
+                    const double* const* d_sc_src, const int32_t* const* d_cnt_src, const float* const* d_gap_src,
+                    int S_lex, const int64_t* const* l_ids_src, const float* const* l_sc_src,
+                    const int32_t* const* l_cnt_src, int64_t* d_ids, double* d_sc, int32_t* d_cnt, float* d_gap,
+                    int64_t* l_ids, float* l_sc, int32_t* l_cnt, void* stream) {
+  if (!h) return THR_EINVAL;
+  cudaSetDevice(h->device);
+  THR_REQUIRE(h, B >= 0 && k_sem >= 1 && k_lex >= 1 && k_sem <= 256 && k_lex <= 256,
+              "thr_shard_merge: need 1 <= k_sem, k_lex <= 256");
+  THR_REQUIRE(h, S_sem >= 1 && S_sem <= 64 && S_lex >= 1 && S_lex <= 64, "thr_shard_merge: need 1 <= S <= 64 per channel");
+  if (B == 0) return THR_OK;
+  const int64_t n_max = (int64_t)S_sem * k_sem > (int64_t)S_lex * k_lex ? (int64_t)S_sem * k_sem : (int64_t)S_lex * k_lex;
+  if (n_max > kShardMergeMax)
+    return thr_fail(h, THR_EUNSUPPORTED, "thr_shard_merge: S * k = %lld exceeds %d", (long long)n_max, kShardMergeMax);
+  THR_REQUIRE(h, d_ids_src && d_sc_src && d_cnt_src && l_ids_src && l_sc_src && l_cnt_src && d_ids && d_sc && d_cnt &&
+                     l_ids && l_sc && l_cnt && (d_gap == nullptr || d_gap_src != nullptr),
+              "thr_shard_merge: NULL argument");
+  const size_t smem = (size_t)n_max * 16;
+  THR_CUDA(h, cudaFuncSetAttribute(shard_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  ShardSources src;
+  src.d_ids = d_ids_src; src.d_sc = d_sc_src; src.d_cnt = d_cnt_src; src.d_gap = d_gap_src;
+  src.l_ids = l_ids_src; src.l_sc = l_sc_src; src.l_cnt = l_cnt_src; src.S_sem = S_sem; src.S_lex = S_lex;
+  const int tok = thr_prof_begin(h, THR_PROF_MERGE, (cudaStream_t)stream);
+  shard_merge_kernel<<<2 * B, 256, smem, (cudaStream_t)stream>>>(src, B, k_sem, k_lex, d_ids, d_sc, d_cnt, d_gap, l_ids,
+                                                                 l_sc, l_cnt);
+  thr_prof_end(h, tok, (cudaStream_t)stream);
+  THR_CHECK_LAUNCH(h, "shard_merge_kernel");
+  return THR_OK;
+}
 
 }  // extern "C"

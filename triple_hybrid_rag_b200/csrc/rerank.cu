@@ -7,7 +7,8 @@
 // keeps what clears the threshold.  The reference does this one query at a time in Python; here one CTA per query.
 // With a sharded corpus each rank scores the candidates whose chunks it owns (rerank_rows_kernel maps the others to
 // -1, which thr_maxsim scores -inf), the ranks exchange the [B, C] score matrix with ONE all-reduce(MAX), and this
-// kernel runs replicated on the merged scores.
+// kernel runs replicated on the merged scores.  In one process (thr_rerank_finish_shards) the kernel takes the element-
+// wise max of the shards' [B, C] arrays itself, read through peer memory.
 #include <math_constants.h>
 
 #include "common.cuh"
@@ -35,6 +36,8 @@ struct FinishArgs {
   const double* rrf;       // [B, stride]
   const int32_t* count;    // [B]
   const float* raw;        // [B, C] MaxSim sums; -inf = nobody scored the candidate
+  const float* const* raws;  // or (raw == nullptr) n_raw such arrays, one per shard: their element-wise max
+  int n_raw;
   double threshold, alpha;
   int64_t* out_ids;        // [B, C] in the reranked order, -1 padded
   double* out_rerank;      // [B, C] rerank_score in [0, 1] (-1 where the candidate has none)
@@ -50,14 +53,27 @@ __global__ void __launch_bounds__(kRerankMaxC) rerank_finish_kernel(const Finish
   __shared__ int s_pos[kRerankMaxC];
   __shared__ double s_red[kRerankMaxC / 32];
   __shared__ int s_cnt[kRerankMaxC / 32];
+  __shared__ float s_raw[kRerankMaxC];
   const int q = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int n = min(min(a.count[q], a.C), kRerankMaxC);
+  // the candidate's raw score, read once (coalesced; the shards' arrays may be in peer memory)
+  if (tid < n) {
+    const size_t o = (size_t)q * a.C + tid;
+    float r;
+    if (a.raw) {
+      r = a.raw[o];
+    } else {
+      r = a.raws[0][o];
+      for (int s = 1; s < a.n_raw; ++s) r = fmaxf(r, a.raws[s][o]);
+    }
+    s_raw[tid] = r;
+  }
   // rerank_score = min(1, max(0, 0.5 * (s / Tq + 1))) in fp64, one rounded operation at a time (the Python of
   // GpuMaxSimReranker.score_rows); a candidate nobody scored has none.
   double score = -1.0;
   bool has = false;
   if (tid < n) {
-    const float r = a.raw[(size_t)q * a.C + tid];
+    const float r = s_raw[tid];
     if (r > -CUDART_INF_F) {
       has = true;
       double x = __dmul_rn(0.5, __dadd_rn(__ddiv_rn((double)r, (double)a.Tq), 1.0));
@@ -88,7 +104,7 @@ __global__ void __launch_bounds__(kRerankMaxC) rerank_finish_kernel(const Finish
   bool hs = false;
   int64_t id = -1;
   if (tid < n) {
-    const float r = a.raw[(size_t)q * a.C + src];
+    const float r = s_raw[src];
     if (r > -CUDART_INF_F) {
       hs = true;
       sc = fmin(1.0, fmax(0.0, __dmul_rn(0.5, __dadd_rn(__ddiv_rn((double)r, (double)a.Tq), 1.0))));
@@ -144,18 +160,20 @@ int thr_rerank_rows(thr_handle* h, const int64_t* ids, const int32_t* count, int
   return THR_OK;
 }
 
-int thr_rerank_finish(thr_handle* h, int B, int C, int stride, const int64_t* ids, const double* rrf,
-                      const int32_t* count, const float* raw, int Tq, double threshold, double alpha, int top_k,
-                      int64_t* out_ids, double* out_rerank, double* out_rrf, uint8_t* out_keep, int32_t* out_n,
-                      uint8_t* refused, double* max_score, void* stream) {
+static int rerank_finish_launch(thr_handle* h, const char* name, int B, int C, int stride, const int64_t* ids,
+                                const double* rrf, const int32_t* count, const float* raw, const float* const* raws,
+                                int n_raw, int Tq, double threshold, double alpha, int top_k, int64_t* out_ids,
+                                double* out_rerank, double* out_rrf, uint8_t* out_keep, int32_t* out_n, uint8_t* refused,
+                                double* max_score, void* stream) {
   if (!h) return THR_EINVAL;
   cudaSetDevice(h->device);
-  THR_REQUIRE(h, B >= 0 && C >= 1 && C <= kRerankMaxC && stride >= C && Tq >= 1, "thr_rerank_finish: need 1 <= C <= %d, stride >= C, Tq >= 1", kRerankMaxC);
+  THR_REQUIRE(h, B >= 0 && C >= 1 && C <= kRerankMaxC && stride >= C && Tq >= 1, "%s: need 1 <= C <= %d, stride >= C, Tq >= 1", name, kRerankMaxC);
   if (B == 0) return THR_OK;
-  THR_REQUIRE(h, ids && rrf && count && raw && out_ids && out_rerank && out_rrf && out_keep && out_n && refused && max_score,
-              "thr_rerank_finish: NULL argument");
+  THR_REQUIRE(h, ids && rrf && count && (raw || raws) && out_ids && out_rerank && out_rrf && out_keep && out_n && refused && max_score,
+              "%s: NULL argument", name);
   FinishArgs a;
   a.B = B; a.C = C; a.stride = stride; a.Tq = Tq; a.top_k = top_k; a.ids = ids; a.rrf = rrf; a.count = count; a.raw = raw;
+  a.raws = raws; a.n_raw = n_raw;
   a.threshold = threshold; a.alpha = alpha; a.out_ids = out_ids; a.out_rerank = out_rerank; a.out_rrf = out_rrf;
   a.out_keep = out_keep; a.out_n = out_n; a.refused = refused; a.max_score = max_score;
   const int tok = thr_prof_begin(h, THR_PROF_RERANK, (cudaStream_t)stream);
@@ -163,6 +181,23 @@ int thr_rerank_finish(thr_handle* h, int B, int C, int stride, const int64_t* id
   thr_prof_end(h, tok, (cudaStream_t)stream);
   THR_CHECK_LAUNCH(h, "rerank_finish_kernel");
   return THR_OK;
+}
+
+int thr_rerank_finish(thr_handle* h, int B, int C, int stride, const int64_t* ids, const double* rrf,
+                      const int32_t* count, const float* raw, int Tq, double threshold, double alpha, int top_k,
+                      int64_t* out_ids, double* out_rerank, double* out_rrf, uint8_t* out_keep, int32_t* out_n,
+                      uint8_t* refused, double* max_score, void* stream) {
+  return rerank_finish_launch(h, "thr_rerank_finish", B, C, stride, ids, rrf, count, raw, nullptr, 0, Tq, threshold, alpha,
+                              top_k, out_ids, out_rerank, out_rrf, out_keep, out_n, refused, max_score, stream);
+}
+
+int thr_rerank_finish_shards(thr_handle* h, int B, int C, int stride, const int64_t* ids, const double* rrf,
+                             const int32_t* count, const float* const* raws, int S, int Tq, double threshold,
+                             double alpha, int top_k, int64_t* out_ids, double* out_rerank, double* out_rrf,
+                             uint8_t* out_keep, int32_t* out_n, uint8_t* refused, double* max_score, void* stream) {
+  if (h && S < 1) return thr_fail(h, THR_EINVAL, "thr_rerank_finish_shards: S < 1");
+  return rerank_finish_launch(h, "thr_rerank_finish_shards", B, C, stride, ids, rrf, count, nullptr, raws, S, Tq, threshold,
+                              alpha, top_k, out_ids, out_rerank, out_rrf, out_keep, out_n, refused, max_score, stream);
 }
 
 }  // extern "C"

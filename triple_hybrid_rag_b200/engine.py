@@ -18,6 +18,15 @@ def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+def _src(t: torch.Tensor, dtype: torch.dtype, shape: tuple, name: str) -> None:
+    """A kernel input that may live on another GPU (read through peer memory): checked, never moved or copied."""
+    if not isinstance(t, torch.Tensor) or t.device.type != "cuda":
+        raise TypeError(f"{name}: expected a CUDA tensor")
+    if t.dtype != dtype or tuple(t.shape) != tuple(shape) or not t.is_contiguous():
+        raise ValueError(f"{name}: expected a contiguous {dtype} tensor of shape {tuple(shape)}, got {t.dtype} "
+                         f"{tuple(t.shape)}")
+
+
 class Engine:
     def __init__(self, device: int | torch.device | None = None):
         if not torch.cuda.is_available():
@@ -61,6 +70,14 @@ class Engine:
 
     def sync(self):
         self._check(self._lib.thr_sync(self._h, self._stream()))
+
+    def peer_enable(self, device: int) -> bool:
+        """Let this handle's kernels read memory of GPU `device` (thr_peer_enable).  False when the pair cannot peer."""
+        rc = self._lib.thr_peer_enable(self._h, int(device))
+        if rc == _lib.THR_EUNSUPPORTED:
+            return False
+        self._check(rc)
+        return True
 
     @property
     def launches(self) -> int:
@@ -348,6 +365,72 @@ class Engine:
                                                 _ptr(o_rrf), _ptr(o_keep), _ptr(o_n), _ptr(o_ref), _ptr(o_mx),
                                                 self._stream()))
         return o_ids, o_rr, o_rrf, o_keep, o_n, o_ref, o_mx
+
+    def rerank_finish_shards(self, ids: torch.Tensor, rrf: torch.Tensor, count: torch.Tensor, raws: Sequence[torch.Tensor],
+                             Tq: int, threshold: float, alpha: float, top_k: int):
+        """rerank_finish on the element-wise max of the shards' raw [B, C] float32 scores (thr_rerank_finish_shards).
+        raws may live on other GPUs this handle peers with (peer_enable); the caller orders their producers before
+        this call on the current stream."""
+        ids = self._dev(ids, torch.int64, "ids")
+        rrf = self._dev(rrf, torch.float64, "rrf")
+        count = self._dev(count, torch.int32, "count")
+        B, stride = ids.shape
+        if not raws:
+            raise ValueError("rerank_finish_shards: no raw score arrays")
+        C = raws[0].shape[1]
+        for r in raws:
+            _src(r, torch.float32, (B, C), "raws")
+        tab = self._ptr_table(raws)
+        dev = self.device
+        o_ids = torch.empty((B, C), dtype=torch.int64, device=dev)
+        o_rr = torch.empty((B, C), dtype=torch.float64, device=dev)
+        o_rrf = torch.empty((B, C), dtype=torch.float64, device=dev)
+        o_keep = torch.empty((B, C), dtype=torch.uint8, device=dev)
+        o_n = torch.empty((B,), dtype=torch.int32, device=dev)
+        o_ref = torch.empty((B,), dtype=torch.uint8, device=dev)
+        o_mx = torch.empty((B,), dtype=torch.float64, device=dev)
+        self._check(self._lib.thr_rerank_finish_shards(self._h, B, C, stride, _ptr(ids), _ptr(rrf), _ptr(count), _ptr(tab),
+                                                       len(raws), int(Tq), float(threshold), float(alpha), int(top_k),
+                                                       _ptr(o_ids), _ptr(o_rr), _ptr(o_rrf), _ptr(o_keep), _ptr(o_n),
+                                                       _ptr(o_ref), _ptr(o_mx), self._stream()))
+        return o_ids, o_rr, o_rrf, o_keep, o_n, o_ref, o_mx
+
+    # -- in-process shard merge ---------------------------------------------------------------
+    def _ptr_table(self, tensors: Sequence[torch.Tensor]) -> torch.Tensor:
+        """The device addresses of `tensors` as an int64 array on this handle's GPU (the kernels' pointer tables)."""
+        h = torch.tensor([t.data_ptr() for t in tensors], dtype=torch.int64).pin_memory()
+        return h.to(self.device, non_blocking=True)
+
+    def shard_merge(self, B: int, k_sem: int, k_lex: int, sem: Sequence[Tuple[torch.Tensor, ...]],
+                    lex: Sequence[Tuple[torch.Tensor, ...]]):
+        """Merge S_sem semantic sources (ids [B,k_sem] i64, scores f64, count [B] i32, gap [B] f32: dense_topk outputs)
+        and S_lex lexical sources (ids [B,k_lex] i64, scores f32, count [B] i32: bm25_topk outputs) in one launch
+        (thr_shard_merge).  Sources may live on GPUs this handle peers with.
+        -> d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt on this handle's GPU, in dense_topk's / bm25_topk's formats."""
+        if not sem or not lex:
+            raise ValueError("shard_merge: each channel needs at least one source")
+        for ids, sc, cnt, gap in sem:
+            _src(ids, torch.int64, (B, k_sem), "d_ids"); _src(sc, torch.float64, (B, k_sem), "d_sc")
+            _src(cnt, torch.int32, (B,), "d_cnt"); _src(gap, torch.float32, (B,), "d_gap")
+        for ids, sc, cnt in lex:
+            _src(ids, torch.int64, (B, k_lex), "l_ids"); _src(sc, torch.float32, (B, k_lex), "l_sc")
+            _src(cnt, torch.int32, (B,), "l_cnt")
+        S, L = len(sem), len(lex)
+        tab = self._ptr_table([t for i in range(4) for t in (x[i] for x in sem)] +
+                              [t for i in range(3) for t in (x[i] for x in lex)])
+        at = lambda j: C.c_void_p(tab.data_ptr() + 8 * j)   # noqa: E731  (sub-table j of the one pointer array)
+        dev = self.device
+        d_ids = torch.empty((B, k_sem), dtype=torch.int64, device=dev)
+        d_sc = torch.empty((B, k_sem), dtype=torch.float64, device=dev)
+        d_cnt = torch.empty((B,), dtype=torch.int32, device=dev)
+        gap = torch.empty((B,), dtype=torch.float32, device=dev)
+        l_ids = torch.empty((B, k_lex), dtype=torch.int64, device=dev)
+        l_sc = torch.empty((B, k_lex), dtype=torch.float32, device=dev)
+        l_cnt = torch.empty((B,), dtype=torch.int32, device=dev)
+        self._check(self._lib.thr_shard_merge(self._h, B, k_sem, k_lex, S, at(0), at(S), at(2 * S), at(3 * S), L,
+                                              at(4 * S), at(4 * S + L), at(4 * S + 2 * L), _ptr(d_ids), _ptr(d_sc),
+                                              _ptr(d_cnt), _ptr(gap), _ptr(l_ids), _ptr(l_sc), _ptr(l_cnt), self._stream()))
+        return d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt
 
     # -- K5 merge ---------------------------------------------------------------------------
     def merge_topk(self, scores: torch.Tensor, ids: torch.Tensor, counts: Optional[torch.Tensor], k_out: int):

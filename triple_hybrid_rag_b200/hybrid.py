@@ -95,8 +95,8 @@ class GpuHybridSearcher:
         q = q / q.norm(dim=1, keepdim=True).clamp_min(1e-30)
         k = max(1, min(self.config.top_k_retrieve, ix.n_live, 228))
         with eng.lock:
-            ids, sc, cnt, gap = eng.dense_topk(pad_dim(q.to(torch.bfloat16)).to(eng.device), k, want=ix.want(category))
-            eng.sync()
+            ids, sc, cnt, gap = ix.dense_topk(pad_dim(q.to(torch.bfloat16)).to(eng.device), k, want=ix.want(category))
+            ix.sync()
         if float(gap[0]) <= dense_error_bound(ix.X.shape[1], 1.01, 1.01):
             import warnings
             warnings.warn("dense top-k: exactness certificate not met", RuntimeWarning)

@@ -237,6 +237,11 @@ class TripleHybridSearcher:
         if self.world > 1:
             d_ids, d_sc, d_cnt, l_ids, l_sc, l_cnt = self._exchange(B, k_sem, k_lex, d_ids, d_sc, d_cnt,
                                                                     l_ids, l_sc, l_cnt)
+        return self._fuse(B, d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt, graph_ids, weights, top_k, tie_mode, rrf_k)
+
+    def _fuse(self, B, d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt, graph_ids, weights, top_k, tie_mode, rrf_k):
+        """K3 on the (merged) channel lists -> SearchOutput."""
+        eng, dev = self.engine, self.engine.device
         if weights is None:
             weights = self._offs.get(("w", B))
             if weights is None:
@@ -388,3 +393,160 @@ class TripleHybridSearcher:
         h2d = sum(t.numel() * t.element_size() for t in ins)
         d2h = sum(t.numel() * t.element_size() for t in host)
         return host[0], host[1], host[2], h2d, d2h
+
+
+class ShardedSearcher:
+    """TripleHybridSearcher over a corpus cut into shards held by several handles of ONE process — the in-process twin
+    of TripleHybridSearcher(group=...), without torchrun and without a collective.  engines[0] is the home handle:
+    results come back on its GPU and its stream (the caller's current stream there).  Several shards may share a GPU,
+    each with its own handle.  Shard s is set up like one rank of the multi-process path: set_dense / set_bm25 /
+    set_tags / set_token_store on shards[s] with its id_base, so K1 and K2 return global ids.
+
+    One step: the query inputs are copied to every shard GPU; K1 and K2 run per shard (shards on one GPU one after
+    another on one stream: K1 and K2 each spread over every SM); the home stream waits for every shard; then one
+    thr_shard_merge launch merges both channels' lists where they lie (peer memory, or a copy on the home GPU when
+    the pair cannot peer) and thr_fuse runs on the merged lists.  The rerank stage scores each candidate on the shard
+    that owns it and thr_rerank_finish_shards takes the max of the shards' score arrays on the home GPU.
+
+    Every shard stream first waits for the home stream, so a shard's outputs of one step are never reused before the
+    home GPU's kernels of that step have read them."""
+
+    def __init__(self, engines: list):
+        if not engines:
+            raise ValueError("ShardedSearcher needs at least one engine")
+        if len(engines) > 64:
+            raise ValueError("at most 64 shards")
+        self.engines = list(engines)
+        self.engine = self.engines[0]
+        self.shards = [TripleHybridSearcher(e) for e in self.engines]
+        self._home = self.shards[0]
+        home = self.engine.device.index
+        # peer[s]: the home GPU reads shard s's outputs in place (and shard s reads the home GPU's)
+        self._peer = [e.device.index == home or (self.engine.peer_enable(e.device.index) and e.peer_enable(home))
+                      for e in self.engines]
+        self._streams = {}
+
+    @property
+    def n_shards(self) -> int:
+        return len(self.engines)
+
+    def _groups(self):
+        """Shard indices grouped by GPU, home GPU first: [(device, stream, [s, ...])]."""
+        main = torch.cuda.current_stream(self.engine.device)
+        out = {}
+        for s, e in enumerate(self.engines):
+            d = e.device.index
+            if d not in out:
+                st = main if d == self.engine.device.index else self._streams.get(d)
+                if st is None:
+                    st = self._streams[d] = torch.cuda.Stream(e.device)
+                out[d] = (e.device, st, [])
+            out[d][2].append(s)
+        return list(out.values())
+
+    def _home_view(self, s: int, t: torch.Tensor) -> torch.Tensor:
+        """Shard s's output as the home GPU's kernels read it: in place (same GPU or peer), else a copy on the home
+        GPU (enqueued on the shard's stream)."""
+        if self._peer[s]:
+            return t
+        return t.to(self.engine.device, copy=True)
+
+    def search(self, Q: torch.Tensor, q_terms: torch.Tensor, q_off: torch.Tensor,
+               graph_ids: Optional[torch.Tensor], weights: Optional[torch.Tensor] = None,
+               k_sem: int = 100, k_lex: int = 100, top_k: int = 100, margin: int = 28,
+               tie_mode: int = _lib.TIE_CHUNK_ID, rrf_k: int = 60, want: Optional[torch.Tensor] = None,
+               require_all: bool = False, lex_delta: Optional[Engine] = None) -> SearchOutput:
+        """TripleHybridSearcher.search's arguments; inputs on the home GPU.  lex_delta: the handle of the LAST shard's
+        lexical delta segment (its ids follow that shard's rows); it is one more lexical source of the merge.
+        SearchOutput.gap is the merged list's certificate: the minimum of the shards' gaps."""
+        B = Q.shape[0]
+        d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt = self._topk(B, Q, q_terms, q_off, k_sem, k_lex, margin, want,
+                                                                 require_all, lex_delta)
+        return self._home._fuse(B, d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt, graph_ids, weights, top_k, tie_mode,
+                                rrf_k)
+
+    def dense_topk(self, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None):
+        """K1 on every shard, merged: Engine.dense_topk's results (gap: the minimum of the shards')."""
+        d_ids, d_sc, d_cnt, gap, _, _, _ = self._topk(Q.shape[0], Q, None, None, k, 1, margin, want, False, None)
+        return d_ids, d_sc, d_cnt, gap
+
+    def bm25_topk(self, q_terms: torch.Tensor, q_off: torch.Tensor, k: int, want: Optional[torch.Tensor] = None,
+                  require_all: bool = False, lex_delta: Optional[Engine] = None):
+        """K2 on every shard (and the last shard's delta segment), merged: Engine.bm25_topk's results."""
+        _, _, _, _, l_ids, l_sc, l_cnt = self._topk(q_off.numel() - 1, None, q_terms, q_off, 1, k, 0, want,
+                                                    require_all, lex_delta)
+        return l_ids, l_sc, l_cnt
+
+    def _empty(self, B: int, k: int, dense: bool):
+        """A source with no entries, for a channel that is not searched (thr_shard_merge merges both)."""
+        dev = self.engine.device
+        ids = torch.full((B, k), -1, dtype=torch.int64, device=dev)
+        cnt = torch.zeros((B,), dtype=torch.int32, device=dev)
+        if dense:
+            return (ids, torch.full((B, k), float("-inf"), dtype=torch.float64, device=dev), cnt,
+                    torch.full((B,), float("inf"), dtype=torch.float32, device=dev))
+        return ids, torch.zeros((B, k), dtype=torch.float32, device=dev), cnt
+
+    def _topk(self, B, Q, q_terms, q_off, k_sem, k_lex, margin, want, require_all, lex_delta):
+        """Both channels (Q None: no semantic search; q_terms None: no lexical one) on every shard, merged on the
+        home GPU in one thr_shard_merge launch -> d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt."""
+        home = self.engine
+        main = torch.cuda.current_stream(home.device)
+        last = len(self.engines) - 1
+        sem, lex = [], []
+        for dev, st, shards in self._groups():
+            if st is not main:
+                st.wait_stream(main)
+            with torch.cuda.device(dev), torch.cuda.stream(st):
+                local = dev == home.device
+                q = Q if Q is None or local else Q.to(dev, non_blocking=True)
+                qt, qo = (q_terms, q_off) if q_terms is None or local else \
+                    (q_terms.to(dev, non_blocking=True), q_off.to(dev, non_blocking=True))
+                w = want if want is None or local else want.to(dev, non_blocking=True)
+                for s in shards:
+                    e = self.engines[s]
+                    if Q is not None:
+                        sem.append((s, tuple(self._home_view(s, t) for t in e.dense_topk(q, k_sem, margin, want=w))))
+                    if q_terms is not None:
+                        l = e.bm25_topk(qt, qo, k_lex, want=w, require_all=require_all)
+                        lex.append((s, tuple(self._home_view(s, t) for t in l)))
+                        if s == last and lex_delta is not None:
+                            l = lex_delta.bm25_topk(qt, qo, k_lex, want=w, require_all=require_all)
+                            lex.append((s + 1, tuple(self._home_view(s, t) for t in l)))
+            if st is not main:
+                main.wait_stream(st)
+        # a fixed source order (shard order, the delta segment last), whatever the grouping by GPU
+        sem = [x for _, x in sorted(sem, key=lambda p: p[0])] or [self._empty(B, k_sem, True)]
+        lex = [x for _, x in sorted(lex, key=lambda p: p[0])] or [self._empty(B, k_lex, False)]
+        return home.shard_merge(B, k_sem, k_lex, sem, lex)
+
+    def rerank(self, out: SearchOutput, Qtok: torch.Tensor, C: int, threshold: float, alpha: float, final_top_k: int,
+               q_len: Optional[torch.Tensor] = None) -> SearchOutput:
+        """TripleHybridSearcher.rerank over the shards: every shard maps the fused ids to rows of its own token store
+        (rerank_rows: -1 where another shard owns the chunk) and scores them (K4, bf16 or packed store); the home GPU
+        orders and applies the safety rule on the max of the shards' [B, C] scores (thr_rerank_finish_shards)."""
+        home = self.engine
+        main = torch.cuda.current_stream(home.device)
+        raws = [None] * len(self.engines)
+        for dev, st, shards in self._groups():
+            if st is not main:
+                st.wait_stream(main)
+            with torch.cuda.device(dev), torch.cuda.stream(st):
+                if dev == home.device:
+                    ids, cnt, qt, ql = out.ids, out.count, Qtok, q_len
+                else:   # a few hundred KB: copied rather than read over the link once per candidate
+                    ids, cnt, qt = (t.to(dev, non_blocking=True) for t in (out.ids, out.count, Qtok))
+                    ql = None if q_len is None else q_len.to(dev, non_blocking=True)
+                for s in shards:
+                    sh = self.shards[s]
+                    rows = sh.engine.rerank_rows(ids, cnt, C, sh.tok_lo, sh.tok_hi, sh.tok_period, sh.tok_off)
+                    if isinstance(sh.tok_store, torch.Tensor):
+                        raw = sh.engine.maxsim(qt, sh.tok_store, rows, q_len=ql, d_len=sh.tok_lens)
+                    else:
+                        raw = sh.engine.maxsim_packed(qt, sh.tok_store, rows, q_len=ql)
+                    raws[s] = self._home_view(s, raw)
+            if st is not main:
+                main.wait_stream(st)
+        (out.rr_ids, out.rr_score, out.rr_rrf, out.rr_keep, out.rr_n, out.refused, out.max_score) = \
+            home.rerank_finish_shards(out.ids, out.rrf, out.count, raws, Qtok.shape[1], threshold, alpha, final_top_k)
+        return out

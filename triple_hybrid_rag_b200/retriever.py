@@ -253,7 +253,7 @@ class ResidentIndex:
         self.dim = int(embeddings.shape[1])
         self.version = 0
         self._delta_engine: Optional[Engine] = None
-        dev = engine.device
+        dev = self._store_dev
         if isinstance(token_store, PackedTokenStore):
             if token_lens is not None:
                 raise ValueError("a packed token store carries its own lens")
@@ -264,6 +264,11 @@ class ResidentIndex:
             token_store = token_store.to(torch.bfloat16).to(dev).contiguous()
         self._build(list(chunks), self._unit_rows(embeddings).to(dev).contiguous(), token_store,
                     None if token_lens is None else token_lens.to(torch.int32).to(dev).contiguous(), avgdl)
+
+    @property
+    def _store_dev(self) -> torch.device:
+        """Where the index keeps its row arrays (embedding rows, token store, BM25 index): the engine's GPU."""
+        return self.engine.device
 
     @staticmethod
     def _unit_rows(embeddings: torch.Tensor) -> torch.Tensor:
@@ -292,7 +297,7 @@ class ResidentIndex:
 
     def _build(self, rows, X, token_store, token_lens, avgdl) -> None:
         """A full build over `rows` (X: their unit rows on the device): the constructor and compact()."""
-        dev = self.engine.device
+        dev = self._store_dev
         self.rows = rows
         self.id_of = {r["child_id"]: i for i, r in enumerate(rows)}
         self.collections = [r.get("collection") for r in rows]
@@ -361,6 +366,12 @@ class ResidentIndex:
         self.bm25.df = torch.from_numpy(self._df[:self.bm25.V].copy()).to(dev)
         eng.dense_deleted_set(pack_bitmap(self._dead).to(dev) if self._dead.any() else None)
         eng.bm25_deleted_set(pack_bitmap(self._dead[:self.n_main]).to(dev) if self._dead[:self.n_main].any() else None)
+        self._publish_delta(eng, idf, delta, self.tags[self.n_main:])
+
+    def _publish_delta(self, eng, idf: torch.Tensor, delta: bool, tags: torch.Tensor) -> None:
+        """The lexical delta segment (rows [n_main, N)) on a second handle on `eng`'s GPU; tags: its rows' tags there."""
+        dev = eng.device
+        N = len(self.rows)
         if N == self.n_main:
             self._delta = None
         else:
@@ -378,7 +389,7 @@ class ResidentIndex:
                 de.bm25_index_set(d.skip, d.postings, d.idf, d.n_docs, d.blk_docs, d.V, id_base=self.n_main)
             else:
                 self._delta.idf.copy_(idf.to(dev))
-            self._delta_tags = self.tags[self.n_main:].clone()   # its own allocation: 8-byte aligned
+            self._delta_tags = tags.clone()   # its own allocation: 8-byte aligned
             de.bm25_tags_set(self._delta_tags)
             dd = self._dead[self.n_main:]
             de.bm25_deleted_set(pack_bitmap(dd).to(dev) if dd.any() else None)
@@ -417,6 +428,22 @@ class ResidentIndex:
         """K2 over both lexical segments (Engine.bm25_topk's arguments and results)."""
         from .pipeline import bm25_topk_segments
         return bm25_topk_segments(self.engine, self.delta_engine, q_terms, q_off, k, want=want, require_all=require_all)
+
+    def dense_topk(self, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None):
+        """K1 over the embedding rows (Engine.dense_topk's arguments and results)."""
+        return self.engine.dense_topk(Q, k, margin, want=want)
+
+    def searcher(self):
+        """The batch searcher over this index (TripleHybridSearcher.search's interface; pass lex_delta=delta_engine)."""
+        from .pipeline import TripleHybridSearcher
+        return TripleHybridSearcher(self.engine)
+
+    def maxsim_rows(self, eng: Engine, qtok: torch.Tensor, rows: Sequence[int]) -> torch.Tensor:
+        """K4 of one query [1, Tq, 128] over token-store rows (< 0: not scored) -> raw scores [len(rows)] float32."""
+        cand = torch.tensor([list(rows)], dtype=torch.int64, device=eng.device)
+        if isinstance(self.token_store, PackedTokenStore):
+            return eng.maxsim_packed(qtok, self.token_store, cand)[0]
+        return eng.maxsim(qtok, self.token_store, cand, d_len=self.token_lens)[0]
 
     # ---- live updates ----
     def add_chunks(self, chunks: Sequence[Dict[str, Any]], embeddings: torch.Tensor,
@@ -527,7 +554,7 @@ class ResidentIndex:
         in, the bitmaps are cleared and avgdl is recomputed.  A packed token store keeps its codebook."""
         with self.engine.lock:
             live = np.flatnonzero(~self._dead)
-            sel = torch.from_numpy(live).to(self.engine.device)
+            sel = torch.from_numpy(live).to(self._store_dev)
             N = len(self.rows)
             self.version += 1
             if self._delta_engine is not None:      # no delta after a full build: free its handle and index
@@ -571,13 +598,18 @@ class ResidentIndex:
     def load(cls, engine: Engine, path, tokenizer: Optional[Callable[[str], List[str]]] = None) -> "ResidentIndex":
         """tokenizer: the callable the index was built with (callables are not persisted; default `tokenize`).
         Reads thr-resident-v3, v2 and v1 files."""
+        self = cls.__new__(cls)
+        self.engine = engine
+        self._read(path, tokenizer)
+        return self
+
+    def _read(self, path, tokenizer) -> None:
+        """The body of load() on an instance whose engine(s) are set."""
         d = torch.load(path, map_location="cpu", weights_only=True)
         fmt = d.get("format")
         if fmt not in ("thr-resident-v1", "thr-resident-v2", "thr-resident-v3"):
             raise ValueError(f"{path}: not a ResidentIndex file")
-        self = cls.__new__(cls)
-        dev = engine.device
-        self.engine = engine
+        dev = self._store_dev
         self.tokenizer = tokenizer or tokenize
         self.version = 0
         self._delta_engine = None
@@ -616,7 +648,6 @@ class ResidentIndex:
         self.id_of = {r["child_id"]: i for i, r in enumerate(self.rows) if not self._dead[i]}
         self._tag = self._tags_of(self.collections)
         self._publish(main=True, delta=True)
-        return self
 
     def want(self, collection: Optional[str]) -> Optional[torch.Tensor]:
         """The per-query filter argument of the tagged kernels for one query (None: no filter).  A collection no
@@ -717,8 +748,8 @@ class _GpuScoring:
         bound = dense_error_bound(ix.X.shape[1], 1.01, 1.01)
         for margin in (min(28, 256 - k), 256 - k):
             with eng.lock:
-                ids, sc, cnt, gap = eng.dense_topk(qd, max(k, 1), margin, want=want)           # predicate inside K1
-                eng.sync()
+                ids, sc, cnt, gap = ix.dense_topk(qd, max(k, 1), margin, want=want)            # predicate inside K1
+                ix.sync()
             if float(gap[0]) > bound:
                 break
         else:
@@ -843,10 +874,9 @@ class _GpuScoring:
         candidates (rrf_score and channel ranks set).  query_vectors [B, D].  tie_mode: exact RRF ties by chunk id
         (north_star) or TIE_INSERTION, the reference's stable-sort order (first seen lexical -> semantic -> graph).
         collections: per query, the collection its semantic and lexical hits must belong to (None: any)."""
-        from .pipeline import TripleHybridSearcher
         eng, ix = self._need_engine(), self.index
         with eng.lock:     # a batch is several C-ABI calls on one handle: one thread at a time (engine.lock)
-            return self._retrieve_batch_locked(TripleHybridSearcher(eng), queries, query_vectors, keywords, graph_ids,
+            return self._retrieve_batch_locked(ix.searcher(), queries, query_vectors, keywords, graph_ids,
                                                top_k, k_sem, k_lex, weights, collections, tie_mode)
 
     def _retrieve_batch_locked(self, s, queries, query_vectors, keywords, graph_ids, top_k, k_sem, k_lex, weights,
@@ -1041,14 +1071,10 @@ class GpuMaxSimReranker:
         qtok = self.token_encoder(query).to(torch.float32)
         qtok = qtok / qtok.norm(dim=-1, keepdim=True).clamp_min(1e-30)
         qtok = qtok.to(torch.bfloat16).to(eng.device).unsqueeze(0).contiguous()
-        cand = torch.tensor([list(rows)], dtype=torch.int64, device=eng.device)
-        if isinstance(ix.token_store, PackedTokenStore):
-            raw = eng.maxsim_packed(qtok, ix.token_store, cand)
-        else:
-            raw = eng.maxsim(qtok, ix.token_store, cand, d_len=ix.token_lens)
+        raw = ix.maxsim_rows(eng, qtok, rows)    # a sharded index scores each row on the shard that holds it
         eng.sync()
         tq = qtok.shape[1]
-        return [0.5 if r < 0 else min(1.0, max(0.0, 0.5 * (float(s) / tq + 1.0))) for r, s in zip(rows, raw[0].tolist())]
+        return [0.5 if r < 0 else min(1.0, max(0.0, 0.5 * (float(s) / tq + 1.0))) for r, s in zip(rows, raw.tolist())]
 
     async def _rerank_batch_native(self, query: str, documents: List[str]) -> List[float]:
         """reranker.py:287-291: texts in, one relevance score per text out, input order."""
