@@ -164,6 +164,26 @@ def test_updates_follow_live_rows():
     assert torch.equal(ix.bm25.postings, fresh.bm25.postings)
 
 
+def test_single_index_holds_one_copy_of_its_arrays():
+    """A ResidentIndex is one shard whose handle reads the index's own embedding rows and BM25 index, not copies."""
+    eng = RecordingEngine()
+    ix = ResidentIndex(eng, _chunks(0, 20), _emb(20, 1), blk_docs=256)
+
+    def check():
+        X = eng.last["dense_index"][0]
+        assert X.data_ptr() == ix.X.data_ptr() and X.shape == ix.X.shape
+        assert eng.last["bm25_index"][1] is ix.bm25.postings
+    check()
+    before = ix.X.data_ptr()
+    ix.add_chunks(_chunks(20, 25, seed=3), _emb(5, 3))
+    assert ix.X.data_ptr() != before              # the rows were reallocated to grow
+    check()
+    ix.delete_chunks(["c2", "c21"])
+    check()
+    ix.compact()
+    check()
+
+
 def test_unknown_id_leaves_index_unchanged():
     eng = RecordingEngine()
     ix = ResidentIndex(eng, _chunks(0, 20), _emb(20, 1), blk_docs=256)

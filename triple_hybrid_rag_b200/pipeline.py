@@ -91,6 +91,16 @@ def bm25_topk_segments(engine: Engine, delta: Optional[Engine], q_terms: torch.T
     return m_ids, m_sc, m_cnt
 
 
+def maxsim_store(engine: Engine, Qtok: torch.Tensor, store, cand: torch.Tensor, q_len: Optional[torch.Tensor] = None,
+                 d_len: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """K4 of Qtok [B, Tq, 128] over candidate rows cand [B, C] (outside the store: not scored, -inf) of a token store:
+    a bf16 [rows, Td, 128] tensor with lengths d_len, or a tokpack.PackedTokenStore, which carries its own
+    (Engine.maxsim_packed).  -> raw scores [B, C] float32."""
+    if isinstance(store, torch.Tensor):
+        return engine.maxsim(Qtok, store, cand, q_len=q_len, d_len=d_len)
+    return engine.maxsim_packed(Qtok, store, cand, q_len=q_len)
+
+
 @dataclass
 class SearchOutput:
     ids: torch.Tensor        # [B, top_k] int64, -1 padded
@@ -127,8 +137,6 @@ class TripleHybridSearcher:
             import torch.distributed as dist
             self.world = dist.get_world_size(group)
             self.rank = dist.get_rank(group)
-        self.has_dense = False
-        self.has_bm25 = False
         self._pinned = {}
         self._offs = {}
         self.exchange_fallback = None   # why the pushed exchange is not in use (None: it is, or world == 1)
@@ -142,7 +150,6 @@ class TripleHybridSearcher:
     # ---- index residency -------------------------------------------------------------------
     def set_dense(self, X_local: torch.Tensor, id_base: int = 0):
         self.engine.dense_index_set(X_local, id_base=id_base)
-        self.has_dense = True
 
     def set_tags(self, tags_local: Optional[torch.Tensor]):
         """Per-chunk tags of this shard (uint16, e.g. collection ids) for search(want=...): the reference's
@@ -154,7 +161,6 @@ class TripleHybridSearcher:
         d = index.to(self.engine.device)
         self.bm25 = d
         self.engine.bm25_index_set(d.skip, d.postings, d.idf, d.n_docs, d.blk_docs, d.V, id_base=id_base)
-        self.has_bm25 = True
 
     def set_token_store(self, store: torch.Tensor, id_lo: int, id_hi: int, period: int = 0,
                         lens: Optional[torch.Tensor] = None, row_off: int = 0):
@@ -182,17 +188,20 @@ class TripleHybridSearcher:
         ONE all-reduce(MAX) when the corpus is sharded (a candidate is scored -inf everywhere but on its owner), and
         thr_rerank_finish orders by rerank score and applies the safety threshold / denoise on every rank."""
         eng = self.engine
-        rows = eng.rerank_rows(out.ids, out.count, C, self.tok_lo, self.tok_hi, self.tok_period, self.tok_off)
-        if isinstance(self.tok_store, torch.Tensor):
-            raw = eng.maxsim(Qtok, self.tok_store, rows, q_len=q_len, d_len=self.tok_lens)
-        else:
-            raw = eng.maxsim_packed(Qtok, self.tok_store, rows, q_len=q_len)
+        raw = self._rerank_scores(out.ids, out.count, Qtok, C, q_len)
         if self.world > 1:
             import torch.distributed as dist
             dist.all_reduce(raw, op=dist.ReduceOp.MAX, group=self.group)
         (out.rr_ids, out.rr_score, out.rr_rrf, out.rr_keep, out.rr_n, out.refused, out.max_score) = eng.rerank_finish(
             out.ids, out.rrf, out.count, raw, Qtok.shape[1], threshold, alpha, final_top_k)
         return out
+
+    def _rerank_scores(self, ids: torch.Tensor, count: torch.Tensor, Qtok: torch.Tensor, C: int,
+                       q_len: Optional[torch.Tensor]) -> torch.Tensor:
+        """K4 of the first C fused candidates on this rank's token store -> raw scores [B, C] (-inf where another
+        rank owns the chunk)."""
+        rows = self.engine.rerank_rows(ids, count, C, self.tok_lo, self.tok_hi, self.tok_period, self.tok_off)
+        return maxsim_store(self.engine, Qtok, self.tok_store, rows, q_len=q_len, d_len=self.tok_lens)
 
     # ---- one batch, device tensors in / out ------------------------------------------------
     def search(self, Q: torch.Tensor, q_terms: torch.Tensor, q_off: torch.Tensor,
@@ -522,8 +531,8 @@ class ShardedSearcher:
 
     def rerank(self, out: SearchOutput, Qtok: torch.Tensor, C: int, threshold: float, alpha: float, final_top_k: int,
                q_len: Optional[torch.Tensor] = None) -> SearchOutput:
-        """TripleHybridSearcher.rerank over the shards: every shard maps the fused ids to rows of its own token store
-        (rerank_rows: -1 where another shard owns the chunk) and scores them (K4, bf16 or packed store); the home GPU
+        """TripleHybridSearcher.rerank over the shards: every shard scores the fused candidates on its own token store
+        (TripleHybridSearcher._rerank_scores: -inf where another shard owns the chunk); the home GPU
         orders and applies the safety rule on the max of the shards' [B, C] scores (thr_rerank_finish_shards)."""
         home = self.engine
         main = torch.cuda.current_stream(home.device)
@@ -538,13 +547,7 @@ class ShardedSearcher:
                     ids, cnt, qt = (t.to(dev, non_blocking=True) for t in (out.ids, out.count, Qtok))
                     ql = None if q_len is None else q_len.to(dev, non_blocking=True)
                 for s in shards:
-                    sh = self.shards[s]
-                    rows = sh.engine.rerank_rows(ids, cnt, C, sh.tok_lo, sh.tok_hi, sh.tok_period, sh.tok_off)
-                    if isinstance(sh.tok_store, torch.Tensor):
-                        raw = sh.engine.maxsim(qt, sh.tok_store, rows, q_len=ql, d_len=sh.tok_lens)
-                    else:
-                        raw = sh.engine.maxsim_packed(qt, sh.tok_store, rows, q_len=ql)
-                    raws[s] = self._home_view(s, raw)
+                    raws[s] = self._home_view(s, self.shards[s]._rerank_scores(ids, cnt, qt, C, ql))
             if st is not main:
                 main.wait_stream(st)
         (out.rr_ids, out.rr_score, out.rr_rrf, out.rr_keep, out.rr_n, out.refused, out.max_score) = \
