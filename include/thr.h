@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define THR_ABI_VERSION 13
+#define THR_ABI_VERSION 14
 
 enum {
   THR_OK = 0,
@@ -137,6 +137,39 @@ int thr_dense_topk_tagged(thr_handle* h, const void* Q, int B, int k, int margin
  * the bitmap is dropped by the next thr_dense_index_set.
  */
 int thr_dense_deleted_set(thr_handle* h, const uint32_t* bits);
+
+/* Prefix funnel of the semantic channel, for Matryoshka embeddings (the leading dimensions carry most of the
+ * similarity): rank the corpus over the first d_scan columns, keep a pool of the best P, re-score the pool at full
+ * width and return the top k.  The scan reads d_scan / D of the bytes.  The result is exactly defined (for a query q
+ * over the eligible live rows, tag filter and deletion bitmap applied as in thr_dense_topk_tagged):
+ *   pool   = the P rows with the largest fp64 dot product of the bf16 inputs over columns [0, d_scan), ordered by
+ *            (prefix score desc, id asc);
+ *   result = the pool's rows re-scored in fp64 over all D columns (the summation order of thr_dense_topk's re-score),
+ *            the first min(k, |pool|) by (full score desc, id asc).
+ * With d_scan = D and P >= k this is thr_dense_topk's result, bit for bit.  It does not depend on the sharding: the
+ * shards' prefix top-P lists merged (thr_shard_merge) are the global pool, and each pool row is re-scored by the shard
+ * that holds it.
+ *
+ * thr_dense_topk_prefix: thr_dense_topk_tagged with every dot product taken over columns [0, d_scan) of X and Q (both
+ *   keep their row pitch of D).  d_scan is a multiple of 64, 64 <= d_scan <= D; d_scan == D is thr_dense_topk_tagged
+ *   (which is this call).  out_gap certifies the pool: the result is the exact prefix top-k when gap exceeds the fp32
+ *   error bound of a d_scan-term accumulation.  It says nothing about equality with a full-width scan.
+ * thr_dense_rescore: ids [B, P] int64 global ids (-1 padded) and count [B] -> out [B, P] double: the full-width fp64
+ *   dot product of Q[q] (bf16 [B, D]) with the row of ids[q, j] when this handle holds it (id_base <= id < id_base + N),
+ *   else -inf; -inf past count[q].  Bit-identical to the scores thr_dense_topk returns for the same rows.  P >= 1.
+ * thr_dense_funnel_finish: scores is a device array of S pointers to [B, P] double (thr_dense_rescore outputs of the
+ *   shards; exactly one scores each id).  Per query: the element-wise max over the S arrays, then the first
+ *   min(k, count[q]) entries by (score desc, id asc), in thr_dense_topk's output format (out_ids [B, k] -1 padded,
+ *   out_scores [B, k] -inf padded, out_count [B]).  1 <= k <= P <= 256, 1 <= S <= 64.  Needs no index.
+ * thr_dense_rescore and thr_dense_funnel_finish are timed in the THR_PROF_DENSE_FINALIZE slot.
+ */
+int thr_dense_topk_prefix(thr_handle* h, const void* Q, int B, int k, int margin, const int32_t* want, int d_scan,
+                          int64_t* out_ids, double* out_scores, int32_t* out_count, float* out_gap, void* stream);
+int thr_dense_rescore(thr_handle* h, const void* Q, int B, const int64_t* ids, const int32_t* count, int P,
+                      double* out, void* stream);
+int thr_dense_funnel_finish(thr_handle* h, int B, int P, int k, const int64_t* ids, const int32_t* count,
+                            const double* const* scores, int S, int64_t* out_ids, double* out_scores,
+                            int32_t* out_count, void* stream);
 
 /* ---- K2: lexical channel — BM25 top-k over a blocked CSR inverted index ----------
  * Replaces RAG2Retriever._lexical_search -> RPC rag2_lexical_search

@@ -18,7 +18,7 @@ THR_EINVAL, THR_ECUDA, THR_EUNSUPPORTED, THR_ENOINDEX, THR_EOVERFLOW, THR_ETIMEO
 FUSE_RAG2, FUSE_LIB, FUSE_RAG1 = 0, 1, 2
 TIE_INSERTION, TIE_CHUNK_ID = 0, 1
 BM25_REQUIRE_ALL = 1
-ABI_VERSION = 13
+ABI_VERSION = 14
 PROF_SLOTS = ("dense_score", "dense_finalize", "bm25", "fuse", "maxsim", "merge", "safety", "bm25_prep", "dense_seed", "rerank")
 
 _p, _i, _i64, _d = C.c_void_p, C.c_int, C.c_int64, C.c_double
@@ -41,6 +41,9 @@ SIGNATURES = {
     "thr_dense_tags_set": (_i, [_p, _p]),
     "thr_dense_topk_tagged": (_i, [_p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _p]),
     "thr_dense_deleted_set": (_i, [_p, _p]),
+    "thr_dense_topk_prefix": (_i, [_p, _p, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p]),
+    "thr_dense_rescore": (_i, [_p, _p, _i, _p, _p, _i, _p, _p]),
+    "thr_dense_funnel_finish": (_i, [_p, _i, _i, _i, _p, _p, _p, _i, _p, _p, _p, _p]),
     "thr_bm25_tags_set": (_i, [_p, _p]),
     "thr_bm25_topk_tagged": (_i, [_p, _p, _p, _i, _i, _p, _p, _p, _p, _p]),
     "thr_bm25_deleted_set": (_i, [_p, _p]),

@@ -55,7 +55,7 @@ typedef CUresult (*encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_
                                     CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
 int thr_encode_tma_2d_bf16(thr_handle* h, CUtensorMap* map, const void* base, uint64_t rows,
-                           uint64_t cols, uint32_t box_rows, uint32_t box_cols) {
+                           uint64_t cols, uint32_t box_rows, uint32_t box_cols, uint64_t ld) {
   static encode_tiled_fn fn = nullptr;
   if (!fn) {
     void* p = nullptr;
@@ -66,10 +66,11 @@ int thr_encode_tma_2d_bf16(thr_handle* h, CUtensorMap* map, const void* base, ui
                       cudaGetErrorString(e));
     fn = (encode_tiled_fn)p;
   }
-  if (((uintptr_t)base & 15u) != 0 || (cols * 2) % 16 != 0)
-    return thr_fail(h, THR_EINVAL, "TMA source must be 16-byte aligned with a 16-byte row pitch");
+  if (ld == 0) ld = cols;
+  if (((uintptr_t)base & 15u) != 0 || (ld * 2) % 16 != 0 || ld < cols)
+    return thr_fail(h, THR_EINVAL, "TMA source must be 16-byte aligned with a 16-byte row pitch of at least its width");
   cuuint64_t dims[2] = {cols, rows};           // innermost first
-  cuuint64_t strides[1] = {cols * 2};          // bytes, dims 1..rank-1
+  cuuint64_t strides[1] = {ld * 2};            // bytes, dims 1..rank-1
   cuuint32_t box[2] = {box_cols, box_rows};
   cuuint32_t estr[2] = {1, 1};
   CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides,

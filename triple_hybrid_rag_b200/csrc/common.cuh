@@ -50,9 +50,10 @@ void thr_prof_end(thr_handle* h, int token, cudaStream_t s);
 int thr_fail(thr_handle* h, int code, const char* fmt, ...);
 // Grow-only device scratch owned by the handle (arena 0: dense, 1: BM25). Returns NULL (and sets err) on failure.
 void* thr_scratch(thr_handle* h, int arena, size_t bytes);
-// cuTensorMapEncodeTiled through the runtime's driver entry point (no -lcuda needed).
+// cuTensorMapEncodeTiled through the runtime's driver entry point (no -lcuda needed).  ld: row pitch in elements
+// (0: cols), so that a map can cover the leading `cols` columns of a wider row-major matrix.
 int thr_encode_tma_2d_bf16(thr_handle* h, CUtensorMap* map, const void* base, uint64_t rows,
-                           uint64_t cols, uint32_t box_rows, uint32_t box_cols);
+                           uint64_t cols, uint32_t box_rows, uint32_t box_cols, uint64_t ld = 0);
 
 #define THR_CUDA(h, expr)                                                              \
   do {                                                                                 \

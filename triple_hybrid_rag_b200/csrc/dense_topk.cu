@@ -13,6 +13,9 @@
 //   dense_finalize_kernel one CTA per query: radix-select the global best K' of the cluster lists,
 //                        re-score them exactly (fp64 dot of the bf16 inputs), sort by
 //                        (score desc, id asc), emit top-k and the exactness certificate gap.
+// Both take the scored width D apart from the row pitch, so thr_dense_topk_prefix runs them over the leading d_scan
+// columns of the same rows (the prefix funnel); dense_rescore_kernel re-scores a pool at full width with the
+// finalize's own re-score, and dense_funnel_finish_kernel orders it.
 //
 // Layout per cluster step ("tile"): 128*kCtaGroup queries x 256 chunks x D.
 //   kCtaGroup = 2 : CTA pair, tcgen05.mma.cta_group::2 M=256 N=256, each CTA loads 128 query rows and
@@ -412,7 +415,8 @@ dense_score_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
 struct FinalArgs {
   const __nv_bfloat16* Q;
   const __nv_bfloat16* X;
-  int B, D;
+  int B, D;         // D: the columns scored (the prefix width); ld: the row pitch of Q and X
+  int64_t ld;
   int64_t N, id_base;
   int k, ksel, n_clusters, Bpad;
   const uint64_t* cand;
@@ -422,6 +426,63 @@ struct FinalArgs {
   int32_t* out_count;
   float* out_gap;
 };
+
+// The exact re-score: fp64 dot of the bf16 inputs over columns [0, D) of kInFlight rows of X (row pitch ld) with the
+// query row qrow (shared memory), by one warp in a fixed summation order: lane l accumulates columns l*8 .. l*8+7 of
+// every 256-column block with fma, then an xor-shuffle reduction.  Every lane returns the sums.  Four rows are in
+// flight so that their scattered row reads overlap.  K1's finalize and thr_dense_rescore both call it, so a row's score
+// is the same bits in either.
+constexpr int kInFlight = 4;
+__device__ __forceinline__ void rescore_rows(const __nv_bfloat16* X, int64_t ld, int D, const uint32_t (&idx)[kInFlight],
+                                             const __nv_bfloat16* qrow, int lane, double (&acc)[kInFlight]) {
+#pragma unroll
+  for (int u = 0; u < kInFlight; ++u) acc[u] = 0.0;
+  for (int d0 = lane * 8; d0 < D; d0 += 256) {
+    uint4 xv[kInFlight];
+#pragma unroll
+    for (int u = 0; u < kInFlight; ++u) xv[u] = *reinterpret_cast<const uint4*>(X + (size_t)idx[u] * ld + d0);
+    double qd[8];
+#pragma unroll
+    for (int e = 0; e < 8; ++e) qd[e] = (double)__bfloat162float(qrow[d0 + e]);
+#pragma unroll
+    for (int u = 0; u < kInFlight; ++u) {
+      const __nv_bfloat16* xe = reinterpret_cast<const __nv_bfloat16*>(&xv[u]);
+#pragma unroll
+      for (int e = 0; e < 8; ++e) acc[u] = fma((double)__bfloat162float(xe[e]), qd[e], acc[u]);
+    }
+  }
+#pragma unroll
+  for (int u = 0; u < kInFlight; ++u) {
+#pragma unroll
+    for (int sh = 16; sh > 0; sh >>= 1) acc[u] += __shfl_xor_sync(0xffffffffu, acc[u], sh);
+  }
+}
+
+// Order n <= kMaxSel (score, id) pairs by (score desc, id asc) without barriers: element e = tid / P is counted by P
+// adjacent threads (P = kFinalThreads / the next power of two >= max(n, 32)), each over every P-th other element.  The
+// pairs are distinct, so the ranks are a permutation.  Every thread of the CTA must call it; it returns the rank of
+// element *e (valid in the thread with part == 0, and only when *e < n).
+template <typename Id>
+__device__ __forceinline__ int rank_by_score_id(const double* sc, const Id* id, int n, int* e, int* part) {
+  const int tid = threadIdx.x;
+  int n2 = 32;
+  while (n2 < n) n2 <<= 1;
+  const int P = kFinalThreads / n2;   // 2 .. 16 threads per element, adjacent lanes
+  *e = tid / P;
+  *part = tid - *e * P;
+  int rank = 0;
+  if (*e < n) {
+    const double se = sc[*e];
+    const Id ie = id[*e];
+    for (int j = *part; j < n; j += P) {
+      const double sj = sc[j];
+      const Id ij = id[j];
+      rank += (sj > se || (sj == se && ij < ie)) ? 1 : 0;
+    }
+  }
+  for (int sh = 1; sh < P; sh <<= 1) rank += __shfl_xor_sync(0xffffffffu, rank, sh);
+  return rank;
+}
 
 __global__ void __launch_bounds__(kFinalThreads, 2) dense_finalize_kernel(const FinalArgs a) {
   extern __shared__ uint8_t fsm[];
@@ -439,7 +500,7 @@ __global__ void __launch_bounds__(kFinalThreads, 2) dense_finalize_kernel(const 
 
   const int q = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   if (tid == 0) { s_nsel = 0; s_minkey = ~0ull; }
-  for (int i = tid; i < a.D; i += kFinalThreads) qrow[i] = a.Q[(size_t)q * a.D + i];
+  for (int i = tid; i < a.D; i += kFinalThreads) qrow[i] = a.Q[(size_t)q * a.ld + i];
   // 1. gather the per-cluster lists of this query: list lengths first (one load per cluster, all in flight), an
   //    exclusive scan over the clusters by the first warp, then one flat copy whose loads do not depend on each other
   for (int c = tid; c < kMaxClusters; c += kFinalThreads)
@@ -520,71 +581,33 @@ __global__ void __launch_bounds__(kFinalThreads, 2) dense_finalize_kernel(const 
     const int lines = (a.D * 2 + 127) / 128;
     for (int j = tid; j < nsel * lines; j += kFinalThreads) {
       const int r = j / lines, l = j - r * lines;
-      const char* p = (const char*)(a.X + (size_t)key_index(sel_key[r]) * a.D) + (size_t)l * 128;
+      const char* p = (const char*)(a.X + (size_t)key_index(sel_key[r]) * a.ld) + (size_t)l * 128;
       asm volatile("prefetch.global.L2 [%0];" ::"l"(p));
     }
   }
 
-  // 4. exact re-score: fp64 dot of the bf16 inputs, one warp per survivor, fixed summation order.  Four
-  //    survivors are in flight per warp so that their scattered row reads overlap.
-  constexpr int kInFlight = 4;
+  // 4. exact re-score: fp64 dot of the bf16 inputs, one warp per kInFlight survivors, fixed summation order
   constexpr int kWarpsF = kFinalThreads / 32;
   for (int i0 = warp * kInFlight; i0 < nsel; i0 += kWarpsF * kInFlight) {
     uint32_t idx[kInFlight];
     double acc[kInFlight];
 #pragma unroll
-    for (int u = 0; u < kInFlight; ++u) {
-      idx[u] = i0 + u < nsel ? key_index(sel_key[i0 + u]) : 0u;
-      acc[u] = 0.0;
-    }
-    for (int d0 = lane * 8; d0 < a.D; d0 += 256) {
-      uint4 xv[kInFlight];
+    for (int u = 0; u < kInFlight; ++u) idx[u] = i0 + u < nsel ? key_index(sel_key[i0 + u]) : 0u;
+    rescore_rows(a.X, a.ld, a.D, idx, qrow, lane, acc);
 #pragma unroll
-      for (int u = 0; u < kInFlight; ++u)
-        xv[u] = *reinterpret_cast<const uint4*>(a.X + (size_t)idx[u] * a.D + d0);
-      double qd[8];
-#pragma unroll
-      for (int e = 0; e < 8; ++e) qd[e] = (double)__bfloat162float(qrow[d0 + e]);
-#pragma unroll
-      for (int u = 0; u < kInFlight; ++u) {
-        const __nv_bfloat16* xe = reinterpret_cast<const __nv_bfloat16*>(&xv[u]);
-#pragma unroll
-        for (int e = 0; e < 8; ++e) acc[u] = fma((double)__bfloat162float(xe[e]), qd[e], acc[u]);
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < kInFlight; ++u) {
-      double s = acc[u];
-#pragma unroll
-      for (int sh = 16; sh > 0; sh >>= 1) s += __shfl_xor_sync(0xffffffffu, s, sh);
-      if (lane == 0 && i0 + u < nsel) { sel_score[i0 + u] = s; sel_idx[i0 + u] = idx[u]; }
-    }
+    for (int u = 0; u < kInFlight; ++u)
+      if (lane == 0 && i0 + u < nsel) { sel_score[i0 + u] = acc[u]; sel_idx[i0 + u] = idx[u]; }
   }
   __syncthreads();
 
-  // 5. order by (score desc, idx asc) without barriers: every survivor counts the survivors that precede it, P
-  //    threads per survivor (the pairs are distinct, so the ranks are a permutation), and writes its own output row
+  // 5. order by (score desc, idx asc) without barriers; every survivor writes its own output row
   const int nout = min(nsel, a.k);
-  int n2 = 32;
-  while (n2 < nsel) n2 <<= 1;
-  const int P = kFinalThreads / n2;   // 2 .. 16 threads per survivor, adjacent lanes
-  const int e = tid / P, part = tid - e * P;
-  int rank = 0;
-  double se = 0.0;
-  uint32_t ie = 0;
-  if (e < nsel) {
-    se = sel_score[e];
-    ie = sel_idx[e];
-    for (int j = part; j < nsel; j += P) {
-      const double sj = sel_score[j];
-      const uint32_t ij = sel_idx[j];
-      rank += (sj > se || (sj == se && ij < ie)) ? 1 : 0;
-    }
-  }
-  for (int sh = 1; sh < P; sh <<= 1) rank += __shfl_xor_sync(0xffffffffu, rank, sh);
+  int e, part;
+  const int rank = rank_by_score_id(sel_score, sel_idx, nsel, &e, &part);
   if (e < nsel && part == 0 && rank < nout) {
+    const double se = sel_score[e];
     const size_t o = (size_t)q * a.k + rank;
-    a.out_ids[o] = a.id_base + (int64_t)ie;
+    a.out_ids[o] = a.id_base + (int64_t)sel_idx[e];
     a.out_scores[o] = se;
     if (rank == nout - 1 && a.out_gap) {
       // every chunk that was not re-scored has a tensor-core score <= the K'-th best key's
@@ -771,6 +794,88 @@ __global__ void __launch_bounds__(kSelThreads) dense_seed_select_kernel(const ui
   if (tid == 0) tau_out[q] = tau;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Prefix funnel: full-width re-score of a candidate pool, and the final order over the shards' scores.
+// ------------------------------------------------------------------------------------------------
+struct RescoreArgs {
+  const __nv_bfloat16* Q;   // [B, D]
+  const __nv_bfloat16* X;   // [N, D]
+  int D, P;
+  int64_t N, id_base;
+  const int64_t* ids;       // [B, P] global ids, -1 padded
+  const int32_t* count;     // [B]
+  double* out;              // [B, P]
+};
+constexpr int kRescoreRows = kFinalThreads / 32 * kInFlight;   // pool entries per CTA
+
+// grid (B, ceil(P / kRescoreRows)): a CTA re-scores kRescoreRows entries of one query's pool, kInFlight per warp
+__global__ void __launch_bounds__(kFinalThreads) dense_rescore_kernel(const RescoreArgs a) {
+  extern __shared__ uint8_t rsm[];
+  __nv_bfloat16* qrow = (__nv_bfloat16*)rsm;
+  const int q = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  for (int i = tid; i < a.D; i += kFinalThreads) qrow[i] = a.Q[(size_t)q * a.D + i];
+  __syncthreads();
+  const int n = min(max(a.count[q], 0), a.P);
+  const int i0 = blockIdx.y * kRescoreRows + warp * kInFlight;
+  if (i0 >= a.P) return;   // warp-uniform
+  uint32_t idx[kInFlight];
+  bool mine[kInFlight], any = false;
+#pragma unroll
+  for (int u = 0; u < kInFlight; ++u) {
+    const int64_t id = i0 + u < n ? a.ids[(size_t)q * a.P + i0 + u] : -1;
+    mine[u] = id >= a.id_base && id < a.id_base + a.N;   // a row of this handle (padding never is)
+    idx[u] = mine[u] ? (uint32_t)(id - a.id_base) : 0u;
+    any |= mine[u];
+  }
+  double acc[kInFlight] = {};
+  if (any) rescore_rows(a.X, a.D, a.D, idx, qrow, lane, acc);
+  if (lane == 0) {
+#pragma unroll
+    for (int u = 0; u < kInFlight; ++u)
+      if (i0 + u < a.P) a.out[(size_t)q * a.P + i0 + u] = mine[u] ? acc[u] : -CUDART_INF;
+  }
+}
+
+struct FunnelFinishArgs {
+  int P, k, S;
+  const int64_t* ids;            // [B, P]
+  const int32_t* count;          // [B]
+  const double* const* scores;   // [S] -> [B, P]
+  int64_t* out_ids;
+  double* out_scores;
+  int32_t* out_count;
+};
+
+// one CTA per query: the element-wise max over the S score arrays, then the first min(k, count) by (score desc, id asc)
+__global__ void __launch_bounds__(kFinalThreads) dense_funnel_finish_kernel(const FunnelFinishArgs a) {
+  __shared__ double s_sc[kMaxSel];
+  __shared__ int64_t s_id[kMaxSel];
+  const int q = blockIdx.x, tid = threadIdx.x;
+  const int n = min(max(a.count[q], 0), a.P);
+  for (int j = tid; j < n; j += kFinalThreads) {
+    const size_t o = (size_t)q * a.P + j;
+    double v = -CUDART_INF;
+    for (int s = 0; s < a.S; ++s) v = fmax(v, a.scores[s][o]);
+    s_sc[j] = v;
+    s_id[j] = a.ids[o];
+  }
+  __syncthreads();
+  const int nout = min(n, a.k);
+  int e, part;
+  const int rank = rank_by_score_id(s_sc, s_id, n, &e, &part);
+  if (e < n && part == 0 && rank < nout) {
+    const size_t o = (size_t)q * a.k + rank;
+    a.out_ids[o] = s_id[e];
+    a.out_scores[o] = s_sc[e];
+  }
+  if (tid == 0) a.out_count[q] = nout;
+  for (int i = nout + tid; i < a.k; i += kFinalThreads) {
+    const size_t o = (size_t)q * a.k + i;
+    a.out_ids[o] = -1;
+    a.out_scores[o] = -CUDART_INF;
+  }
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------
@@ -781,7 +886,8 @@ struct thr_dense_state {
   int64_t N;
   int D;
   int64_t id_base;
-  CUtensorMap map_x;
+  CUtensorMap map_x;   // the leading map_d columns of X (row pitch D): D when the index is set, then the last d_scan
+  int map_d;
   int cta_group;  // 2 (pair) or 1; THR_DENSE_CTA_GROUP overrides for bring-up
   const uint16_t* tags;  // [N] device, nullable
   const uint32_t* deleted;  // [ceil(N / 32)] device, nullable
@@ -834,6 +940,7 @@ int thr_dense_index_set(thr_handle* h, const void* X, int64_t N, int D, int64_t 
   st->X = X; st->N = N; st->D = D; st->id_base = id_base;
   int rc = thr_encode_tma_2d_bf16(h, &st->map_x, X, (uint64_t)N, (uint64_t)D, 128, kBlockK);
   if (rc != THR_OK) { free(st); return rc; }
+  st->map_d = D;
   st->cta_group = 2;
   const char* env = getenv("THR_DENSE_CTA_GROUP");
   if (env && env[0] == '1') st->cta_group = 1;
@@ -871,19 +978,37 @@ int thr_dense_topk_tagged(thr_handle* h, const void* Q, int B, int k, int margin
                           int64_t* out_ids, double* out_scores, int32_t* out_count, float* out_gap,
                           void* stream) {
   if (!h) return THR_EINVAL;
+  if (!h->dense) return thr_fail(h, THR_ENOINDEX, "thr_dense_topk: call thr_dense_index_set first");
+  return thr_dense_topk_prefix(h, Q, B, k, margin, want, h->dense->D, out_ids, out_scores, out_count, out_gap,
+                               stream);
+}
+
+int thr_dense_topk_prefix(thr_handle* h, const void* Q, int B, int k, int margin, const int32_t* want, int d_scan,
+                          int64_t* out_ids, double* out_scores, int32_t* out_count, float* out_gap, void* stream) {
+  if (!h) return THR_EINVAL;
   cudaSetDevice(h->device);
   thr_dense_state* st = h->dense;
   if (!st) return thr_fail(h, THR_ENOINDEX, "thr_dense_topk: call thr_dense_index_set first");
   THR_REQUIRE(h, want == nullptr || st->tags != nullptr, "thr_dense_topk_tagged: call thr_dense_tags_set first");
   THR_REQUIRE(h, B >= 0 && k >= 1 && margin >= 0, "thr_dense_topk: bad B/k/margin");
+  THR_REQUIRE(h, d_scan % kBlockK == 0 && d_scan >= kBlockK && d_scan <= st->D,
+              "thr_dense_topk_prefix: d_scan = %d must be a multiple of 64 in [64, D = %d]", d_scan, st->D);
   if (B == 0) return THR_OK;
   THR_REQUIRE(h, k + margin <= kMaxSel, "thr_dense_topk: k + margin = %d exceeds %d", k + margin, kMaxSel);
   THR_REQUIRE(h, Q && out_ids && out_scores && out_count, "thr_dense_topk: NULL argument");
   cudaStream_t s = (cudaStream_t)stream;
+  int rc;
+  if (st->map_d != d_scan) {   // the same rows, fewer columns: the map's width changes, its row pitch stays D
+    st->map_d = 0;
+    rc = thr_encode_tma_2d_bf16(h, &st->map_x, st->X, (uint64_t)st->N, (uint64_t)d_scan, 128, kBlockK,
+                                (uint64_t)st->D);
+    if (rc != THR_OK) return rc;
+    st->map_d = d_scan;
+  }
   // up to 128 queries fit one CTA's M = 128 tile: the single-CTA kernel then does half the MMA work per
   // chunk tile and the scan is HBM-bound (batch-1 latency); larger batches use the CTA pair (M = 256)
   // (only while the finalize kernel's shared memory — one K' list per CTA — still fits)
-  const bool small_ok = (size_t)h->num_sms * (k + margin) * 8 + (size_t)st->D * 2 <= 200 * 1024;
+  const bool small_ok = (size_t)h->num_sms * (k + margin) * 8 + (size_t)d_scan * 2 <= 200 * 1024;
   const int G = (B <= kBlockM && small_ok) ? 1 : st->cta_group;
   const int64_t tiles = (st->N + kTileN - 1) / kTileN;
   int n_clusters = h->num_sms / G;
@@ -896,11 +1021,11 @@ int thr_dense_topk_tagged(thr_handle* h, const void* Q, int B, int k, int margin
   if (!ws) return THR_ENOMEM;
 
   CUtensorMap map_q;
-  int rc = thr_encode_tma_2d_bf16(h, &map_q, Q, (uint64_t)B, (uint64_t)st->D, 128, kBlockK);
+  rc = thr_encode_tma_2d_bf16(h, &map_q, Q, (uint64_t)B, (uint64_t)d_scan, 128, kBlockK, (uint64_t)st->D);
   if (rc != THR_OK) return rc;
 
   ScoreArgs a;
-  a.B = B; a.N = st->N; a.D = st->D; a.ksel = k + margin; a.n_clusters = n_clusters; a.Bpad = Bpad;
+  a.B = B; a.N = st->N; a.D = d_scan; a.ksel = k + margin; a.n_clusters = n_clusters; a.Bpad = Bpad;
   a.cand = (uint64_t*)ws; a.cnt = (int32_t*)(ws + cand_bytes); a.status = h->d_status;
   a.tau_init = nullptr;
   a.seed_mode = 0;
@@ -910,11 +1035,11 @@ int thr_dense_topk_tagged(thr_handle* h, const void* Q, int B, int k, int margin
   float* tau_seed = (float*)(ws + cand_bytes + cnt_bytes);
 
   FinalArgs f;
-  f.Q = (const __nv_bfloat16*)Q; f.X = (const __nv_bfloat16*)st->X; f.B = B; f.D = st->D; f.N = st->N;
+  f.Q = (const __nv_bfloat16*)Q; f.X = (const __nv_bfloat16*)st->X; f.B = B; f.D = d_scan; f.ld = st->D; f.N = st->N;
   f.id_base = st->id_base; f.k = k; f.ksel = k + margin; f.n_clusters = n_clusters; f.Bpad = Bpad;
   f.cand = a.cand; f.cnt = a.cnt; f.out_ids = out_ids; f.out_scores = out_scores;
   f.out_count = out_count; f.out_gap = out_gap;
-  const size_t fsmem = (size_t)n_clusters * f.ksel * sizeof(uint64_t) + (size_t)st->D * 2;
+  const size_t fsmem = (size_t)n_clusters * f.ksel * sizeof(uint64_t) + (size_t)d_scan * 2;
   THR_CUDA(h, cudaFuncSetAttribute(dense_finalize_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsmem));
 
   // Seed pass: score a small prefix of the corpus first and start the full pass from its K'-th best
@@ -948,6 +1073,48 @@ int thr_dense_topk_tagged(thr_handle* h, const void* Q, int B, int k, int margin
   dense_finalize_kernel<<<B, kFinalThreads, fsmem, s>>>(f);
   thr_prof_end(h, tok, s);
   THR_CHECK_LAUNCH(h, "dense_finalize_kernel");
+  return THR_OK;
+}
+
+int thr_dense_rescore(thr_handle* h, const void* Q, int B, const int64_t* ids, const int32_t* count, int P,
+                      double* out, void* stream) {
+  if (!h) return THR_EINVAL;
+  cudaSetDevice(h->device);
+  thr_dense_state* st = h->dense;
+  if (!st) return thr_fail(h, THR_ENOINDEX, "thr_dense_rescore: call thr_dense_index_set first");
+  THR_REQUIRE(h, B >= 0 && P >= 1, "thr_dense_rescore: bad B/P");
+  if (B == 0) return THR_OK;
+  THR_REQUIRE(h, Q && ids && count && out, "thr_dense_rescore: NULL argument");
+  RescoreArgs a;
+  a.Q = (const __nv_bfloat16*)Q; a.X = (const __nv_bfloat16*)st->X; a.D = st->D; a.P = P; a.N = st->N;
+  a.id_base = st->id_base; a.ids = ids; a.count = count; a.out = out;
+  const size_t smem = (size_t)st->D * 2;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int tok = thr_prof_begin(h, THR_PROF_DENSE_FINALIZE, s);
+  dense_rescore_kernel<<<dim3(B, (P + kRescoreRows - 1) / kRescoreRows), kFinalThreads, smem, s>>>(a);
+  thr_prof_end(h, tok, s);
+  THR_CHECK_LAUNCH(h, "dense_rescore_kernel");
+  return THR_OK;
+}
+
+int thr_dense_funnel_finish(thr_handle* h, int B, int P, int k, const int64_t* ids, const int32_t* count,
+                            const double* const* scores, int S, int64_t* out_ids, double* out_scores,
+                            int32_t* out_count, void* stream) {
+  if (!h) return THR_EINVAL;
+  cudaSetDevice(h->device);
+  THR_REQUIRE(h, B >= 0 && k >= 1 && k <= P && P <= kMaxSel && S >= 1 && S <= 64,
+              "thr_dense_funnel_finish: need 1 <= k <= P <= %d and 1 <= S <= 64 (k = %d, P = %d, S = %d)", kMaxSel, k,
+              P, S);
+  if (B == 0) return THR_OK;
+  THR_REQUIRE(h, ids && count && scores && out_ids && out_scores && out_count, "thr_dense_funnel_finish: NULL argument");
+  FunnelFinishArgs a;
+  a.P = P; a.k = k; a.S = S; a.ids = ids; a.count = count; a.scores = scores;
+  a.out_ids = out_ids; a.out_scores = out_scores; a.out_count = out_count;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int tok = thr_prof_begin(h, THR_PROF_DENSE_FINALIZE, s);
+  dense_funnel_finish_kernel<<<B, kFinalThreads, 0, s>>>(a);
+  thr_prof_end(h, tok, s);
+  THR_CHECK_LAUNCH(h, "dense_funnel_finish_kernel");
   return THR_OK;
 }
 

@@ -141,10 +141,12 @@ class Engine:
         self._keep["dense_deleted"] = bits
         self._check(self._lib.thr_dense_deleted_set(self._h, _ptr(bits)))
 
-    def dense_topk(self, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None
-                   ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    def dense_topk(self, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None,
+                   d_scan: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
         """-> ids [B,k] int64, scores [B,k] float64, count [B] int32, gap [B] float32.
-        want: int32 [B] on the device — restrict query q to chunks tagged want[q] (< 0: no restriction)."""
+        want: int32 [B] on the device — restrict query q to chunks tagged want[q] (< 0: no restriction).
+        d_scan: score over the leading d_scan columns only (thr_dense_topk_prefix: the first step of the prefix funnel;
+        scores and gap are then the prefix's)."""
         Q = self._dev(Q, torch.bfloat16, "Q")
         B = Q.shape[0]
         if want is not None:
@@ -155,9 +157,46 @@ class Engine:
         sc = torch.empty((B, k), dtype=torch.float64, device=self.device)
         cnt = torch.empty((B,), dtype=torch.int32, device=self.device)
         gap = torch.empty((B,), dtype=torch.float32, device=self.device)
-        self._check(self._lib.thr_dense_topk_tagged(self._h, _ptr(Q), B, k, margin, _ptr(want), _ptr(ids), _ptr(sc),
-                                                    _ptr(cnt), _ptr(gap), self._stream()))
+        if d_scan is None:
+            self._check(self._lib.thr_dense_topk_tagged(self._h, _ptr(Q), B, k, margin, _ptr(want), _ptr(ids), _ptr(sc),
+                                                        _ptr(cnt), _ptr(gap), self._stream()))
+        else:
+            self._check(self._lib.thr_dense_topk_prefix(self._h, _ptr(Q), B, k, margin, _ptr(want), int(d_scan),
+                                                        _ptr(ids), _ptr(sc), _ptr(cnt), _ptr(gap), self._stream()))
         return ids, sc, cnt, gap
+
+    def dense_rescore(self, Q: torch.Tensor, ids: torch.Tensor, count: torch.Tensor) -> torch.Tensor:
+        """Full-width fp64 scores of a candidate pool (thr_dense_rescore): Q [B, D] bf16, ids [B, P] global ids (-1
+        padded), count [B] -> [B, P] float64, -inf where this handle does not hold the row and past count."""
+        Q = self._dev(Q, torch.bfloat16, "Q")
+        ids = self._dev(ids, torch.int64, "ids")
+        count = self._dev(count, torch.int32, "count")
+        B, P = ids.shape
+        if Q.shape[0] != B or count.numel() != B:
+            raise ValueError("Q, ids and count must have one row per query")
+        out = torch.empty((B, P), dtype=torch.float64, device=self.device)
+        self._check(self._lib.thr_dense_rescore(self._h, _ptr(Q), B, _ptr(ids), _ptr(count), P, _ptr(out),
+                                                self._stream()))
+        return out
+
+    def dense_funnel_finish(self, ids: torch.Tensor, count: torch.Tensor, scores: Sequence[torch.Tensor], k: int):
+        """The top k of a re-scored pool (thr_dense_funnel_finish): ids [B, P], count [B] and S score arrays [B, P]
+        float64 (dense_rescore outputs; they may live on GPUs this handle peers with) -> ids [B, k], scores [B, k]
+        float64, count [B] in dense_topk's format."""
+        ids = self._dev(ids, torch.int64, "ids")
+        count = self._dev(count, torch.int32, "count")
+        B, P = ids.shape
+        if not scores:
+            raise ValueError("dense_funnel_finish: no score arrays")
+        for t in scores:
+            _src(t, torch.float64, (B, P), "scores")
+        tab = self._ptr_table(scores)
+        o_ids = torch.empty((B, k), dtype=torch.int64, device=self.device)
+        o_sc = torch.empty((B, k), dtype=torch.float64, device=self.device)
+        o_cnt = torch.empty((B,), dtype=torch.int32, device=self.device)
+        self._check(self._lib.thr_dense_funnel_finish(self._h, B, P, k, _ptr(ids), _ptr(count), _ptr(tab), len(scores),
+                                                      _ptr(o_ids), _ptr(o_sc), _ptr(o_cnt), self._stream()))
+        return o_ids, o_sc, o_cnt
 
     # -- K2 BM25 ----------------------------------------------------------------------------
     def bm25_index_set(self, skip: torch.Tensor, postings: torch.Tensor, idf: torch.Tensor, n_docs: int,

@@ -20,6 +20,7 @@ import torch
 
 from .fusion import rag1_rrf_fusion
 from .index import pack_queries
+from .pipeline import DenseFunnel
 from .retriever import ResidentIndex, dense_error_bound, pad_dim
 
 
@@ -67,7 +68,11 @@ class GpuHybridSearcher:
     (`source_document`, `chunk_index`, `category`, `title`, `is_table`, ...); `collection` serves as `category`."""
 
     def __init__(self, org_id: str, index: ResidentIndex, config: Optional[SearchConfig] = None, embedder: Any = None,
-                 reranker: Any = None):
+                 reranker: Any = None, dense_funnel: Optional[DenseFunnel] = None):
+        """dense_funnel: run `_vector_search` through the prefix funnel (pipeline.DenseFunnel); None: the exact scan."""
+        if dense_funnel is not None and not isinstance(dense_funnel, DenseFunnel):
+            raise TypeError("dense_funnel must be a pipeline.DenseFunnel or None")
+        self.dense_funnel = dense_funnel
         self.org_id = org_id
         self.index = index
         self.engine = index.engine
@@ -94,10 +99,14 @@ class GpuHybridSearcher:
             raise ValueError(f"query embedding has {q.shape[1]} dimensions, the index {ix.dim}")
         q = q / q.norm(dim=1, keepdim=True).clamp_min(1e-30)
         k = max(1, min(self.config.top_k_retrieve, ix.n_live, 228))
+        fn = self.dense_funnel
+        if fn is not None and self.config.top_k_retrieve > fn.pool:
+            raise ValueError(f"top_k_retrieve {self.config.top_k_retrieve} > the dense funnel's pool of {fn.pool}")
         with eng.lock:
-            ids, sc, cnt, gap = ix.dense_topk(pad_dim(q.to(torch.bfloat16)).to(eng.device), k, want=ix.want(category))
+            ids, sc, cnt, gap = ix.dense_topk(pad_dim(q.to(torch.bfloat16)).to(eng.device), k, want=ix.want(category),
+                                              funnel=fn)
             ix.sync()
-        if float(gap[0]) <= dense_error_bound(ix.X.shape[1], 1.01, 1.01):
+        if float(gap[0]) <= dense_error_bound(ix.X.shape[1] if fn is None else fn.dims, 1.01, 1.01):
             import warnings
             warnings.warn("dense top-k: exactness certificate not met", RuntimeWarning)
         out = [self._result(i, "vector", similarity_score=s) for i, s in zip(ids[0, :int(cnt[0])].tolist(), sc[0, :int(cnt[0])].tolist())]

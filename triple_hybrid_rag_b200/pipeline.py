@@ -101,6 +101,46 @@ def maxsim_store(engine: Engine, Qtok: torch.Tensor, store, cand: torch.Tensor, 
     return engine.maxsim_packed(Qtok, store, cand, q_len=q_len)
 
 
+@dataclass(frozen=True)
+class DenseFunnel:
+    """The prefix funnel of the semantic channel, for Matryoshka embeddings: rank the corpus by the dot product over
+    the first `dims` columns, keep the best `pool`, re-score those at full width and return the top k (include/thr.h,
+    thr_dense_topk_prefix).  The scan reads dims / D of the bytes; the result is exactly defined, but it is the full
+    scan's only when the true top k lie in the prefix pool.  The certificate a funnel search returns covers the pool."""
+    dims: int
+    pool: int
+
+    def __post_init__(self):
+        if not isinstance(self.dims, int) or not isinstance(self.pool, int):
+            raise TypeError("DenseFunnel: dims and pool must be ints")
+        if self.dims < 64 or self.dims % 64:
+            raise ValueError(f"DenseFunnel: dims = {self.dims} must be a positive multiple of 64")
+        if self.pool < 1:
+            raise ValueError(f"DenseFunnel: pool = {self.pool} must be >= 1")
+
+    def check(self, D: int, k: int, margin: int) -> None:
+        """The conditions that depend on the index and the call: dims <= D, k <= pool, pool + margin <= 256."""
+        if self.dims > D:
+            raise ValueError(f"DenseFunnel: dims = {self.dims} exceeds the index's {D} columns")
+        if k > self.pool:
+            raise ValueError(f"DenseFunnel: k = {k} exceeds the pool of {self.pool}")
+        if self.pool + margin > 256:
+            raise ValueError(f"DenseFunnel: pool + margin = {self.pool + margin} exceeds 256")
+
+
+def dense_topk_one(engine: Engine, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None,
+                   funnel: Optional[DenseFunnel] = None):
+    """K1 on one handle (Engine.dense_topk's results).  With a funnel: the prefix K1 with k = pool, the full-width
+    re-score of the pool and its top k (thr_dense_topk_prefix -> thr_dense_rescore -> thr_dense_funnel_finish); the gap
+    is then the pool's certificate."""
+    if funnel is None:
+        return engine.dense_topk(Q, k, margin, want=want)
+    funnel.check(Q.shape[1], k, margin)
+    p_ids, _, p_cnt, gap = engine.dense_topk(Q, funnel.pool, margin, want=want, d_scan=funnel.dims)
+    ids, sc, cnt = engine.dense_funnel_finish(p_ids, p_cnt, [engine.dense_rescore(Q, p_ids, p_cnt)], k)
+    return ids, sc, cnt, gap
+
+
 @dataclass
 class SearchOutput:
     ids: torch.Tensor        # [B, top_k] int64, -1 padded
@@ -208,17 +248,20 @@ class TripleHybridSearcher:
                graph_ids: Optional[torch.Tensor], weights: Optional[torch.Tensor] = None,
                k_sem: int = 100, k_lex: int = 100, top_k: int = 100, margin: int = 28,
                tie_mode: int = _lib.TIE_CHUNK_ID, rrf_k: int = 60, want: Optional[torch.Tensor] = None,
-               require_all: bool = False, lex_delta: Optional[Engine] = None) -> SearchOutput:
+               require_all: bool = False, lex_delta: Optional[Engine] = None,
+               funnel: Optional[DenseFunnel] = None) -> SearchOutput:
         """want: int32 [B] on the device — per query, the tag its semantic and lexical hits must carry (< 0: any);
         needs set_tags.  require_all: AND semantics of the lexical channel (thr_bm25_topk_ex).  lex_delta: the handle
         of a lexical delta segment (ResidentIndex.delta_engine), searched and merged with the main list; single GPU
-        only.  The graph list is an
-        input and is taken as given.  SearchOutput.gap is K1's exactness certificate of THIS shard (compare with
-        dense_error_bound; `certify` does it on the host)."""
+        only.  funnel: the semantic channel through the prefix funnel (DenseFunnel; single GPU only).  The graph list is
+        an input and is taken as given.  SearchOutput.gap is K1's exactness certificate of THIS shard (compare with
+        dense_error_bound; `certify` does it on the host); with a funnel it certifies the prefix pool."""
         eng, dev = self.engine, self.engine.device
         B = Q.shape[0]
         if lex_delta is not None and self.world > 1:
             raise NotImplementedError("a lexical delta segment is not supported with a sharded corpus")
+        if funnel is not None and self.world > 1:
+            raise NotImplementedError("the dense funnel is not supported with a process group")
         if self.overlap:
             # The two channels do not depend on each other: K2's chain (plan, range kernel, unit merge) goes on a
             # second stream and K1's (seed, select, score, finalize) on a high-priority one.  Both big kernels take
@@ -234,13 +277,13 @@ class TripleHybridSearcher:
                 l_ids, l_sc, l_cnt = bm25_topk_segments(eng, lex_delta, q_terms, q_off, k_lex, want=want,
                                                         require_all=require_all)
             with torch.cuda.stream(s_dense):
-                d_ids, d_sc, d_cnt, gap = eng.dense_topk(Q, k_sem, margin, want=want)
+                d_ids, d_sc, d_cnt, gap = dense_topk_one(eng, Q, k_sem, margin, want=want, funnel=funnel)
             main.wait_stream(s_dense)
             main.wait_stream(s_lex)
             for t in (l_ids, l_sc, l_cnt, d_ids, d_sc, d_cnt, gap):   # allocated on the side streams, consumed on `main`
                 t.record_stream(main)
         else:
-            d_ids, d_sc, d_cnt, gap = eng.dense_topk(Q, k_sem, margin, want=want)
+            d_ids, d_sc, d_cnt, gap = dense_topk_one(eng, Q, k_sem, margin, want=want, funnel=funnel)
             l_ids, l_sc, l_cnt = bm25_topk_segments(eng, lex_delta, q_terms, q_off, k_lex, want=want,
                                                     require_all=require_all)
         if self.world > 1:
@@ -464,19 +507,25 @@ class ShardedSearcher:
                graph_ids: Optional[torch.Tensor], weights: Optional[torch.Tensor] = None,
                k_sem: int = 100, k_lex: int = 100, top_k: int = 100, margin: int = 28,
                tie_mode: int = _lib.TIE_CHUNK_ID, rrf_k: int = 60, want: Optional[torch.Tensor] = None,
-               require_all: bool = False, lex_delta: Optional[Engine] = None) -> SearchOutput:
+               require_all: bool = False, lex_delta: Optional[Engine] = None,
+               funnel: Optional[DenseFunnel] = None) -> SearchOutput:
         """TripleHybridSearcher.search's arguments; inputs on the home GPU.  lex_delta: the handle of the LAST shard's
         lexical delta segment (its ids follow that shard's rows); it is one more lexical source of the merge.
-        SearchOutput.gap is the merged list's certificate: the minimum of the shards' gaps."""
+        SearchOutput.gap is the merged list's certificate: the minimum of the shards' gaps (with a funnel: of the
+        merged prefix pool)."""
         B = Q.shape[0]
         d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt = self._topk(B, Q, q_terms, q_off, k_sem, k_lex, margin, want,
-                                                                 require_all, lex_delta)
+                                                                 require_all, lex_delta, funnel)
         return self._home._fuse(B, d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt, graph_ids, weights, top_k, tie_mode,
                                 rrf_k)
 
-    def dense_topk(self, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None):
-        """K1 on every shard, merged: Engine.dense_topk's results (gap: the minimum of the shards')."""
-        d_ids, d_sc, d_cnt, gap, _, _, _ = self._topk(Q.shape[0], Q, None, None, k, 1, margin, want, False, None)
+    def dense_topk(self, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None,
+                   funnel: Optional[DenseFunnel] = None):
+        """K1 on every shard, merged: Engine.dense_topk's results (gap: the minimum of the shards').  With a funnel:
+        the shards' prefix top-pool lists merged into the global pool, each pool row re-scored on the shard that holds
+        it, and the top k of the pool (dense_topk_one's result, whatever the sharding)."""
+        d_ids, d_sc, d_cnt, gap, _, _, _ = self._topk(Q.shape[0], Q, None, None, k, 1, margin, want, False, None,
+                                                      funnel)
         return d_ids, d_sc, d_cnt, gap
 
     def bm25_topk(self, q_terms: torch.Tensor, q_off: torch.Tensor, k: int, want: Optional[torch.Tensor] = None,
@@ -496,9 +545,15 @@ class ShardedSearcher:
                     torch.full((B,), float("inf"), dtype=torch.float32, device=dev))
         return ids, torch.zeros((B, k), dtype=torch.float32, device=dev), cnt
 
-    def _topk(self, B, Q, q_terms, q_off, k_sem, k_lex, margin, want, require_all, lex_delta):
+    def _topk(self, B, Q, q_terms, q_off, k_sem, k_lex, margin, want, require_all, lex_delta, funnel=None):
         """Both channels (Q None: no semantic search; q_terms None: no lexical one) on every shard, merged on the
-        home GPU in one thr_shard_merge launch -> d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt."""
+        home GPU in one thr_shard_merge launch -> d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt.  With a funnel the
+        semantic lists are the shards' prefix pools, and the merged pool is finished by _funnel_finish."""
+        k_out = k_sem
+        d_scan = None
+        if funnel is not None and Q is not None:
+            funnel.check(Q.shape[1], k_sem, margin)
+            k_sem, d_scan = funnel.pool, funnel.dims
         home = self.engine
         main = torch.cuda.current_stream(home.device)
         last = len(self.engines) - 1
@@ -515,7 +570,8 @@ class ShardedSearcher:
                 for s in shards:
                     e = self.engines[s]
                     if Q is not None:
-                        sem.append((s, tuple(self._home_view(s, t) for t in e.dense_topk(q, k_sem, margin, want=w))))
+                        sem.append((s, tuple(self._home_view(s, t)
+                                             for t in e.dense_topk(q, k_sem, margin, want=w, d_scan=d_scan))))
                     if q_terms is not None:
                         l = e.bm25_topk(qt, qo, k_lex, want=w, require_all=require_all)
                         lex.append((s, tuple(self._home_view(s, t) for t in l)))
@@ -527,7 +583,30 @@ class ShardedSearcher:
         # a fixed source order (shard order, the delta segment last), whatever the grouping by GPU
         sem = [x for _, x in sorted(sem, key=lambda p: p[0])] or [self._empty(B, k_sem, True)]
         lex = [x for _, x in sorted(lex, key=lambda p: p[0])] or [self._empty(B, k_lex, False)]
-        return home.shard_merge(B, k_sem, k_lex, sem, lex)
+        out = home.shard_merge(B, k_sem, k_lex, sem, lex)
+        if d_scan is None:
+            return out
+        d_ids, d_sc, d_cnt = self._funnel_finish(Q, out[0], out[2], k_out)
+        return (d_ids, d_sc, d_cnt) + tuple(out[3:])
+
+    def _funnel_finish(self, Q, ids, cnt, k):
+        """The merged prefix pool (ids [B, pool], cnt [B] on the home GPU) re-scored at full width, each row on the
+        shard that holds it (thr_dense_rescore: -inf elsewhere), and its top k on the home GPU (thr_dense_funnel_finish
+        over the shards' score arrays).  The pool is copied to every other GPU, as the rerank stage copies its ids."""
+        home = self.engine
+        main = torch.cuda.current_stream(home.device)
+        scores = [None] * len(self.engines)
+        for dev, st, shards in self._groups():
+            if st is not main:
+                st.wait_stream(main)
+            with torch.cuda.device(dev), torch.cuda.stream(st):
+                q, i, c = (Q, ids, cnt) if dev == home.device else \
+                    (t.to(dev, non_blocking=True) for t in (Q, ids, cnt))
+                for s in shards:
+                    scores[s] = self._home_view(s, self.engines[s].dense_rescore(q, i, c))
+            if st is not main:
+                main.wait_stream(st)
+        return home.dense_funnel_finish(ids, cnt, scores, k)
 
     def rerank(self, out: SearchOutput, Qtok: torch.Tensor, C: int, threshold: float, alpha: float, final_top_k: int,
                q_len: Optional[torch.Tensor] = None) -> SearchOutput:

@@ -17,7 +17,8 @@ import torch
 
 from .engine import Engine
 from .index import BM25Index, bm25_idf
-from .pipeline import ShardedSearcher, TripleHybridSearcher, bm25_topk_segments, maxsim_store
+from .pipeline import (DenseFunnel, ShardedSearcher, TripleHybridSearcher, bm25_topk_segments, dense_topk_one,
+                       maxsim_store)
 from .tokpack import Codebook, PackedTokenStore, encode as encode_tokens
 
 _WORD = re.compile(r"\w+", re.UNICODE)
@@ -381,12 +382,14 @@ class ResidentIndex:
                 ts.set_token_store(sh.store, sh.lo, sh.top, lens=sh.lens)
         return s
 
-    def dense_topk(self, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None):
+    def dense_topk(self, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None,
+                   funnel: Optional[DenseFunnel] = None):
         """K1 over the embedding rows (Engine.dense_topk's arguments and results; over several shards the certificate
-        is the minimum of theirs)."""
+        is the minimum of theirs).  funnel: through the prefix funnel (pipeline.DenseFunnel); the same result for any
+        sharding, and the certificate is the prefix pool's."""
         if self.n_shards == 1:
-            return self.engine.dense_topk(Q, k, margin, want=want)
-        return self.searcher().dense_topk(Q, k, margin, want=want)
+            return dense_topk_one(self.engine, Q, k, margin, want=want, funnel=funnel)
+        return self.searcher().dense_topk(Q, k, margin, want=want, funnel=funnel)
 
     def bm25_topk(self, q_terms: torch.Tensor, q_off: torch.Tensor, k: int, want: Optional[torch.Tensor] = None,
                   require_all: bool = False):

@@ -37,6 +37,7 @@ import torch
 from . import _lib
 from .engine import Engine
 from .index import pack_queries
+from .pipeline import DenseFunnel
 from .resident import (PORTUGUESE_STOPWORDS, ResidentIndex, Tokenizer, light_stem_pt, pack_bitmap,  # noqa: F401
                        pad_dim, tokenize)
 
@@ -147,9 +148,12 @@ class _GpuScoring:
 
     _cfg = SETTINGS
 
-    def _gpu_init(self, index, engine, graph_search, token_encoder, lexical_match):
+    def _gpu_init(self, index, engine, graph_search, token_encoder, lexical_match, dense_funnel=None):
         if lexical_match not in ("all", "any"):
             raise ValueError("lexical_match must be 'all' (the reference's plainto_tsquery AND) or 'any' (BM25 OR)")
+        if dense_funnel is not None and not isinstance(dense_funnel, DenseFunnel):
+            raise TypeError("dense_funnel must be a pipeline.DenseFunnel or None")
+        self.dense_funnel = dense_funnel
         self.index = index
         self.engine = engine or (index.engine if index is not None else None)
         self._graph_search_fn = graph_search
@@ -204,21 +208,27 @@ class _GpuScoring:
         """Reference: retrieval.py:294-314 (embed the query, top-`limit` by cosine similarity, best first).
         Exact: the result carries K1's certificate (gap above the fp32 accumulation bound); an uncertified result is
         recomputed once with the widest re-scoring margin and, if still uncertified (more exact ties than the
-        margin holds), returned with a RuntimeWarning."""
-        eng, ix = self._need_engine(), self.index
+        margin holds), returned with a RuntimeWarning.  With the retriever's dense_funnel the search goes through the
+        prefix funnel, and the certificate (over its `dims` columns) is the prefix pool's."""
+        eng, ix, fn = self._need_engine(), self.index, self.dense_funnel
         q = torch.as_tensor(self.embedder.embed_query(query_text), dtype=torch.float32).reshape(1, -1)
         if q.shape[1] != ix.dim:
             raise ValueError(f"query embedding has {q.shape[1]} dimensions, the index {ix.dim}")
         q = q / q.norm(dim=1, keepdim=True).clamp_min(1e-30)
         k = min(limit, ix.n_live)
-        if k > 252:
+        depth = k if fn is None else fn.pool     # the list K1 selects: k, or the funnel's pool
+        if fn is not None:
+            if limit > fn.pool:
+                raise ValueError(f"semantic limit {limit} > the dense funnel's pool of {fn.pool}")
+            fn.check(ix.X.shape[1], max(k, 1), max(0, min(28, 256 - depth)))
+        elif k > 252:
             raise ValueError(f"semantic limit {limit} > 252 (K1 re-scores k + margin <= 256 survivors)")
         qd = pad_dim(q.to(torch.bfloat16)).to(eng.device)
         want = ix.want(collection)
-        bound = dense_error_bound(ix.X.shape[1], 1.01, 1.01)
-        for margin in (min(28, 256 - k), 256 - k):
+        bound = dense_error_bound(ix.X.shape[1] if fn is None else fn.dims, 1.01, 1.01)
+        for margin in (min(28, 256 - depth), 256 - depth):
             with eng.lock:
-                ids, sc, cnt, gap = ix.dense_topk(qd, max(k, 1), margin, want=want)            # predicate inside K1
+                ids, sc, cnt, gap = ix.dense_topk(qd, max(k, 1), margin, want=want, funnel=fn)  # predicate inside K1
                 ix.sync()
             if float(gap[0]) > bound:
                 break
@@ -374,8 +384,12 @@ class _GpuScoring:
         if collections is not None and any(c is not None for c in collections):
             want = torch.tensor([-1 if c is None else ix.tag_of.get(c, 0xfffe) for c in collections], dtype=torch.int32,
                                 device=eng.device)
+        fn = self.dense_funnel
+        if fn is not None and k_sem > fn.pool:
+            raise ValueError(f"k_sem {k_sem} > the dense funnel's pool of {fn.pool}")
         out = s.search(Q, qt, qo, g, weights=wt, k_sem=max(1, min(k_sem, ix.n_live)), k_lex=k_lex, top_k=top_k,
-                       want=want, require_all=self.lexical_match == "all", tie_mode=tie_mode, lex_delta=ix.delta_engine)
+                       want=want, require_all=self.lexical_match == "all", tie_mode=tie_mode, lex_delta=ix.delta_engine,
+                       funnel=fn)
         ix.sync()
         ids, rrf, rk, cnt = out.ids.tolist(), out.rrf.tolist(), out.ranks.tolist(), out.count.tolist()
         res = []
@@ -412,17 +426,20 @@ class StandaloneGpuRAG2Retriever(_GpuScoring):
     def __init__(self, org_id: str, embedder: Any = None, query_planner: Any = None, graph_enabled: bool = False, *,
                  index: Optional[ResidentIndex] = None, engine: Optional[Engine] = None,
                  graph_search: Optional[Callable[..., Sequence[str]]] = None,
-                 token_encoder: Optional[Callable[[str], torch.Tensor]] = None, lexical_match: str = "all"):
+                 token_encoder: Optional[Callable[[str], torch.Tensor]] = None, lexical_match: str = "all",
+                 dense_funnel: Optional[DenseFunnel] = None):
         """org_id / embedder / query_planner / graph_enabled: as in the reference (retrieval.py:79-101).
         index: the tenant's ResidentIndex.  graph_search(cypher=, keywords=, collection=, limit=) -> ranked
         child ids, or an object with `.chunk_ids` like the reference's GraphSearchResult (the graph engine stays
         external).  token_encoder(query) -> [Tq, 128] token embeddings.  lexical_match: "all" = every keyword must
-        match, the reference's `tsv @@ plainto_tsquery` (20260114_rag2_schema.sql:369); "any" = plain BM25 (OR)."""
+        match, the reference's `tsv @@ plainto_tsquery` (20260114_rag2_schema.sql:369); "any" = plain BM25 (OR).
+        dense_funnel: run the semantic channel through the prefix funnel (pipeline.DenseFunnel: scan the leading
+        `dims` columns, re-score a pool of `pool` at full width); None: the exact full-width scan."""
         self.org_id = org_id
         self.embedder = embedder
         self.query_planner = query_planner or FallbackQueryPlanner(self._cfg)   # the reference: get_query_planner()
         self.graph_enabled = graph_enabled and self._cfg.rag2_graph_enabled
-        self._gpu_init(index, engine, graph_search, token_encoder, lexical_match)
+        self._gpu_init(index, engine, graph_search, token_encoder, lexical_match, dense_funnel)
 
     # ---- pipeline (reference: retrieval.py:118-201) ---------------------------------------------
     async def retrieve(self, query: str, collection: Optional[str] = None, top_k: Optional[int] = None,
@@ -612,9 +629,10 @@ def make_reference_subclass(ref=None, cfg=None):
         def __init__(self, org_id: str, embedder: Any = None, query_planner: Any = None, graph_enabled: bool = False, *,
                      index: Optional[ResidentIndex] = None, engine: Optional[Engine] = None,
                      graph_search: Optional[Callable[..., Sequence[str]]] = None,
-                     token_encoder: Optional[Callable[[str], torch.Tensor]] = None, lexical_match: str = "all"):
+                     token_encoder: Optional[Callable[[str], torch.Tensor]] = None, lexical_match: str = "all",
+                     dense_funnel: Optional[DenseFunnel] = None):
             base.__init__(self, org_id, embedder=embedder, query_planner=query_planner, graph_enabled=graph_enabled)
-            self._gpu_init(index, engine, graph_search, token_encoder, lexical_match)
+            self._gpu_init(index, engine, graph_search, token_encoder, lexical_match, dense_funnel)
 
     return GpuRAG2Retriever
 
@@ -634,5 +652,5 @@ async def retrieve(org_id: str, query: str, **kwargs: Any) -> RetrievalResult:
     """Convenience wrapper with the reference's signature (retrieval.py:498-505); the tenant's index and
     engine come through kwargs (`index=`, `embedder=`, ...), retrieval arguments through the rest."""
     ctor = {k: kwargs.pop(k) for k in ("embedder", "query_planner", "graph_enabled", "index", "engine",
-                                       "graph_search", "token_encoder", "lexical_match") if k in kwargs}
+                                       "graph_search", "token_encoder", "lexical_match", "dense_funnel") if k in kwargs}
     return await GpuRAG2Retriever(org_id=org_id, **ctor).retrieve(query, **kwargs)
