@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define THR_ABI_VERSION 14
+#define THR_ABI_VERSION 15
 
 enum {
   THR_OK = 0,
@@ -232,6 +232,34 @@ enum { THR_BM25_REQUIRE_ALL = 1 };
 int thr_bm25_topk_ex(thr_handle* h, const int32_t* q_terms, const int32_t* q_off, int B, int k,
                      const int32_t* want, int flags, int64_t* out_ids, float* out_scores, int32_t* out_count,
                      void* stream);
+
+/* ---- document-scoped search: the exact top-k over a per-query list of rows ------------------
+ * The questions users ask about particular documents ("what does this contract say about cancellation"): each query
+ * carries its own scope, a list of global row ids built by the host from document ids, and is answered exactly over
+ * those rows by scoring them directly — |scope| * D * 2 bytes read instead of a corpus scan.
+ *   rows [off[B]] int64 global ids; query q's scope is rows[off[q] .. off[q+1]) (off [B+1] int64, non-decreasing).  Ids
+ *     must be unique within a query (the caller guarantees it); an id < 0 or not held by this handle (outside
+ *     [id_base, id_base + N)) is skipped, so every shard can be given the whole scope.  rows must not be NULL, also
+ *     when every scope is empty (any valid device address will do then: no row is read).
+ *   For query q, over the rows of its scope that are held, live (the deletion bitmap) and carry the tag want[q] (want
+ *   nullable as in the *_tagged calls; < 0 = any):
+ *   thr_dense_topk_rows: the min(k, eligible) rows with the largest fp64 dot product, ordered by (score desc, id asc),
+ *     each score bit-identical to thr_dense_topk's / thr_dense_rescore's for that row; every row is scored exactly, so
+ *     out_gap (nullable) is +inf.  Output format of thr_dense_topk (ids -1 and scores -inf past out_count).
+ *   thr_bm25_topk_rows: thr_bm25_topk_ex's definition restricted to the scope (same terms, flags, idf, repeated and
+ *     out-of-range term ids, score bits and eligibility), output format of thr_bm25_topk (ids -1, scores 0 past count).
+ *     Each query term's posting of a row is found by a binary search of the row's skip range.
+ * Equivalently: the result is K1's / K2's on the same handle with every row outside the scope added to the deletion
+ * bitmap (ids, score bits and counts).  1 <= k <= 256; at most 32 terms per query, as thr_bm25_topk.  Two launches (a
+ * scoring pass over fixed slices of the concatenated scopes writing per-slice top-k lists, one reduction per query);
+ * scratch ~12 (2 SMs + B) k bytes in the channel's arena.  Timed in THR_PROF_DENSE_SCORE / THR_PROF_BM25.
+ */
+int thr_dense_topk_rows(thr_handle* h, const void* Q, int B, const int64_t* rows, const int64_t* off, int k,
+                        const int32_t* want, int64_t* out_ids, double* out_scores, int32_t* out_count, float* out_gap,
+                        void* stream);
+int thr_bm25_topk_rows(thr_handle* h, const int32_t* q_terms, const int32_t* q_off, int B, const int64_t* rows,
+                       const int64_t* off, int k, const int32_t* want, int flags, int64_t* out_ids, float* out_scores,
+                       int32_t* out_count, void* stream);
 
 /* ---- K3: weighted RRF fusion + safety threshold + conformal denoise ---------------
  * Replaces, bit-exactly in fp64:

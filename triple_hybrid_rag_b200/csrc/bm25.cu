@@ -815,6 +815,14 @@ void thr_bm25_state_free(thr_handle* h) {
   }
 }
 
+int thr_bm25_view_get(thr_handle* h, thr_bm25_view* v) {
+  const thr_bm25_state* st = h->bm25;
+  if (!st) return thr_fail(h, THR_ENOINDEX, "call thr_bm25_index_set first");
+  v->skip = st->skip; v->post = st->post; v->idf = st->idf; v->n_docs = st->n_docs; v->id_base = st->id_base;
+  v->n_blk = st->n_blk; v->blk_shift = st->blk_shift; v->V = st->V; v->tags = st->tags; v->deleted = st->deleted;
+  return THR_OK;
+}
+
 static int bm25_topk_impl(thr_handle* h, const int32_t* q_terms, const int32_t* q_off, int B, int k,
                           const int32_t* want, int require_all, int64_t* out_ids, float* out_scores,
                           int32_t* out_count, void* stream);

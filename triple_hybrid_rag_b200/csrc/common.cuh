@@ -55,6 +55,27 @@ void* thr_scratch(thr_handle* h, int arena, size_t bytes);
 int thr_encode_tma_2d_bf16(thr_handle* h, CUtensorMap* map, const void* base, uint64_t rows,
                            uint64_t cols, uint32_t box_rows, uint32_t box_cols, uint64_t ld = 0);
 
+// What a handle's indexes hold, for kernels outside the file that owns the index state (scope.cu).
+// THR_ENOINDEX (with the message set) when the index is not set.
+struct thr_dense_view {
+  const void* X;              // bf16 [N, D]
+  int64_t N, id_base;
+  int D;
+  const uint16_t* tags;       // nullable
+  const uint32_t* deleted;    // nullable
+};
+struct thr_bm25_view {
+  const int64_t* skip;        // [V * n_blk + 1]
+  const void* post;           // {u32 doc, f32 impact} records
+  const float* idf;
+  int64_t n_docs, id_base;
+  int n_blk, blk_shift, V;
+  const uint16_t* tags;       // nullable
+  const uint32_t* deleted;    // nullable
+};
+int thr_dense_view_get(thr_handle* h, thr_dense_view* v);
+int thr_bm25_view_get(thr_handle* h, thr_bm25_view* v);
+
 #define THR_CUDA(h, expr)                                                              \
   do {                                                                                 \
     cudaError_t _e = (expr);                                                           \
@@ -450,4 +471,36 @@ __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&r)[32])
 }
 __device__ __forceinline__ void tmem_ld_wait() {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+}
+
+// ---- the exact dense re-score ---------------------------------------------------------------
+// The exact re-score: fp64 dot of the bf16 inputs over columns [0, D) of kInFlight rows of X (row pitch ld) with the
+// query row qrow (shared memory), by one warp in a fixed summation order: lane l accumulates columns l*8 .. l*8+7 of
+// every 256-column block with fma, then an xor-shuffle reduction.  Every lane returns the sums.  Four rows are in
+// flight so that their scattered row reads overlap.  K1's finalize, thr_dense_rescore and thr_dense_topk_rows all call
+// it, so a row's score is the same bits in each.
+constexpr int kInFlight = 4;
+__device__ __forceinline__ void rescore_rows(const __nv_bfloat16* X, int64_t ld, int D, const uint32_t (&idx)[kInFlight],
+                                             const __nv_bfloat16* qrow, int lane, double (&acc)[kInFlight]) {
+#pragma unroll
+  for (int u = 0; u < kInFlight; ++u) acc[u] = 0.0;
+  for (int d0 = lane * 8; d0 < D; d0 += 256) {
+    uint4 xv[kInFlight];
+#pragma unroll
+    for (int u = 0; u < kInFlight; ++u) xv[u] = *reinterpret_cast<const uint4*>(X + (size_t)idx[u] * ld + d0);
+    double qd[8];
+#pragma unroll
+    for (int e = 0; e < 8; ++e) qd[e] = (double)__bfloat162float(qrow[d0 + e]);
+#pragma unroll
+    for (int u = 0; u < kInFlight; ++u) {
+      const __nv_bfloat16* xe = reinterpret_cast<const __nv_bfloat16*>(&xv[u]);
+#pragma unroll
+      for (int e = 0; e < 8; ++e) acc[u] = fma((double)__bfloat162float(xe[e]), qd[e], acc[u]);
+    }
+  }
+#pragma unroll
+  for (int u = 0; u < kInFlight; ++u) {
+#pragma unroll
+    for (int sh = 16; sh > 0; sh >>= 1) acc[u] += __shfl_xor_sync(0xffffffffu, acc[u], sh);
+  }
 }

@@ -427,37 +427,6 @@ struct FinalArgs {
   float* out_gap;
 };
 
-// The exact re-score: fp64 dot of the bf16 inputs over columns [0, D) of kInFlight rows of X (row pitch ld) with the
-// query row qrow (shared memory), by one warp in a fixed summation order: lane l accumulates columns l*8 .. l*8+7 of
-// every 256-column block with fma, then an xor-shuffle reduction.  Every lane returns the sums.  Four rows are in
-// flight so that their scattered row reads overlap.  K1's finalize and thr_dense_rescore both call it, so a row's score
-// is the same bits in either.
-constexpr int kInFlight = 4;
-__device__ __forceinline__ void rescore_rows(const __nv_bfloat16* X, int64_t ld, int D, const uint32_t (&idx)[kInFlight],
-                                             const __nv_bfloat16* qrow, int lane, double (&acc)[kInFlight]) {
-#pragma unroll
-  for (int u = 0; u < kInFlight; ++u) acc[u] = 0.0;
-  for (int d0 = lane * 8; d0 < D; d0 += 256) {
-    uint4 xv[kInFlight];
-#pragma unroll
-    for (int u = 0; u < kInFlight; ++u) xv[u] = *reinterpret_cast<const uint4*>(X + (size_t)idx[u] * ld + d0);
-    double qd[8];
-#pragma unroll
-    for (int e = 0; e < 8; ++e) qd[e] = (double)__bfloat162float(qrow[d0 + e]);
-#pragma unroll
-    for (int u = 0; u < kInFlight; ++u) {
-      const __nv_bfloat16* xe = reinterpret_cast<const __nv_bfloat16*>(&xv[u]);
-#pragma unroll
-      for (int e = 0; e < 8; ++e) acc[u] = fma((double)__bfloat162float(xe[e]), qd[e], acc[u]);
-    }
-  }
-#pragma unroll
-  for (int u = 0; u < kInFlight; ++u) {
-#pragma unroll
-    for (int sh = 16; sh > 0; sh >>= 1) acc[u] += __shfl_xor_sync(0xffffffffu, acc[u], sh);
-  }
-}
-
 // Order n <= kMaxSel (score, id) pairs by (score desc, id asc) without barriers: element e = tid / P is counted by P
 // adjacent threads (P = kFinalThreads / the next power of two >= max(n, 32)), each over every P-th other element.  The
 // pairs are distinct, so the ranks are a permutation.  Every thread of the CTA must call it; it returns the rank of
@@ -898,6 +867,13 @@ struct thr_dense_state {
 
 void thr_dense_state_free(thr_handle* h) {
   if (h->dense) { free(h->dense); h->dense = nullptr; }
+}
+
+int thr_dense_view_get(thr_handle* h, thr_dense_view* v) {
+  const thr_dense_state* st = h->dense;
+  if (!st) return thr_fail(h, THR_ENOINDEX, "call thr_dense_index_set first");
+  v->X = st->X; v->N = st->N; v->id_base = st->id_base; v->D = st->D; v->tags = st->tags; v->deleted = st->deleted;
+  return THR_OK;
 }
 
 template <int G>

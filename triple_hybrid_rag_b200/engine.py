@@ -247,6 +247,54 @@ class Engine:
                                                _ptr(sc), _ptr(cnt), self._stream()))
         return ids, sc, cnt
 
+    # -- document-scoped search ------------------------------------------------------------------
+    def _scope_args(self, rows: torch.Tensor, off: torch.Tensor, B: int):
+        rows = self._dev(rows, torch.int64, "rows")
+        off = self._dev(off, torch.int64, "off")
+        if rows.dim() != 1 or off.dim() != 1 or off.numel() != B + 1:
+            raise ValueError("rows must be 1-D and off [B + 1]")
+        if rows.numel() == 0:   # a zero-size tensor has a NULL data pointer; the kernels read no row of it
+            rows = torch.full((1,), -1, dtype=torch.int64, device=self.device)
+        return rows, off
+
+    def dense_topk_rows(self, Q: torch.Tensor, rows: torch.Tensor, off: torch.Tensor, k: int,
+                        want: Optional[torch.Tensor] = None):
+        """The exact top k of each query over its scope, rows[off[q]:off[q+1]] (int64 global ids; ids this handle
+        does not hold are skipped) (thr_dense_topk_rows) -> dense_topk's ids, scores, count, gap (+inf)."""
+        Q = self._dev(Q, torch.bfloat16, "Q")
+        B = Q.shape[0]
+        rows, off = self._scope_args(rows, off, B)
+        if want is not None:
+            want = self._dev(want, torch.int32, "want")
+            if want.numel() != B:
+                raise ValueError("want must have one entry per query")
+        ids = torch.empty((B, k), dtype=torch.int64, device=self.device)
+        sc = torch.empty((B, k), dtype=torch.float64, device=self.device)
+        cnt = torch.empty((B,), dtype=torch.int32, device=self.device)
+        gap = torch.empty((B,), dtype=torch.float32, device=self.device)
+        self._check(self._lib.thr_dense_topk_rows(self._h, _ptr(Q), B, _ptr(rows), _ptr(off), k, _ptr(want), _ptr(ids),
+                                                  _ptr(sc), _ptr(cnt), _ptr(gap), self._stream()))
+        return ids, sc, cnt, gap
+
+    def bm25_topk_rows(self, q_terms: torch.Tensor, q_off: torch.Tensor, rows: torch.Tensor, off: torch.Tensor, k: int,
+                       want: Optional[torch.Tensor] = None, require_all: bool = False):
+        """bm25_topk restricted to each query's scope, rows[off[q]:off[q+1]] (thr_bm25_topk_rows) -> bm25_topk's."""
+        q_terms = self._dev(q_terms, torch.int32, "q_terms")
+        q_off = self._dev(q_off, torch.int32, "q_off")
+        B = q_off.numel() - 1
+        rows, off = self._scope_args(rows, off, B)
+        if want is not None:
+            want = self._dev(want, torch.int32, "want")
+            if want.numel() != B:
+                raise ValueError("want must have one entry per query")
+        ids = torch.empty((B, k), dtype=torch.int64, device=self.device)
+        sc = torch.empty((B, k), dtype=torch.float32, device=self.device)
+        cnt = torch.empty((B,), dtype=torch.int32, device=self.device)
+        flags = _lib.BM25_REQUIRE_ALL if require_all else 0
+        self._check(self._lib.thr_bm25_topk_rows(self._h, _ptr(q_terms), _ptr(q_off), B, _ptr(rows), _ptr(off), k,
+                                                 _ptr(want), flags, _ptr(ids), _ptr(sc), _ptr(cnt), self._stream()))
+        return ids, sc, cnt
+
     # -- K3 fusion --------------------------------------------------------------------------
     def fuse(self, variant: int, B: int, lists: Sequence[Optional[Tuple[torch.Tensor, torch.Tensor, Optional[torch.Tensor]]]],
              weights: torch.Tensor, rrf_k: int = 60, safety_thr: float = 0.0, alpha: float = 0.0,

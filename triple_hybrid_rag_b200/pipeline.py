@@ -75,16 +75,59 @@ def exchange_topk(group, world, B, k_sem, k_lex, d_ids, d_sc, d_cnt, l_ids, l_sc
             l_ids, l_sc, m_cnt[B:].clamp(max=k_lex))
 
 
+@dataclass(frozen=True)
+class Scope:
+    """Per-query document scopes: query q is answered over the global rows rows[off[q]:off[q+1]] only
+    (ResidentIndex.scope builds one from document ids).  rows int64 [n] and off int64 [B + 1] on the device; a row
+    the index does not hold, or a deleted one, contributes nothing.  A scoped search scores its rows directly
+    (thr_dense_topk_rows / thr_bm25_topk_rows): exact in both channels, and the semantic channel never goes through a
+    DenseFunnel."""
+    rows: torch.Tensor
+    off: torch.Tensor
+
+    def __post_init__(self):
+        for name, t in (("rows", self.rows), ("off", self.off)):
+            if not isinstance(t, torch.Tensor) or t.dtype != torch.int64 or t.dim() != 1:
+                raise TypeError(f"Scope.{name}: expected a 1-D int64 tensor")
+        if self.off.numel() < 1 or self.rows.device != self.off.device:
+            raise ValueError("Scope: off needs B + 1 entries on the device of rows")
+
+    @property
+    def B(self) -> int:
+        return self.off.numel() - 1
+
+    def to(self, device) -> "Scope":
+        device = torch.device(device)
+        if self.off.device == device:
+            return self
+        return Scope(self.rows.to(device, non_blocking=True), self.off.to(device, non_blocking=True))
+
+
+def _check_scope(scope: Optional[Scope], B: int) -> None:
+    if scope is not None:
+        if not isinstance(scope, Scope):
+            raise TypeError("scope must be a pipeline.Scope or None")
+        if scope.B != B:
+            raise ValueError(f"scope has {scope.B} queries, the batch {B}")
+
+
 def bm25_topk_segments(engine: Engine, delta: Optional[Engine], q_terms: torch.Tensor, q_off: torch.Tensor, k: int,
-                       want: Optional[torch.Tensor] = None, require_all: bool = False):
+                       want: Optional[torch.Tensor] = None, require_all: bool = False, scope: Optional[Scope] = None):
     """K2 over a main index and, when `delta` is a handle, a delta segment whose ids follow the main index's (its
     id_base): each segment's top-k, merged by K5 (G = 2).  fp32 -> fp64 -> fp32 is exact and K5 orders by (score
     desc, id asc) as K2 does, so the result is what one index over both segments returns.  -> Engine.bm25_topk's.
+    With a scope, each segment scores the scope's rows it holds (thr_bm25_topk_rows) instead.
     Sync both handles afterwards (ResidentIndex.sync): each reports its own device-side failures."""
-    ids, sc, cnt = engine.bm25_topk(q_terms, q_off, k, want=want, require_all=require_all)
+    _check_scope(scope, q_off.numel() - 1)
+
+    def run(e: Engine):
+        if scope is None:
+            return e.bm25_topk(q_terms, q_off, k, want=want, require_all=require_all)
+        return e.bm25_topk_rows(q_terms, q_off, scope.rows, scope.off, k, want=want, require_all=require_all)
+    ids, sc, cnt = run(engine)
     if delta is None:
         return ids, sc, cnt
-    d_ids, d_sc, d_cnt = delta.bm25_topk(q_terms, q_off, k, want=want, require_all=require_all)
+    d_ids, d_sc, d_cnt = run(delta)
     m_sc, m_ids, m_cnt = engine.merge_topk(torch.stack([sc, d_sc]).to(torch.float64), torch.stack([ids, d_ids]),
                                            torch.stack([cnt, d_cnt]), k)
     m_sc = torch.where(m_ids < 0, torch.zeros_like(m_sc), m_sc).to(torch.float32)   # thr_bm25_topk pads with 0
@@ -129,10 +172,14 @@ class DenseFunnel:
 
 
 def dense_topk_one(engine: Engine, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None,
-                   funnel: Optional[DenseFunnel] = None):
+                   funnel: Optional[DenseFunnel] = None, scope: Optional[Scope] = None):
     """K1 on one handle (Engine.dense_topk's results).  With a funnel: the prefix K1 with k = pool, the full-width
     re-score of the pool and its top k (thr_dense_topk_prefix -> thr_dense_rescore -> thr_dense_funnel_finish); the gap
-    is then the pool's certificate."""
+    is then the pool's certificate.  With a scope: the exact top k of each query's rows (thr_dense_topk_rows; the
+    funnel and the margin do not apply, the gap is +inf)."""
+    if scope is not None:
+        _check_scope(scope, Q.shape[0])
+        return engine.dense_topk_rows(Q, scope.rows, scope.off, k, want=want)
     if funnel is None:
         return engine.dense_topk(Q, k, margin, want=want)
     funnel.check(Q.shape[1], k, margin)
@@ -249,8 +296,9 @@ class TripleHybridSearcher:
                k_sem: int = 100, k_lex: int = 100, top_k: int = 100, margin: int = 28,
                tie_mode: int = _lib.TIE_CHUNK_ID, rrf_k: int = 60, want: Optional[torch.Tensor] = None,
                require_all: bool = False, lex_delta: Optional[Engine] = None,
-               funnel: Optional[DenseFunnel] = None) -> SearchOutput:
-        """want: int32 [B] on the device — per query, the tag its semantic and lexical hits must carry (< 0: any);
+               funnel: Optional[DenseFunnel] = None, scope: Optional[Scope] = None) -> SearchOutput:
+        """scope: per-query document scopes (Scope; single GPU only): both channels answer over each query's rows
+        only, exactly, and the funnel is not applied.  want: int32 [B] on the device — per query, the tag its semantic and lexical hits must carry (< 0: any);
         needs set_tags.  require_all: AND semantics of the lexical channel (thr_bm25_topk_ex).  lex_delta: the handle
         of a lexical delta segment (ResidentIndex.delta_engine), searched and merged with the main list; single GPU
         only.  funnel: the semantic channel through the prefix funnel (DenseFunnel; single GPU only).  The graph list is
@@ -262,6 +310,9 @@ class TripleHybridSearcher:
             raise NotImplementedError("a lexical delta segment is not supported with a sharded corpus")
         if funnel is not None and self.world > 1:
             raise NotImplementedError("the dense funnel is not supported with a process group")
+        if scope is not None and self.world > 1:
+            raise NotImplementedError("a document scope is not supported with a process group")
+        _check_scope(scope, B)
         if self.overlap:
             # The two channels do not depend on each other: K2's chain (plan, range kernel, unit merge) goes on a
             # second stream and K1's (seed, select, score, finalize) on a high-priority one.  Both big kernels take
@@ -275,17 +326,17 @@ class TripleHybridSearcher:
             s_lex.wait_stream(main)
             with torch.cuda.stream(s_lex):
                 l_ids, l_sc, l_cnt = bm25_topk_segments(eng, lex_delta, q_terms, q_off, k_lex, want=want,
-                                                        require_all=require_all)
+                                                        require_all=require_all, scope=scope)
             with torch.cuda.stream(s_dense):
-                d_ids, d_sc, d_cnt, gap = dense_topk_one(eng, Q, k_sem, margin, want=want, funnel=funnel)
+                d_ids, d_sc, d_cnt, gap = dense_topk_one(eng, Q, k_sem, margin, want=want, funnel=funnel, scope=scope)
             main.wait_stream(s_dense)
             main.wait_stream(s_lex)
             for t in (l_ids, l_sc, l_cnt, d_ids, d_sc, d_cnt, gap):   # allocated on the side streams, consumed on `main`
                 t.record_stream(main)
         else:
-            d_ids, d_sc, d_cnt, gap = dense_topk_one(eng, Q, k_sem, margin, want=want, funnel=funnel)
+            d_ids, d_sc, d_cnt, gap = dense_topk_one(eng, Q, k_sem, margin, want=want, funnel=funnel, scope=scope)
             l_ids, l_sc, l_cnt = bm25_topk_segments(eng, lex_delta, q_terms, q_off, k_lex, want=want,
-                                                    require_all=require_all)
+                                                    require_all=require_all, scope=scope)
         if self.world > 1:
             d_ids, d_sc, d_cnt, l_ids, l_sc, l_cnt = self._exchange(B, k_sem, k_lex, d_ids, d_sc, d_cnt,
                                                                     l_ids, l_sc, l_cnt)
@@ -508,31 +559,34 @@ class ShardedSearcher:
                k_sem: int = 100, k_lex: int = 100, top_k: int = 100, margin: int = 28,
                tie_mode: int = _lib.TIE_CHUNK_ID, rrf_k: int = 60, want: Optional[torch.Tensor] = None,
                require_all: bool = False, lex_delta: Optional[Engine] = None,
-               funnel: Optional[DenseFunnel] = None) -> SearchOutput:
-        """TripleHybridSearcher.search's arguments; inputs on the home GPU.  lex_delta: the handle of the LAST shard's
+               funnel: Optional[DenseFunnel] = None, scope: Optional[Scope] = None) -> SearchOutput:
+        """TripleHybridSearcher.search's arguments; inputs on the home GPU.  scope: every shard scores the scope's rows
+        it holds (the scope is copied to each other GPU), and the lists are merged as the scans' are.  lex_delta: the handle of the LAST shard's
         lexical delta segment (its ids follow that shard's rows); it is one more lexical source of the merge.
         SearchOutput.gap is the merged list's certificate: the minimum of the shards' gaps (with a funnel: of the
         merged prefix pool)."""
         B = Q.shape[0]
         d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt = self._topk(B, Q, q_terms, q_off, k_sem, k_lex, margin, want,
-                                                                 require_all, lex_delta, funnel)
+                                                                 require_all, lex_delta, funnel, scope)
         return self._home._fuse(B, d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt, graph_ids, weights, top_k, tie_mode,
                                 rrf_k)
 
     def dense_topk(self, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None,
-                   funnel: Optional[DenseFunnel] = None):
+                   funnel: Optional[DenseFunnel] = None, scope: Optional[Scope] = None):
         """K1 on every shard, merged: Engine.dense_topk's results (gap: the minimum of the shards').  With a funnel:
         the shards' prefix top-pool lists merged into the global pool, each pool row re-scored on the shard that holds
-        it, and the top k of the pool (dense_topk_one's result, whatever the sharding)."""
+        it, and the top k of the pool (dense_topk_one's result, whatever the sharding).  With a scope:
+        thr_dense_topk_rows on every shard, merged (the funnel does not apply)."""
         d_ids, d_sc, d_cnt, gap, _, _, _ = self._topk(Q.shape[0], Q, None, None, k, 1, margin, want, False, None,
-                                                      funnel)
+                                                      funnel, scope)
         return d_ids, d_sc, d_cnt, gap
 
     def bm25_topk(self, q_terms: torch.Tensor, q_off: torch.Tensor, k: int, want: Optional[torch.Tensor] = None,
-                  require_all: bool = False, lex_delta: Optional[Engine] = None):
-        """K2 on every shard (and the last shard's delta segment), merged: Engine.bm25_topk's results."""
+                  require_all: bool = False, lex_delta: Optional[Engine] = None, scope: Optional[Scope] = None):
+        """K2 on every shard (and the last shard's delta segment), merged: Engine.bm25_topk's results.  With a scope:
+        thr_bm25_topk_rows on every shard and the delta segment, merged."""
         _, _, _, _, l_ids, l_sc, l_cnt = self._topk(q_off.numel() - 1, None, q_terms, q_off, 1, k, 0, want,
-                                                    require_all, lex_delta)
+                                                    require_all, lex_delta, None, scope)
         return l_ids, l_sc, l_cnt
 
     def _empty(self, B: int, k: int, dense: bool):
@@ -545,12 +599,15 @@ class ShardedSearcher:
                     torch.full((B,), float("inf"), dtype=torch.float32, device=dev))
         return ids, torch.zeros((B, k), dtype=torch.float32, device=dev), cnt
 
-    def _topk(self, B, Q, q_terms, q_off, k_sem, k_lex, margin, want, require_all, lex_delta, funnel=None):
+    def _topk(self, B, Q, q_terms, q_off, k_sem, k_lex, margin, want, require_all, lex_delta, funnel=None, scope=None):
         """Both channels (Q None: no semantic search; q_terms None: no lexical one) on every shard, merged on the
         home GPU in one thr_shard_merge launch -> d_ids, d_sc, d_cnt, gap, l_ids, l_sc, l_cnt.  With a funnel the
         semantic lists are the shards' prefix pools, and the merged pool is finished by _funnel_finish."""
         k_out = k_sem
         d_scan = None
+        _check_scope(scope, B)
+        if scope is not None:
+            funnel = None        # a scoped search is exact: the funnel does not apply
         if funnel is not None and Q is not None:
             funnel.check(Q.shape[1], k_sem, margin)
             k_sem, d_scan = funnel.pool, funnel.dims
@@ -567,17 +624,22 @@ class ShardedSearcher:
                 qt, qo = (q_terms, q_off) if q_terms is None or local else \
                     (q_terms.to(dev, non_blocking=True), q_off.to(dev, non_blocking=True))
                 w = want if want is None or local else want.to(dev, non_blocking=True)
+                sc = None if scope is None else scope.to(dev)
+
+                def lexical(e):
+                    if sc is None:
+                        return e.bm25_topk(qt, qo, k_lex, want=w, require_all=require_all)
+                    return e.bm25_topk_rows(qt, qo, sc.rows, sc.off, k_lex, want=w, require_all=require_all)
                 for s in shards:
                     e = self.engines[s]
                     if Q is not None:
-                        sem.append((s, tuple(self._home_view(s, t)
-                                             for t in e.dense_topk(q, k_sem, margin, want=w, d_scan=d_scan))))
+                        d = e.dense_topk(q, k_sem, margin, want=w, d_scan=d_scan) if sc is None else \
+                            e.dense_topk_rows(q, sc.rows, sc.off, k_sem, want=w)
+                        sem.append((s, tuple(self._home_view(s, t) for t in d)))
                     if q_terms is not None:
-                        l = e.bm25_topk(qt, qo, k_lex, want=w, require_all=require_all)
-                        lex.append((s, tuple(self._home_view(s, t) for t in l)))
+                        lex.append((s, tuple(self._home_view(s, t) for t in lexical(e))))
                         if s == last and lex_delta is not None:
-                            l = lex_delta.bm25_topk(qt, qo, k_lex, want=w, require_all=require_all)
-                            lex.append((s + 1, tuple(self._home_view(s, t) for t in l)))
+                            lex.append((s + 1, tuple(self._home_view(s, t) for t in lexical(lex_delta))))
             if st is not main:
                 main.wait_stream(st)
         # a fixed source order (shard order, the delta segment last), whatever the grouping by GPU

@@ -17,7 +17,7 @@ import torch
 
 from .engine import Engine
 from .index import BM25Index, bm25_idf
-from .pipeline import (DenseFunnel, ShardedSearcher, TripleHybridSearcher, bm25_topk_segments, dense_topk_one,
+from .pipeline import (DenseFunnel, Scope, ShardedSearcher, TripleHybridSearcher, bm25_topk_segments, dense_topk_one,
                        maxsim_store)
 from .tokpack import Codebook, PackedTokenStore, encode as encode_tokens
 
@@ -209,6 +209,7 @@ class ResidentIndex:
         dev = self._store_dev
         self.rows = rows
         self.id_of = {r["child_id"]: i for i, r in enumerate(rows)}
+        self._index_documents()
         self.collections = [r.get("collection") for r in rows]
         self._Xbuf = X
         self._set_tokens(token_store, token_lens)
@@ -338,6 +339,32 @@ class ResidentIndex:
             dd = self._dead[self.n_main:]
             de.bm25_deleted_set(pack_bitmap(dd).to(dev) if dd.any() else None)
 
+    def _index_documents(self) -> None:
+        """document_id -> its live rows, from id_of (after a build or a load); updates keep it in step row by row."""
+        self._doc_rows: Dict[Any, set] = {}
+        for i in self.id_of.values():
+            self._doc_rows.setdefault(self.rows[i].get("document_id"), set()).add(i)
+
+    def document_rows(self, document_id) -> List[int]:
+        """The live rows of a document, ascending (empty for an unknown id)."""
+        return sorted(self._doc_rows.get(document_id, ()))
+
+    def scope(self, documents_per_query: Sequence[Sequence[Any]]) -> Scope:
+        """Per query, the document ids it may be answered from -> a pipeline.Scope on the home GPU: each query's live
+        rows of those documents, ascending (an unknown id contributes nothing; an empty list gives an empty scope,
+        which returns nothing in either channel).  Pass it as scope= to dense_topk / bm25_topk / searcher().search."""
+        per_q = []
+        for docs in documents_per_query:
+            rows = set()
+            for d in docs:
+                rows |= self._doc_rows.get(d, set())
+            per_q.append(sorted(rows))
+        off = np.zeros(len(per_q) + 1, dtype=np.int64)
+        np.cumsum([len(r) for r in per_q], out=off[1:])
+        flat = np.fromiter((i for r in per_q for i in r), dtype=np.int64, count=int(off[-1]))
+        dev = self.engine.device
+        return Scope(torch.from_numpy(flat).to(dev), torch.from_numpy(off).to(dev))
+
     @property
     def n_live(self) -> int:
         """Live chunks: the corpus size every search sees."""
@@ -383,22 +410,24 @@ class ResidentIndex:
         return s
 
     def dense_topk(self, Q: torch.Tensor, k: int, margin: int = 28, want: Optional[torch.Tensor] = None,
-                   funnel: Optional[DenseFunnel] = None):
+                   funnel: Optional[DenseFunnel] = None, scope: Optional[Scope] = None):
         """K1 over the embedding rows (Engine.dense_topk's arguments and results; over several shards the certificate
         is the minimum of theirs).  funnel: through the prefix funnel (pipeline.DenseFunnel); the same result for any
-        sharding, and the certificate is the prefix pool's."""
+        sharding, and the certificate is the prefix pool's.  scope: each query's exact top k over its scope's rows
+        (`scope()`); the funnel does not apply and the certificate is +inf."""
         if self.n_shards == 1:
-            return dense_topk_one(self.engine, Q, k, margin, want=want, funnel=funnel)
-        return self.searcher().dense_topk(Q, k, margin, want=want, funnel=funnel)
+            return dense_topk_one(self.engine, Q, k, margin, want=want, funnel=funnel, scope=scope)
+        return self.searcher().dense_topk(Q, k, margin, want=want, funnel=funnel, scope=scope)
 
     def bm25_topk(self, q_terms: torch.Tensor, q_off: torch.Tensor, k: int, want: Optional[torch.Tensor] = None,
-                  require_all: bool = False):
-        """K2 over the main segment(s) and the delta segment (Engine.bm25_topk's arguments and results)."""
+                  require_all: bool = False, scope: Optional[Scope] = None):
+        """K2 over the main segment(s) and the delta segment (Engine.bm25_topk's arguments and results); scope: over
+        each query's scope's rows only."""
         if self.n_shards == 1:
             return bm25_topk_segments(self.engine, self.delta_engine, q_terms, q_off, k, want=want,
-                                      require_all=require_all)
+                                      require_all=require_all, scope=scope)
         return self.searcher().bm25_topk(q_terms, q_off, k, want=want, require_all=require_all,
-                                         lex_delta=self.delta_engine)
+                                         lex_delta=self.delta_engine, scope=scope)
 
     def maxsim_rows(self, eng: Engine, qtok: torch.Tensor, rows: Sequence[int]) -> torch.Tensor:
         """K4 of one query [1, Tq, 128] over token-store rows (< 0: not scored), each row scored on the shard that
@@ -480,6 +509,7 @@ class ResidentIndex:
             self._dead = np.concatenate([self._dead, np.zeros(n, dtype=bool)])
             for i, c in enumerate(ids):
                 self.id_of[c] = N + i
+                self._doc_rows.setdefault(chunks[i].get("document_id"), set()).add(N + i)
             self.parents.update(parents or {})
             self.version += 1
             self._publish(main=False, delta=True)
@@ -514,6 +544,11 @@ class ResidentIndex:
         for i in rows:
             self._dead[i] = True
             del self.id_of[self.rows[i]["child_id"]]
+            doc = self.rows[i].get("document_id")
+            live = self._doc_rows[doc]
+            live.discard(i)
+            if not live:
+                del self._doc_rows[doc]
             np.subtract.at(self._df, self._coo_t[self._row_ptr[i]:self._row_ptr[i + 1]], 1)
 
     def compact(self) -> None:
@@ -610,6 +645,7 @@ class ResidentIndex:
             self._df = self.bm25.df.cpu().numpy().astype(np.int64)
             self._coo_t = None                     # recovered by _host_terms on the first update
         self.id_of = {r["child_id"]: i for i, r in enumerate(self.rows) if not self._dead[i]}
+        self._index_documents()
         self._tag = self._tags_of(self.collections)
         self._publish(main=True, delta=True)
 

@@ -154,6 +154,7 @@ class _GpuScoring:
         if dense_funnel is not None and not isinstance(dense_funnel, DenseFunnel):
             raise TypeError("dense_funnel must be a pipeline.DenseFunnel or None")
         self.dense_funnel = dense_funnel
+        self.documents = None      # the document scope `scoped()` binds: None = the whole index
         self.index = index
         self.engine = engine or (index.engine if index is not None else None)
         self._graph_search_fn = graph_search
@@ -164,6 +165,21 @@ class _GpuScoring:
         if self.engine is None:
             raise RuntimeError("GpuRAG2Retriever needs an Engine (libthr.so on a B200); there is no CPU fallback")
         return self.engine
+
+    def scoped(self, documents: Sequence[Any]):
+        """A shallow copy of this retriever bound to a document scope: its channels (and so its own retrieve())
+        answer from the live chunks of `documents` only — exactly, scored on those rows (thr_dense_topk_rows /
+        thr_bm25_topk_rows; the dense funnel does not apply), and graph hits outside them are dropped.  This
+        retriever is not changed."""
+        import copy
+        if isinstance(documents, (str, bytes)):
+            raise TypeError("documents: expected a sequence of document ids")
+        out = copy.copy(self)
+        out.documents = list(documents)
+        return out
+
+    def _scope(self):
+        return None if self.documents is None else self.index.scope([self.documents])
 
 
     # ---- channels ---------------------------------------------------------------------------------
@@ -199,7 +215,7 @@ class _GpuScoring:
         qt, qo = pack_queries([terms], eng.device)
         with eng.lock:     # one state of the index (updates hold the same lock)
             ids, sc, cnt = ix.bm25_topk(qt, qo, max(1, limit), want=ix.want(collection),     # predicate inside K2
-                                        require_all=self.lexical_match == "all")
+                                        require_all=self.lexical_match == "all", scope=self._scope())
             ix.sync()
         n = int(cnt[0])
         return [ix.row_dict(i, rank=r) for i, r in zip(ids[0, :n].tolist(), sc[0, :n].tolist())]
@@ -209,13 +225,23 @@ class _GpuScoring:
         Exact: the result carries K1's certificate (gap above the fp32 accumulation bound); an uncertified result is
         recomputed once with the widest re-scoring margin and, if still uncertified (more exact ties than the
         margin holds), returned with a RuntimeWarning.  With the retriever's dense_funnel the search goes through the
-        prefix funnel, and the certificate (over its `dims` columns) is the prefix pool's."""
+        prefix funnel, and the certificate (over its `dims` columns) is the prefix pool's.  A scoped retriever
+        (`scoped`) scores its scope's rows exactly, with neither funnel nor certificate."""
         eng, ix, fn = self._need_engine(), self.index, self.dense_funnel
         q = torch.as_tensor(self.embedder.embed_query(query_text), dtype=torch.float32).reshape(1, -1)
         if q.shape[1] != ix.dim:
             raise ValueError(f"query embedding has {q.shape[1]} dimensions, the index {ix.dim}")
         q = q / q.norm(dim=1, keepdim=True).clamp_min(1e-30)
         k = min(limit, ix.n_live)
+        if self.documents is not None:
+            if limit > 256:
+                raise ValueError(f"semantic limit {limit} > 256 (the scoped search's largest k)")
+            qd = pad_dim(q.to(torch.bfloat16)).to(eng.device)
+            with eng.lock:
+                ids, sc, cnt, _ = ix.dense_topk(qd, max(k, 1), want=ix.want(collection), scope=self._scope())
+                ix.sync()
+            n = int(cnt[0])
+            return [ix.row_dict(i, similarity=v) for i, v in zip(ids[0, :n].tolist(), sc[0, :n].tolist())]
         depth = k if fn is None else fn.pool     # the list K1 selects: k, or the funnel's pool
         if fn is not None:
             if limit > fn.pool:
@@ -249,9 +275,10 @@ class _GpuScoring:
             ids = self._graph_search_fn(cypher=cypher, keywords=keywords, collection=collection, limit=limit)
             ids = getattr(ids, "chunk_ids", ids)     # the reference's GraphSearchResult (graph_search.py:44-52)
             out = []
+            allowed = None if self.documents is None else set(self.documents)
             for cid in list(ids)[:limit]:
                 i = self.index.id_of.get(cid)
-                if i is not None:
+                if i is not None and (allowed is None or self.index.rows[i].get("document_id") in allowed):
                     out.append(self.index.row_dict(i))
             return out
         except Exception:
@@ -349,18 +376,42 @@ class _GpuScoring:
                        keywords: Sequence[Sequence[str]], graph_ids: Optional[Sequence[Sequence[str]]] = None,
                        top_k: int = 100, k_sem: int = 100, k_lex: int = 50, weights: Optional[Dict[str, float]] = None,
                        collections: Optional[Sequence[Optional[str]]] = None,
-                       tie_mode: int = _lib.TIE_CHUNK_ID) -> List[List[RetrievalCandidate]]:
+                       tie_mode: int = _lib.TIE_CHUNK_ID,
+                       documents: Optional[Sequence[Optional[Sequence[Any]]]] = None) -> List[List[RetrievalCandidate]]:
         """B queries in one pass of K1 + K2 + K3 (no planner, no rerank): returns per query the fused
         candidates (rrf_score and channel ranks set).  query_vectors [B, D].  tie_mode: exact RRF ties by chunk id
         (north_star) or TIE_INSERTION, the reference's stable-sort order (first seen lexical -> semantic -> graph).
-        collections: per query, the collection its semantic and lexical hits must belong to (None: any)."""
+        collections: per query, the collection its semantic and lexical hits must belong to (None: any).
+        documents: per query, the document ids it is answered from (None: the whole index): both channels score the
+        scope's rows exactly and graph ids outside it are dropped before fusion.  A batch that mixes scoped and
+        unscoped queries runs as two searches under one hold of the engine lock (so the whole batch sees one state
+        of the index) and is reassembled in query order; fusion is per query, so every query's result is what it
+        gets alone."""
+        B = len(queries)
         eng, ix = self._need_engine(), self.index
+        if documents is not None:
+            if len(documents) != B:
+                raise ValueError("documents: one entry (a list of document ids, or None) per query")
+            scoped = [b for b in range(B) if documents[b] is not None]
+            if not scoped:
+                documents = None
+            elif len(scoped) < B:
+                res: List[Optional[List[RetrievalCandidate]]] = [None] * B
+                with eng.lock:   # re-entrant: both halves run in this one hold
+                    for idx in (scoped, [b for b in range(B) if documents[b] is None]):
+                        pick = lambda xs: None if xs is None else [xs[b] for b in idx]   # noqa: E731
+                        sub = self.retrieve_batch(pick(queries), query_vectors[idx], pick(keywords), pick(graph_ids),
+                                                  top_k, k_sem, k_lex, weights, pick(collections), tie_mode,
+                                                  documents=pick(documents) if idx is scoped else None)
+                        for b, r in zip(idx, sub):
+                            res[b] = r
+                return res
         with eng.lock:     # a batch is several C-ABI calls on one handle: one thread at a time (engine.lock)
             return self._retrieve_batch_locked(ix.searcher(), queries, query_vectors, keywords, graph_ids,
-                                               top_k, k_sem, k_lex, weights, collections, tie_mode)
+                                               top_k, k_sem, k_lex, weights, collections, tie_mode, documents)
 
     def _retrieve_batch_locked(self, s, queries, query_vectors, keywords, graph_ids, top_k, k_sem, k_lex, weights,
-                               collections, tie_mode):
+                               collections, tie_mode, documents=None):
         eng, ix = self.engine, self.index
         B = len(queries)
         Q = query_vectors.to(torch.float32)
@@ -374,7 +425,9 @@ class _GpuScoring:
             width = max(1, max(len(x) for x in graph_ids))
             g = torch.full((B, width), -1, dtype=torch.int64)
             for b, lst in enumerate(graph_ids):
-                row = [ix.id_of[c] for c in lst if c in ix.id_of]
+                allowed = None if documents is None else set(documents[b])
+                row = [ix.id_of[c] for c in lst
+                       if c in ix.id_of and (allowed is None or ix.rows[ix.id_of[c]].get("document_id") in allowed)]
                 g[b, :len(row)] = torch.tensor(row, dtype=torch.int64)
             g = g.to(eng.device)
         w = weights or {}
@@ -385,11 +438,14 @@ class _GpuScoring:
             want = torch.tensor([-1 if c is None else ix.tag_of.get(c, 0xfffe) for c in collections], dtype=torch.int32,
                                 device=eng.device)
         fn = self.dense_funnel
+        scope = None if documents is None else ix.scope(documents)
+        if scope is not None:
+            fn = None      # a scoped search is exact: the funnel does not apply
         if fn is not None and k_sem > fn.pool:
             raise ValueError(f"k_sem {k_sem} > the dense funnel's pool of {fn.pool}")
         out = s.search(Q, qt, qo, g, weights=wt, k_sem=max(1, min(k_sem, ix.n_live)), k_lex=k_lex, top_k=top_k,
                        want=want, require_all=self.lexical_match == "all", tie_mode=tie_mode, lex_delta=ix.delta_engine,
-                       funnel=fn)
+                       funnel=fn, scope=scope)
         ix.sync()
         ids, rrf, rk, cnt = out.ids.tolist(), out.rrf.tolist(), out.ranks.tolist(), out.count.tolist()
         res = []
